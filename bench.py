@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (libdvfe.so)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's records as .npy, to compare two builds
 
 Workload (`config.workload`): BASELINE.json configs[4] — 64 independent synthetic 1280x720 stereo camera
 streams per GPU, raw mode (TrackImage: temporal LK with forward-backward check, Shi-Tomasi top-up to 400
@@ -32,10 +33,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree may be read-only: no __pycache__ either.  The reference arm's spawned workers re-run this line (spawn executes the
+# main module's top level) before they import the package or the oracle.
+sys.dont_write_bytecode = True
 
 METRIC = "front-end frames/s (stereo KLT+corners)"
 UNIT = "frames/s"
 WORKLOAD = "c5_zed_streams"
+DYN_MAX_INSTANCES = 8          # instance slots per stream of the dynamic-mode workload (dvfe_config::max_instances)
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -60,7 +65,15 @@ def parse_args():
                          "image and fail the round-trip test, i.e. feature churn (new corners per step)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the records each timed leg returned for its last step to DIR/<leg>_<kind>_<field>.npy "
+                         "(float64; rank 0's streams, a fixed sample of them if all would pass 64 MB)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "dvfe":
+        ap.error("--dump-outputs writes the records of the CUDA path (--impl dvfe)")
+    return a
 
 
 def nvml_handle(cuda_index: int):
@@ -267,6 +280,41 @@ def kernel_sources_sha() -> str:
     return h.hexdigest()[:16]
 
 
+DUMP_BYTES = 64 << 20
+
+
+def record_columns(dtype: np.dtype) -> int:
+    """float64 columns one record of `dtype` takes in the dump, the stream index included"""
+    return 1 + sum(int(np.prod(dtype[f].shape)) for f in dtype.names if f != "reserved")
+
+
+def dump_streams(S: int, bytes_per_stream: int) -> list:
+    """The streams --dump-outputs writes: all S, or a seeded sample when S streams at full record capacity
+    (`bytes_per_stream`) would pass DUMP_BYTES.  The choice depends on S and the capacity only, never on the records,
+    so two builds run with the same arguments dump the same streams."""
+    k = min(S, max(1, DUMP_BYTES // bytes_per_stream))
+    if k == S:
+        return list(range(S))
+    return sorted(np.random.default_rng(0).choice(S, k, replace=False).tolist())
+
+
+def write_dumps(out_dir: str, streams: list, legs: dict) -> None:
+    """legs: {leg: {kind: [records of each stream of `streams`]}} -> out_dir/<leg>_<kind>_<field>.npy, float64, one row per
+    record in (stream, record) order, plus <leg>_<kind>_stream.npy.  Ids, camera and stream indices are integers far
+    below 2**53, exact in float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    n_files = n_bytes = 0
+    for leg, kinds in legs.items():
+        for kind, recs in kinds.items():
+            cols = {"stream": np.concatenate([np.full(len(r), s, np.float64) for s, r in zip(streams, recs)])}
+            allr = np.concatenate(recs)
+            cols.update((f, allr[f].astype(np.float64)) for f in allr.dtype.names if f != "reserved")
+            for f, a in cols.items():
+                np.save(os.path.join(out_dir, f"{leg}_{kind}_{f}.npy"), a)
+                n_files, n_bytes = n_files + 1, n_bytes + a.nbytes
+    print(f"bench.py: {n_files} arrays ({n_bytes} B) of {len(streams)} streams written to {out_dir}", file=sys.stderr)
+
+
 def run_dvfe(args):
     import torch
     import torch.distributed as dist
@@ -318,6 +366,12 @@ def run_dvfe(args):
         t.set_stream(stream.cuda_stream)
         return t
 
+    # --dump-outputs: the records of the last timed step of the value and e2e legs (rank 0)
+    dumps, dump_ids = {}, []
+    if args.dump_outputs and rank == 0:
+        from dynamic_vins_b200._lib import OBS_DTYPE
+        dump_ids = dump_streams(S, 2 * (2 * c["max_cnt"]) * record_columns(OBS_DTYPE) * 8)
+
     # ------------------------------------------------------------------ stage split + roofline pass
     # Per-kernel CUDA-event timers only mean something when kernels do not overlap, so the stage split and the roofline
     # of the dominant kernel are measured on the same steps with ONE stream group (every launch covers all S streams);
@@ -366,6 +420,8 @@ def run_dvfe(args):
         launches = lib().dvfe_kernel_launches() - launches0
         ms_value = e0.elapsed_time(e1)
         n_obs = sum(len(trk.features(s)) for s in range(S))
+        if dump_ids:
+            dumps["value"] = {"features": [trk.features(s) for s in dump_ids]}
     trk.close()
 
     # ------------------------------------------------------------------ e2e: host buffers through dvfe_track_image
@@ -407,7 +463,11 @@ def run_dvfe(args):
         barrier()
         ms_e2e = e0.elapsed_time(e1)
         n_obs_e2e = sum(len(trk.features(s)) for s in range(S))
+        if dump_ids:
+            dumps["e2e"] = {"features": [trk.features(s) for s in dump_ids]}
     trk.close()
+    if dump_ids:
+        write_dumps(args.dump_outputs, dump_ids, dumps)
 
     ms_value, ms_e2e, ms_probe = shard.reduce_max([ms_value, ms_e2e, ms_probe], dist if world > 1 else None, dev)
     total_frames = world * S * args.steps
@@ -517,12 +577,17 @@ def run_dvfe_dynamic(args):
     lboxes = [BatchTracker.marshal_boxes([labs[k][s % len(base)][1] for s in range(S)]) for k in range(T)]
     order = synth.pingpong_positions(T, args.warmup + args.steps)
     ones = [1] * S
+    dump_ids = []
+    if args.dump_outputs:
+        from dynamic_vins_b200._lib import INST_OBS_DTYPE, OBS_DTYPE
+        dump_ids = dump_streams(S, 3 * 8 * (2 * c["max_cnt"] * record_columns(OBS_DTYPE)
+                                            + DYN_MAX_INSTANCES * c["max_dynamic_cnt"] * record_columns(INST_OBS_DTYPE)))
 
     def run(kind, groups):
         cfg = make_config(c["width"], c["height"], c["max_cnt"], c["min_dist"], c["cam0"], c["cam1"], stereo=True, n_streams=S,
                           max_dynamic_cnt=c["max_dynamic_cnt"], min_dynamic_dist=c["min_dynamic_dist"],
                           use_mask_morphology=c["use_mask_morphology"], mask_morphology_size=c["mask_morphology_size"],
-                          max_instances=8, device=local, n_groups=max(1, min(groups, S)))
+                          max_instances=DYN_MAX_INSTANCES, device=local, n_groups=max(1, min(groups, S)))
         trk = BatchTracker(cfg)
         def step(i):       # pipelined: frame i is enqueued, then the records of frame i-1 are waited for
             k = order[i]
@@ -547,7 +612,8 @@ def run_dvfe_dynamic(args):
         res = dict(ms=dt / args.steps * 1e3, fps=S * args.steps / dt, launches=int(lib().dvfe_kernel_launches() - launches0),
                    n_inst=sum(len(trk.insts_output(s)) for s in range(S)),
                    n_bg=sum(int((trk.features(s)["cam"] == 0).sum()) for s in range(S)), groups=cfg.n_groups,
-                   records=[(trk.features(s).tobytes(), trk.insts_output(s).tobytes()) for s in range(min(S, 8))])
+                   records=[(trk.features(s).tobytes(), trk.insts_output(s).tobytes()) for s in range(min(S, 8))],
+                   dump={"features": [trk.features(s) for s in dump_ids], "insts": [trk.insts_output(s) for s in dump_ids]})
         trk.close()
         return res
 
@@ -555,6 +621,8 @@ def run_dvfe_dynamic(args):
     lab = run("labels", args.dyn_groups)
     msk = run("masks", args.dyn_groups)
     assert dev["records"] == lab["records"] == msk["records"], "the three input forms must give identical records"
+    if dump_ids:
+        write_dumps(args.dump_outputs, dump_ids, {"value": dev["dump"], "e2e": lab["dump"], "e2e_host_masks": msk["dump"]})
     mask_bytes = sum(int(b["mask"].size) for s_ in range(S) for b in frames[0][s_ % len(base)].boxes)
     P = c["width"] * c["height"]
     out = {"metric": METRIC, "value": dev["fps"], "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": args.warmup,

@@ -13,6 +13,8 @@ from oracle import ref_lib, spec
 
 CAM = synth.CONFIGS["c3_zed_dynamic"]["cam0"]
 CAM_DIST = dict(fx=380.0, fy=382.5, cx=322.1, cy=239.7, k1=-0.31, k2=0.11, p1=1.3e-3, p2=-7.0e-4)
+NEEDS_REF = ("needs oracle/_ref/libdvref.so, compiled from the original dynamic_vins sources: "
+             "make -C oracle/ref REF=<dynamic_vins checkout>")
 
 
 def two_views(rs, n, noise=0.3, out_frac=0.2, f=460.0, c=(640.0, 360.0)):
@@ -69,7 +71,7 @@ def test_find_fundamental_mat_small_inputs():
     assert cv2.findFundamentalMat(same, same.copy(), cv2.FM_RANSAC, 1.0, 0.99)[0] is None
 
 
-@pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref/libdvref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not ref_lib.available(), reason=NEEDS_REF)
 def test_reject_with_f_spec_vs_reference_compiled():
     """The reference's own InstsFeatManager::RejectWithF (compiled from dynamic_tracker.cpp, findFundamentalMat served by cv2)
     against the restatement: undistortion + kFocalLength re-projection + float narrowing + RANSAC."""
@@ -95,7 +97,7 @@ def test_reject_with_f_spec_vs_reference_compiled():
     assert same >= total - 1, (same, total)
 
 
-@pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref/libdvref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not ref_lib.available(), reason=NEEDS_REF)
 @pytest.mark.parametrize("rows,cols", [(37, 53), (120, 200), (300, 420), (8, 8)])
 def test_detect_extra_points_spec_vs_reference_compiled(rows, cols):
     rs = np.random.RandomState(rows)
@@ -158,7 +160,7 @@ def test_cuda_reject_with_f_edge_cases():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref/libdvref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not ref_lib.available(), reason=NEEDS_REF)
 def test_cuda_reject_with_f_equals_reference_compiled():
     from dynamic_vins_b200 import ops
     from test_ref_compiled import _params

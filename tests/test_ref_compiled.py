@@ -17,7 +17,9 @@ from dynamic_vins_b200 import synth
 from oracle import cv_front_end as cvfe
 from oracle import ref_lib, spec
 
-pytestmark = [pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref/libdvref.so not built (needs /root/reference)"),
+NEEDS_REF = ("needs oracle/_ref/libdvref.so, compiled from the original dynamic_vins sources: "
+             "make -C oracle/ref REF=<dynamic_vins checkout>")
+pytestmark = [pytest.mark.skipif(not ref_lib.available(), reason=NEEDS_REF),
               pytest.mark.filterwarnings("ignore::RuntimeWarning")]     # far outside the image the 8-step model overflows: inf / nan
                                                                          # must come out the same, too
 

@@ -62,6 +62,11 @@ class BatchTracker:
         L.check(L.lib().dvfe_create(C.byref(cfg), C.byref(self._h)))
         self._obs = np.zeros(2 * cfg.max_cnt, dtype=L.OBS_DTYPE)
         self._iobs = np.zeros(max(1, cfg.max_instances) * max(1, cfg.max_dynamic_cnt), dtype=L.INST_OBS_DTYPE)
+        # the caller's LK modes and detector (include/dvfe.h defaults); TrackImageNaive overrides the semantic ones for its
+        # own calls only
+        self._lk = [(1, 0.5), (1, 0.5), (1, 0.5), (3, 1.0)]
+        self._detect_cuda = False
+        self._naive = False
 
     def close(self):
         if self._h:
@@ -122,6 +127,7 @@ class BatchTracker:
 
     def track_image(self, left: np.ndarray, right: Optional[np.ndarray], time0) -> None:
         """left/right: (B,H,W) or (H,W) uint8 host arrays."""
+        self._leave_naive()
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
@@ -129,6 +135,7 @@ class BatchTracker:
 
     def track_image_async(self, left: np.ndarray, right: Optional[np.ndarray], time0) -> None:
         """pipelined: enqueue the step and return; the arrays must stay alive until the matching wait()"""
+        self._leave_naive()
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
@@ -141,11 +148,13 @@ class BatchTracker:
 
     def track_image_device(self, d_left: int, d_right: int, stream_stride: int, pitch: int, time0) -> None:
         """d_left/d_right: device pointers (ints), e.g. torch tensor .data_ptr()."""
+        self._leave_naive()
         t = self._times(time0)
         L.check(L.lib().dvfe_track_image_device(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
                                                 stream_stride, pitch, L.ptr(t)))
 
     def track_image_device_async(self, d_left: int, d_right: int, stream_stride: int, pitch: int, time0) -> None:
+        self._leave_naive()
         t = self._times(time0)
         self._keep_t = (t, getattr(self, "_keep_t", (None,))[0])
         L.check(L.lib().dvfe_track_image_device_async(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
@@ -155,24 +164,49 @@ class BatchTracker:
 
     def set_lk_mode(self, back_max_level: int = 1, fb_threshold: float = 0.5, site: int = -1) -> None:
         """Backward-pass depth / round-trip threshold of the LK at one call site (LK_*) or, site = -1, at all four.
-        CPU FeatureTrackByLK: (1, 0.5); cv::cuda call pattern of FeatureTrackByLKGpu: (3, 1.0)."""
+        CPU FeatureTrackByLK: (1, 0.5); cv::cuda call pattern of FeatureTrackByLKGpu: (3, 1.0).  track_image_naive does not
+        change it: its own call pattern applies to the naive calls only."""
+        self._leave_naive()
         L.check(L.lib().dvfe_set_lk_mode_site(self._h, int(site), int(back_max_level), float(fb_threshold)))
+        for i in range(4):
+            if site < 0 or site == i:
+                self._lk[i] = (int(back_max_level), float(fb_threshold))
 
     def set_detect_mode(self, cuda_semantics: bool) -> None:
         """Detector of the semantic path: cv::goodFeaturesToTrack (False, TrackSemanticImage) or the cv::cuda detector's
         threshold rule (True, TrackImageNaive's DetectShiTomasiCornersGpu)."""
+        self._leave_naive()
         L.check(L.lib().dvfe_set_detect_mode(self._h, 1 if cuda_semantics else 0))
+        self._detect_cuda = bool(cuda_semantics)
+
+    # TrackImageNaive switches the two semantic LK sites and the detector; the switch is made when a naive call follows another
+    # entry point and undone when another entry point follows a naive call (each switch drops the tracker's captured graphs)
+    def _enter_naive(self) -> None:
+        if not self._naive:
+            for site in (self.LK_SEMANTIC_TEMPORAL, self.LK_SEMANTIC_STEREO):
+                L.check(L.lib().dvfe_set_lk_mode_site(self._h, site, 3, 1.0))
+            L.check(L.lib().dvfe_set_detect_mode(self._h, 1))
+            self._naive = True
+
+    def _leave_naive(self) -> None:
+        if self._naive:
+            for site in (self.LK_SEMANTIC_TEMPORAL, self.LK_SEMANTIC_STEREO):
+                L.check(L.lib().dvfe_set_lk_mode_site(self._h, site, *self._lk[site]))
+            L.check(L.lib().dvfe_set_detect_mode(self._h, 1 if self._detect_cuda else 0))
+            self._naive = False
 
     def track_image_naive(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
         """FeatureTracker::TrackImageNaive (front_end/background_tracker.cpp:400-516): the semantic step with the cv::cuda call
-        pattern at both LK sites and the cv::cuda detector's threshold."""
-        if not getattr(self, "_naive", False):
-            self.set_lk_mode(3, 1.0)
-            self.set_detect_mode(True)
-            self._naive = True
-        self.track_semantic_image(left, right, inv_merge_mask, exist_inst, time0)
+        pattern (3, 1.0) at both semantic LK sites and the cv::cuda detector's threshold.  The modes of the other entry points
+        (set_lk_mode, set_detect_mode) are left as they were."""
+        self._enter_naive()
+        self._semantic(left, right, inv_merge_mask, exist_inst, time0)
 
     def track_semantic_image(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
+        self._leave_naive()
+        self._semantic(left, right, inv_merge_mask, exist_inst, time0)
+
+    def _semantic(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         m = self._batch(inv_merge_mask, self.B, self.H, self.W)
@@ -223,6 +257,7 @@ class BatchTracker:
 
     def track_dynamic_async(self, left, right, inv_merge_mask, exist_inst, boxes_per_stream, time0) -> None:
         """TrackSemanticImage + InstsTrack of one frame for all streams, pipelined; results after the matching wait()"""
+        self._leave_naive()
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         m = self._batch(inv_merge_mask, self.B, self.H, self.W)
@@ -252,6 +287,7 @@ class BatchTracker:
         """SemanticImage::SetMaskAndRoi on the device: `labels` holds one u8 label image per stream (bit b = the instance whose
         box has label_bit == b).  Host arrays, or (device=True) device addresses `left`, `right`, `labels` of dense
         [B][H][W] buffers.  Pipelined like track_dynamic_async; results after the matching wait()."""
+        self._leave_naive()
         arr, counts, keep = boxes_per_stream if isinstance(boxes_per_stream, tuple) else self.marshal_boxes(boxes_per_stream)
         assert len(counts) == self.B
         t = self._times(time0)

@@ -186,7 +186,9 @@ int dvfe_set_lk_mode_site(dvfe_tracker* t, int site, int back_max_level, double 
  *                     ordering and the distance grid are the same.  Evaluated with this library's CPU-parity response arithmetic
  *                     (cv::cuda's fp32 box sums are not reproduced; its candidate buffer of max(1000, 5 % of the pixels) entries
  *                     is not modelled either).
- * TrackImageNaive = dvfe_set_lk_mode(t, 3, 1.0) + dvfe_set_detect_mode(t, DVFE_DETECT_CUDA) + dvfe_track_semantic_image. */
+ * TrackImageNaive = dvfe_set_lk_mode_site(t, DVFE_LK_SEMANTIC_TEMPORAL and _STEREO, 3, 1.0) + dvfe_set_detect_mode(t,
+ * DVFE_DETECT_CUDA) + dvfe_track_semantic_image; the host wrappers (include/dvfe/feature_tracker.hpp, dynamic_vins_b200/tracker.py)
+ * put the caller's modes back before the next call of another entry point. */
 #define DVFE_DETECT_CPU 0
 #define DVFE_DETECT_CUDA 1
 int dvfe_set_detect_mode(dvfe_tracker* t, int mode);

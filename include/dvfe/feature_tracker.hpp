@@ -159,6 +159,7 @@ public:
     // front_end/background_tracker.cpp:52-158
     FeatureBackground TrackImage(SemanticImage& img) {
         check_input(img);
+        leave_naive();
         cur_img = img;
         const bool right = cfg_.stereo && !img.gray1.empty();
         if (dvfe_track_image(h_, img.gray0.data, right ? img.gray1.data : nullptr, (size_t)img.gray0.step * img.gray0.rows,
@@ -169,30 +170,35 @@ public:
     }
     // front_end/background_tracker.cpp:757-837
     FeatureBackground TrackSemanticImage(SemanticImage& img) {
-        check_input(img);
-        cur_img = img;
-        const bool right = cfg_.stereo && !img.gray1.empty();
-        const int exist = img.exist_inst ? 1 : 0;
-        if (img.exist_inst && (img.inv_merge_mask.empty() || img.inv_merge_mask.step != img.gray0.step / channels_))
-            throw std::runtime_error("TrackSemanticImage: inv_merge_mask must have the layout of gray0");
-        if (dvfe_track_semantic_image(h_, img.gray0.data, right ? img.gray1.data : nullptr,
-                                      img.exist_inst ? img.inv_merge_mask.data : nullptr,
-                                      (size_t)img.gray0.step * img.gray0.rows, img.gray0.step, &exist,
-                                      &img.time0) != DVFE_OK)
-            throw std::runtime_error(dvfe_last_error(h_));
-        prev_img = cur_img;
-        return SetOutputFeats();
+        leave_naive();
+        return semantic(img);
     }
     // FeatureTracker::TrackImageNaive (:400-516): the cv::cuda flow — ErodeMaskGpu, TrackLeftGPU, DetectNewFeature(use_gpu),
-    // TrackRightGPU — i.e. the cv::cuda call pattern at both LK sites and the cv::cuda detector's threshold rule, evaluated with
-    // this library's CPU-parity arithmetic; the dynamic regions are removed through inv_merge_mask like TrackSemanticImage does.
+    // TrackRightGPU — i.e. the cv::cuda call pattern (3, 1.0) at both semantic LK sites and the cv::cuda detector's threshold rule,
+    // evaluated with this library's CPU-parity arithmetic; the dynamic regions are removed through inv_merge_mask like
+    // TrackSemanticImage does.  These modes hold for the naive calls only: the next TrackImage / TrackSemanticImage runs with the
+    // modes set through SetLkMode / SetDetectMode (the library's defaults unless changed).
     FeatureBackground TrackImageNaive(SemanticImage& img) {
         if (!naive_mode_) {
-            if (dvfe_set_lk_mode(h_, 3, 1.0) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+            set_lk_site(DVFE_LK_SEMANTIC_TEMPORAL, 3, 1.0);
+            set_lk_site(DVFE_LK_SEMANTIC_STEREO, 3, 1.0);
             if (dvfe_set_detect_mode(h_, DVFE_DETECT_CUDA) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
             naive_mode_ = true;
         }
-        return TrackSemanticImage(img);
+        return semantic(img);
+    }
+    // dvfe_set_lk_mode_site / dvfe_set_detect_mode for the TrackImage and TrackSemanticImage calls of this tracker (site -1: all four)
+    void SetLkMode(int back_max_level, double fb_threshold, int site = -1) {
+        leave_naive();
+        if (dvfe_set_lk_mode_site(h_, site, back_max_level, fb_threshold) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+        for (int i = 0; i < 4; i++)
+            if (site < 0 || site == i) lk_[i] = {back_max_level, fb_threshold};
+    }
+    void SetDetectMode(bool cuda_semantics) {
+        leave_naive();
+        if (dvfe_set_detect_mode(h_, cuda_semantics ? DVFE_DETECT_CUDA : DVFE_DETECT_CPU) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+        detect_cuda_ = cuda_semantics;
     }
     // visualisation (DrawTrack) is outside the path: the image stays empty, the accessor exists for source compatibility
     GrayImage& img_track() { return img_vis_; }
@@ -219,6 +225,33 @@ public:
     static FeatureTracker*& current() { static FeatureTracker* cur = nullptr; return cur; }
 
 private:
+    // front_end/background_tracker.cpp:757-837 with the modes in force
+    FeatureBackground semantic(SemanticImage& img) {
+        check_input(img);
+        cur_img = img;
+        const bool right = cfg_.stereo && !img.gray1.empty();
+        const int exist = img.exist_inst ? 1 : 0;
+        if (img.exist_inst && (img.inv_merge_mask.empty() || img.inv_merge_mask.step != img.gray0.step / channels_))
+            throw std::runtime_error("TrackSemanticImage: inv_merge_mask must have the layout of gray0");
+        if (dvfe_track_semantic_image(h_, img.gray0.data, right ? img.gray1.data : nullptr,
+                                      img.exist_inst ? img.inv_merge_mask.data : nullptr,
+                                      (size_t)img.gray0.step * img.gray0.rows, img.gray0.step, &exist,
+                                      &img.time0) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+        prev_img = cur_img;
+        return SetOutputFeats();
+    }
+    void set_lk_site(int site, int back_max_level, double fb_threshold) {
+        if (dvfe_set_lk_mode_site(h_, site, back_max_level, fb_threshold) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+    }
+    // the caller's modes again at the two sites and the detector a naive call switched
+    void leave_naive() {
+        if (!naive_mode_) return;
+        for (int site : {DVFE_LK_SEMANTIC_TEMPORAL, DVFE_LK_SEMANTIC_STEREO}) set_lk_site(site, lk_[site].first, lk_[site].second);
+        if (dvfe_set_detect_mode(h_, detect_cuda_ ? DVFE_DETECT_CUDA : DVFE_DETECT_CPU) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+        naive_mode_ = false;
+    }
     void check_input(const SemanticImage& img) const {
         if (img.gray0.empty() || img.gray0.cols != cfg_.width || img.gray0.rows != cfg_.height)
             throw std::runtime_error("FeatureTracker: gray0 is empty or does not match image_width/image_height");
@@ -240,7 +273,9 @@ private:
     dvfe_tracker* h_ = nullptr;
     std::string config_path_;
     int channels_ = 1;
-    bool naive_mode_ = false;
+    bool naive_mode_ = false;                                            // the naive call pattern is switched on
+    std::pair<int, double> lk_[4] = {{1, 0.5}, {1, 0.5}, {1, 0.5}, {3, 1.0}};    // SetLkMode per site (include/dvfe.h defaults)
+    bool detect_cuda_ = false;                                           // SetDetectMode
     GrayImage img_vis_;
 };
 

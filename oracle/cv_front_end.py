@@ -65,6 +65,10 @@ class FrontEndParams:
     # background_tracker.cpp:36-38), used by TrackSemanticImage for the right image (TrackRightGPU)
     gpu_lk_back_max_level: int = 3
     gpu_fb_threshold: float = 1.0
+    # "cv2": the OpenCV entry points the reference calls.  "exact": the same calls composed from oracle/spec.c (LK with the
+    # exact integer arithmetic, the minimum-eigenvalue map + the selection of goodFeaturesToTrack), which the CUDA kernels
+    # reproduce bit for bit; a whole frame step is then comparable with the library without a tolerance.
+    arith: str = "cv2"
 
 
 class IdCounter:
@@ -160,21 +164,30 @@ LK_CRIT = (cv2.TERM_CRITERIA_COUNT + cv2.TERM_CRITERIA_EPS, 30, 0.01)
 
 
 def feature_track_by_lk(img1: np.ndarray, img2: np.ndarray, pts1: np.ndarray,
-                        flow_back: bool = True, max_level: int = 3, back_max_level: int = 1, fb_threshold: float = 0.5):
+                        flow_back: bool = True, max_level: int = 3, back_max_level: int = 1, fb_threshold: float = 0.5,
+                        arith: str = "cv2"):
     """front_end/feature_utils.cpp:35-69.  Returns (pts2 float32 (N,2), status uint8 (N,)).
-    Throws on empty input like the reference (:39-41)."""
+    Throws on empty input like the reference (:39-41).  arith="exact": both calcOpticalFlowPyrLK calls are spec.lk with
+    the exact integer arithmetic (FrontEndParams.arith)."""
     if img1 is None or img2 is None or img1.size == 0 or img2.size == 0 or len(pts1) == 0:
         raise RuntimeError("FeatureTrackByLK() input wrong, received at least one of parameter are empty")
     p1 = np.ascontiguousarray(pts1, dtype=f32).reshape(-1, 1, 2)
-    p2, st, _ = cv2.calcOpticalFlowPyrLK(img1, img2, p1, None, winSize=LK_WIN, maxLevel=max_level,
-                                         criteria=LK_CRIT)
-    status = st.reshape(-1).astype(np.uint8).copy()
+    if arith == "exact":
+        from oracle import spec
+        p2, status = spec.lk(img1, img2, p1, None, max_level, exact_int=True)
+    else:
+        p2, st, _ = cv2.calcOpticalFlowPyrLK(img1, img2, p1, None, winSize=LK_WIN, maxLevel=max_level,
+                                             criteria=LK_CRIT)
+        status = st.reshape(-1).astype(np.uint8).copy()
     p2 = p2.reshape(-1, 2)
     if flow_back:
         rev0 = p1.copy()
-        rev, rst, _ = cv2.calcOpticalFlowPyrLK(img2, img1, p2.reshape(-1, 1, 2).copy(), rev0,
-                                               winSize=LK_WIN, maxLevel=back_max_level, criteria=LK_CRIT,
-                                               flags=cv2.OPTFLOW_USE_INITIAL_FLOW)
+        if arith == "exact":
+            rev, rst = spec.lk(img2, img1, p2, rev0, back_max_level, exact_int=True)
+        else:
+            rev, rst, _ = cv2.calcOpticalFlowPyrLK(img2, img1, p2.reshape(-1, 1, 2).copy(), rev0,
+                                                   winSize=LK_WIN, maxLevel=back_max_level, criteria=LK_CRIT,
+                                                   flags=cv2.OPTFLOW_USE_INITIAL_FLOW)
         rev = rev.reshape(-1, 2)
         rst = rst.reshape(-1)
         for i in range(len(status)):
@@ -199,17 +212,21 @@ def draw_discs(mask: np.ndarray, pts: np.ndarray, radius: int) -> None:
         cv2.circle(mask, (cv_round(p[0]), cv_round(p[1])), int(radius), 0, -1)
 
 
-def good_features(gray: np.ndarray, max_corners: int, min_dist: float, mask: Optional[np.ndarray]):
+def good_features(gray: np.ndarray, max_corners: int, min_dist: float, mask: Optional[np.ndarray], arith: str = "cv2"):
     if max_corners <= 0:
         # cv::goodFeaturesToTrack treats maxCorners <= 0 as "no limit"; the reference never calls it so
         return np.zeros((0, 2), dtype=f32)
+    if arith == "exact":
+        from oracle import spec
+        return spec.gftt_select(spec.min_eigen_val(gray), mask, max_corners, 0.01, float(min_dist))[0].astype(f32)
     p = cv2.goodFeaturesToTrack(gray, max_corners, 0.01, float(min_dist), mask=mask)
     if p is None:
         return np.zeros((0, 2), dtype=f32)
     return p.reshape(-1, 2).astype(f32)
 
 
-def good_features_cuda_semantics(gray: np.ndarray, max_corners: int, min_dist: float, mask: Optional[np.ndarray]):
+def good_features_cuda_semantics(gray: np.ndarray, max_corners: int, min_dist: float, mask: Optional[np.ndarray],
+                                 arith: str = "cv2"):
     """DetectShiTomasiCornersGpu (front_end/feature_utils.cpp:339-348): cv::cuda::createGoodFeaturesToTrackDetector(CV_8UC1, n,
     0.01, min_dist)->detect(img, pts, mask).  The detector lives in a CUDA build of OpenCV that does not exist in this image
     (UNPINNED); its published algorithm (opencv/modules/cudaimgproc/src/gftt.cpp, cuda/gftt.cu) is restated here with the CPU
@@ -218,11 +235,12 @@ def good_features_cuda_semantics(gray: np.ndarray, max_corners: int, min_dist: f
     val > (float)(maxVal * quality) and val == max of its 3x3 neighbourhood; sorted by val descending (thrust's order among
     equal values is unspecified: address descending here, as the CPU detector); the host-side distance grid of the CPU detector.
     Not reproduced: fp32 box sums of the cuda kernel, and its candidate buffer of max(1000, 5 % of the pixels) entries, which
-    drops candidates in atomic order when it overflows (it does not at the candidate counts of this path)."""
+    drops candidates in atomic order when it overflows (it does not at the candidate counts of this path).
+    arith="exact": the response map of spec.min_eigen_val."""
     from oracle import spec
     if max_corners <= 0:
         return np.zeros((0, 2), dtype=f32)
-    eig = cv2.cornerMinEigenVal(gray, 3, ksize=3)
+    eig = spec.min_eigen_val(gray) if arith == "exact" else cv2.cornerMinEigenVal(gray, 3, ksize=3)
     pts, _ = spec.gftt_select(eig, mask, max_corners, 0.01, float(min_dist), unmasked_max=True)
     return pts.astype(f32)
 
@@ -319,7 +337,7 @@ class InstFeat:
         # gpu_pattern: InstFeat::TrackLeftGPU (:191-225) -> FeatureTrackByLKGpu's backward level / threshold
         pts2, status = feature_track_by_lk(last_img, curr_img, self.last_points, bool(P.flow_back), P.lk_max_level,
                                            P.gpu_lk_back_max_level if gpu_pattern else P.lk_back_max_level,
-                                           P.gpu_fb_threshold if gpu_pattern else P.fb_threshold)
+                                           P.gpu_fb_threshold if gpu_pattern else P.fb_threshold, P.arith)
         self.curr_points = pts2
         if mask is not None:
             for i in range(len(status)):
@@ -343,7 +361,7 @@ class InstFeat:
         # gpu_pattern: InstFeat::TrackRightGPU (:278-312) -> FeatureTrackByLKGpu's backward level / threshold
         rp, status = feature_track_by_lk(gray0, gray1, pts, bool(P.flow_back), P.lk_max_level,
                                          P.gpu_lk_back_max_level if gpu_pattern else P.lk_back_max_level,
-                                         P.gpu_fb_threshold if gpu_pattern else P.fb_threshold)
+                                         P.gpu_fb_threshold if gpu_pattern else P.fb_threshold, P.arith)
         self.right_points = _reduce(rp, status)
         self.right_ids = _reduce(list(self.ids), status)
 
@@ -355,9 +373,9 @@ class InstFeat:
         mask_detect = mask.copy() if mask is not None else np.full(gray0.shape, 255, np.uint8)
         draw_discs(mask_detect, self.curr_points, min_dist)
         if use_gpu:                                                            # :373-379 DetectShiTomasiCornersGpu(.., min_dist)
-            n_pts = good_features_cuda_semantics(gray0, n_max_cnt, min_dist, mask_detect)
+            n_pts = good_features_cuda_semantics(gray0, n_max_cnt, min_dist, mask_detect, P.arith)
         else:
-            n_pts = good_features(gray0, n_max_cnt, P.min_dist, mask_detect)   # uses fe_para::kMinDist (:381-382)
+            n_pts = good_features(gray0, n_max_cnt, P.min_dist, mask_detect, P.arith)   # uses fe_para::kMinDist (:381-382)
         self.append_new(n_pts)
 
     def append_new(self, n_pts):
@@ -435,7 +453,7 @@ class FeatureTracker:
         self.stage = {}
         if len(bg.last_points) > 0:                                                 # :61-68
             pts2, status = feature_track_by_lk(self.prev_gray0, gray0, bg.last_points, bool(P.flow_back),
-                                               P.lk_max_level, P.lk_back_max_level, P.fb_threshold)
+                                               P.lk_max_level, P.lk_back_max_level, P.fb_threshold, P.arith)
             self.stage["lk_pts"], self.stage["lk_status"] = pts2.copy(), status.copy()
             bg.last_points = _reduce(bg.last_points, status)
             bg.curr_points = _reduce(pts2, status)
@@ -446,7 +464,7 @@ class FeatureTracker:
         # output map or the disc mask (SURVEY.md Q9); order is kept.
         draw_discs(mask, bg.curr_points, P.min_dist)                                # :79-80
         n_max_cnt = P.max_cnt - len(bg.curr_points)
-        n_pts = good_features(gray0, n_max_cnt, P.min_dist, mask) if n_max_cnt > 0 else np.zeros((0, 2), f32)
+        n_pts = good_features(gray0, n_max_cnt, P.min_dist, mask, P.arith) if n_max_cnt > 0 else np.zeros((0, 2), f32)
         self.last_mask = mask
         self.stage["new_pts"] = n_pts.copy()
         bg.append_new(n_pts)                                                        # :92-96
@@ -587,7 +605,7 @@ class InstsFeatManager:
                 inst.roi_mask = erode_mask(inst.roi_mask, 5)                        # in place in the reference
                 inst_mask = inst.roi_mask.copy()
                 draw_discs(inst_mask, inst.curr_points, P.min_dynamic_dist)
-                new_pts = good_features(inst.roi_gray, max_new, P.min_dynamic_dist, inst_mask)
+                new_pts = good_features(inst.roi_gray, max_new, P.min_dynamic_dist, inst_mask, P.arith)
                 inst.append_new(new_pts)
             dt = self.curr_time - self.last_time
             for key in sorted(self.instances):                                      # :448-457

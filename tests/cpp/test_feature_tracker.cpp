@@ -196,8 +196,46 @@ static int run_dynbatch(int argc, char** argv) {
     return 0;
 }
 
+// test_feature_tracker switch <config.yaml> <frames.bin> <calls> <out_prefix> [<back_max_level> <fb_threshold>]
+// One FeatureTracker, frame k through the entry point calls[k]: 'R' TrackImage, 'S' TrackSemanticImage, 'N' TrackImageNaive.
+// With the optional pair, SetLkMode sets the three sites of the CPU call pattern (both TrackImage sites and the temporal site
+// of TrackSemanticImage) first.  frames.bin: per frame time0 f64, exist_inst i32, gray0, gray1, inv_merge_mask (H*W each)
+static int run_switch(int argc, char** argv) {
+    const std::string calls = argv[4];
+    dynamic_vins::FeatureTracker tracker(argv[2]);
+    if (argc >= 8)
+        for (int site : {DVFE_LK_RAW_TEMPORAL, DVFE_LK_RAW_STEREO, DVFE_LK_SEMANTIC_TEMPORAL})
+            tracker.SetLkMode(std::atoi(argv[6]), std::atof(argv[7]), site);
+    const int W = tracker.config().width, H = tracker.config().height;
+    std::ifstream fin(argv[3], std::ios::binary);
+    std::vector<uint8_t> g0((size_t)W * H), g1((size_t)W * H), inv((size_t)W * H);
+    for (size_t k = 0; k < calls.size(); k++) {
+        dynamic_vins::SemanticImage img;
+        int32_t exist = 0;
+        fin.read(reinterpret_cast<char*>(&img.time0), sizeof(double));
+        fin.read(reinterpret_cast<char*>(&exist), sizeof(exist));
+        fin.read(reinterpret_cast<char*>(g0.data()), (std::streamsize)g0.size());
+        fin.read(reinterpret_cast<char*>(g1.data()), (std::streamsize)g1.size());
+        fin.read(reinterpret_cast<char*>(inv.data()), (std::streamsize)inv.size());
+        img.gray0 = {g0.data(), H, W, W};
+        img.gray1 = {g1.data(), H, W, W};
+        img.inv_merge_mask = {inv.data(), H, W, W};
+        img.exist_inst = exist != 0;
+        img.seq = (unsigned)k;
+        const char c = calls[k];
+        const dynamic_vins::FeatureBackground fb = c == 'R' ? tracker.TrackImage(img)
+                                                 : c == 'S' ? tracker.TrackSemanticImage(img)
+                                                            : tracker.TrackImageNaive(img);
+        write_points(argv[5], -1, (int)k, fb);
+    }
+    return 0;
+}
+
 int main(int argc, char** argv) {
     if (argc < 6) { std::fprintf(stderr, "usage\n"); return 2; }
+    if (std::string(argv[1]) == "switch") {
+        try { return run_switch(argc, argv); } catch (const std::exception& e) { std::fprintf(stderr, "error: %s\n", e.what()); return 1; }
+    }
     if (std::string(argv[1]) == "batch") {
         try { return run_batch(argc, argv); } catch (const std::exception& e) { std::fprintf(stderr, "error: %s\n", e.what()); return 1; }
     }

@@ -4,9 +4,9 @@ The compute path is libdvfe.so (hand-written sm_100a CUDA kernels behind the C A
 This package is the thin host-side mirror of the reference's FeatureTracker interface over that ABI.
 """
 from . import synth  # noqa: F401  (numpy only)
-from ._lib import DvfeError, LIB_PATH, lib  # noqa: F401
+from ._lib import DvfeError, LIB_PATH, lib, FRAME_SKIP, FRAME_NO_RIGHT, FRAME_RESET, STEP_DEVICE_INPUT  # noqa: F401
 from .tracker import BatchTracker, FeatureTracker, config_from_yaml, make_config, obs_to_map  # noqa: F401
 from . import ops  # noqa: F401
 
 __all__ = ["BatchTracker", "FeatureTracker", "config_from_yaml", "make_config", "obs_to_map", "ops", "synth",
-           "DvfeError", "lib", "LIB_PATH"]
+           "DvfeError", "lib", "LIB_PATH", "FRAME_SKIP", "FRAME_NO_RIGHT", "FRAME_RESET", "STEP_DEVICE_INPUT"]

@@ -79,7 +79,12 @@ SYMBOLS = [
     "dvfe_op_disc_mask", "dvfe_op_erode_rect", "dvfe_op_lift_projective", "dvfe_op_bgr_to_gray", "dvfe_op_merge_masks",
     "dvfe_op_remap", "dvfe_set_input", "dvfe_set_undistort_maps", "dvfe_track_dynamic_async", "dvfe_op_punch_out", "dvfe_insts_table", "dvfe_track_dynamic_ex",
     "dvfe_op_reject_with_f", "dvfe_op_detect_extra_points", "dvfe_op_build_pyramid_bordered", "dvfe_set_detect_mode", "dvfe_op_good_features_cuda",
+    "dvfe_track_image_ex",
 ]
+
+# dvfe_track_image_ex: per-stream frame flags and step flags (include/dvfe.h)
+FRAME_SKIP, FRAME_NO_RIGHT, FRAME_RESET = 1, 2, 4
+STEP_DEVICE_INPUT = 1
 
 _lib = None
 
@@ -107,6 +112,7 @@ def lib() -> C.CDLL:
         L.dvfe_track_image_async.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
         L.dvfe_wait.argtypes = [C.c_void_p]
         L.dvfe_track_image_device_async.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
+        L.dvfe_track_image_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p, C.c_uint]
         L.dvfe_set_lk_mode.argtypes = [C.c_void_p, C.c_int, C.c_double]
         L.dvfe_set_lk_mode_site.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double]
         L.dvfe_track_image_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]

@@ -61,6 +61,18 @@ int grp_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* r
     return DVFE_OK;
 }
 
+// every group submits a step, also one whose streams are all skipped, so that each dvfe_wait still pairs with one step per group
+int grp_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
+                       const double* time0, const uint8_t* stream_flags, bool device) {
+    for (size_t g = 0; g < t->groups.size(); g++) {
+        const int f = t->group_first[g];
+        const size_t off = (size_t)f * stride;
+        DVFE_CHECK(dvfe_track_image_ex(t->groups[g], left + off, right ? right + off : nullptr, stride, pitch, time0 + f,
+                                       stream_flags ? stream_flags + f : nullptr, device ? DVFE_STEP_DEVICE_INPUT : 0u));
+    }
+    return DVFE_OK;
+}
+
 int grp_wait(dvfe_tracker* t) {
     for (dvfe_tracker* g : t->groups) DVFE_CHECK(dvfe_wait(g));
     return DVFE_OK;

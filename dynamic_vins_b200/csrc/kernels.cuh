@@ -126,6 +126,25 @@ int launch_erode_rect(const uint8_t* src, int spitch, uint8_t* dst, int dpitch, 
 
 int launch_erode_jobs(const ErodeJob* d_jobs, int n_jobs, int max_w, int max_h, cudaStream_t st);
 
+// presence.cu: the extra work of a step in which some streams have no frame, no right image or start over
+#define SF_TCACHE_VALID 0x80u    // stream flag byte, set by the host: the stream's forward-template cache matches its points
+#define LANE_PRESENT 1u          // lane byte (d_lane): the stream has a frame in this step (0 = skipped)
+#define LANE_STEREO 2u           // ... and a right image
+struct PartialTables {
+    const LkGroup* full_temporal;    // the tables of the step's buffer phase
+    const LkGroup* full_stereo;
+    const GfttJob* full_jobs;
+    LkGroup* temporal;               // out
+    LkGroup* stereo;                 // out
+    GfttJob* jobs;                   // out
+    uint8_t* lane;                   // out
+    const int* zero;                 // a device 0: the point count of a stream a table leaves out
+    int* n;                          // [B] point counts (RESET: 0)
+    uint32_t* next_id;               // [B] id counters (RESET: 1)
+};
+int launch_partial_tables(const PartialTables& p, const uint8_t* d_sflags, int n_streams, int stereo_now, cudaStream_t st);
+int launch_carry_pyramids(uint8_t* cur, const uint8_t* prev, size_t bytes, const uint8_t* d_sflags, int n_streams, cudaStream_t st);
+
 // points.cu
 struct CamParams {
     double inv_K11, inv_K13, inv_K22, inv_K23;

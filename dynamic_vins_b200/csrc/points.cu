@@ -151,11 +151,19 @@ int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamPara
 // ---- right image: RightUndistortedPts + RightPtsVelocity + SetOutputFeats --------------------------------
 // One block per point set.  Emits dvfe_obs records sorted by (id, cam): the point arrays are always in
 // ascending id order (survivors keep their order, new ids are appended).
+// lanes (nullable, per set): 0 = the set had no frame in this step (no records, nothing written), else LANE_PRESENT and
+// LANE_STEREO when it had a right image; null = every set present, with a right image iff stereo_now.
 __global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int cap, CamParams cam1, const double* __restrict__ dt,
-                                                         int stereo_now, dvfe_obs* __restrict__ obs, int* __restrict__ n_obs) {
+                                                         int stereo_all, const uint8_t* __restrict__ lanes,
+                                                         dvfe_obs* __restrict__ obs, int* __restrict__ n_obs) {
     __shared__ int s_warp[8];
     __shared__ int s_base;
     const int set = blockIdx.x;
+    if (lanes != nullptr && lanes[set] == 0) {
+        if (threadIdx.x == 0) n_obs[set] = 0;
+        return;
+    }
+    const int stereo_now = lanes != nullptr ? (lanes[set] & LANE_STEREO) != 0 : stereo_all;
     const size_t o = (size_t)set * cap;
     const int n = S.n[set];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -210,9 +218,9 @@ __global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int c
 }
 
 int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
-                           int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st) {
+                           int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st, const uint8_t* d_lane) {
     if (n_sets <= 0) return DVFE_OK;
-    DVFE_LAUNCH(k_right_post_pack, n_sets, 256, 0, st, S, cap, cam1, d_dt, stereo_now, obs, n_obs);
+    DVFE_LAUNCH(k_right_post_pack, n_sets, 256, 0, st, S, cap, cam1, d_dt, stereo_now, d_lane, obs, n_obs);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }

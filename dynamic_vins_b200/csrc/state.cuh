@@ -28,4 +28,4 @@ int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const Ca
                           int* d_n_out, cudaStream_t st);
 int launch_clear_sets(int* d_n, const uint8_t* d_flags, int n_sets, cudaStream_t st);
 int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
-                           int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st);
+                           int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st, const uint8_t* d_lane = nullptr);

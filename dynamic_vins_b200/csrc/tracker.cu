@@ -35,6 +35,8 @@ int grp_create(const dvfe_config* cfg, dvfe_tracker** out);
 void grp_destroy(dvfe_tracker* t);
 int grp_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
                           const double* time0, bool device);
+int grp_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
+                       const double* time0, const uint8_t* stream_flags, bool device);
 int grp_wait(dvfe_tracker* t);
 int grp_wait_all(dvfe_tracker* t);
 int grp_track_semantic(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv, size_t stride, int pitch,
@@ -197,6 +199,17 @@ int dvfe_tracker::init() {
     DVFE_CHECK(dmalloc(&d_dt, (size_t)B));
     DVFE_CHECK(dmalloc(&d_err, (size_t)2));
     prev_time.assign(B, 0.0);
+    tc_valid.assign(B, 0);
+    DVFE_CHECK(dmalloc(&d_sflags, (size_t)B));
+    DVFE_CHECK(dmalloc(&d_lane, (size_t)B));
+    DVFE_CHECK(dmalloc(&d_pgroups[0], (size_t)B));
+    DVFE_CHECK(dmalloc(&d_pgroups[1], (size_t)B));
+    DVFE_CHECK(dmalloc(&d_pjobs, (size_t)B));
+    DVFE_CHECK(dmalloc(&d_zero, (size_t)1));
+    for (int p = 0; p < 2; p++) {
+        DVFE_CUDA(cudaMallocHost((void**)&h_sflags[p], (size_t)B));
+        memset(h_sflags[p], 0, (size_t)B);
+    }
     for (int p = 0; p < 2; p++) {
         DVFE_CHECK(dmalloc(&d_obs[p], (size_t)B * 2 * cap));
         DVFE_CHECK(dmalloc(&d_nobs[p], (size_t)B));
@@ -315,7 +328,10 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     free_point_sets(&t->bg);
     cudaFree(t->d_next_id); cudaFree(t->d_dt); cudaFree(t->d_err); cudaFree(t->d_tcache); cudaFree(t->d_tcache_bwd);
     cudaFree(t->d_old_idx);
+    cudaFree(t->d_sflags); cudaFree(t->d_lane); cudaFree(t->d_pgroups[0]); cudaFree(t->d_pgroups[1]); cudaFree(t->d_pjobs);
+    cudaFree(t->d_zero);
     for (int p = 0; p < 2; p++) {
+        cudaFreeHost(t->h_sflags[p]);
         cudaFree(t->d_obs[p]); cudaFree(t->d_nobs[p]);
         if (t->ev_packed[p]) cudaEventDestroy(t->ev_packed[p]);
         if (t->ev_resp[p]) cudaEventDestroy(t->ev_resp[p]);
@@ -361,8 +377,10 @@ void dvfe_tracker::drop_graphs() {
 // The kernels of one frame step on the compute stream `st` (+ the right pyramid on `rs`, forked and joined by events).
 // No host-dependent state is read: the same call with the same arguments enqueues the same work, which is what lets
 // submit() capture it into a graph.
+// partial: the step of dvfe_track_image_ex with some stream flag set (raw mode only).  The same kernels run on the partial tables
+// (presence.cu), which k_partial_tables derives from the flags copied here; skipped streams' previous pyramids are carried.
 int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch, bool semantic,
-                                  int level0_mode, bool stereo_now, long k, bool with_marks) {
+                                  int level0_mode, bool stereo_now, long k, bool with_marks, bool partial) {
     const int ph = (int)(k % 6), par = (int)(k % 2);
     auto mark = [&](int i) { if (with_marks) cudaEventRecord(ev[par][i], st); };
     DVFE_CUDA(cudaMemcpyAsync(d_dt, h_dt[par], B * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -370,6 +388,16 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
     // been read back before slot `par` is reused)
     DVFE_CUDA(cudaMemsetAsync(d_err + par, 0, sizeof(int), st));
     mark(0);
+    // One set of partial tables serves every step: all their readers run on this stream, before the next step rebuilds them.
+    if (partial) {
+        DVFE_CUDA(cudaMemcpyAsync(d_sflags, h_sflags[par], (size_t)B, cudaMemcpyHostToDevice, st));
+        PartialTables pt;
+        pt.full_temporal = d_groups[ph][0]; pt.full_stereo = d_groups[ph][2]; pt.full_jobs = d_jobs[ph][0];
+        pt.temporal = d_pgroups[0]; pt.stereo = d_pgroups[1]; pt.jobs = d_pjobs; pt.lane = d_lane;
+        pt.zero = d_zero; pt.n = bg.n; pt.next_id = d_next_id;
+        DVFE_CHECK(launch_partial_tables(pt, d_sflags, B, stereo_now ? 1 : 0, st));     // also RESET: n = 0, next_id = 1
+    }
+    const uint8_t* lane = partial ? d_lane : nullptr;
     // left pyramid now; the right pyramid is built on its own stream while the selection kernel (one CTA per
     // stream) leaves most SMs idle, and joins before the stereo LK
     PyrImgSet set;
@@ -377,21 +405,27 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
     set.dst[0] = left_slot(k); set.dst[1] = nullptr;
     set.src_stride = stream_stride; set.dst_stride = desc.bytes; set.per_set = B;
     DVFE_CHECK(launch_build_pyramids(set, B, desc, pitch, st, level0_mode));
+    // A skipped stream's "current" pyramid becomes its previous one again.  Nothing else touches either slot meanwhile: the
+    // upload of step k+1 writes slot (k+1) % 3, and the uploads (upload_*, the device-input copy in submit) wait for step k-2,
+    // the last reader of that slot, before they write it; slots k % 3 and (k+2) % 3 are read only by this step's kernels.
+    if (partial) DVFE_CHECK(launch_carry_pyramids(left_slot(k), left_slot(k + 2), desc.bytes, d_sflags, B, st));
     mark(ST_PYRAMID + 1);
     // The temporal call's backward templates (current left image at the tracked positions, levels <= its backward maxLevel)
     // are the stereo call's forward templates at those levels for the survivors: stored by the former, picked up through
     // the compaction's old-index map by the latter.
     const int site_t = semantic ? DVFE_LK_SEMANTIC_TEMPORAL : DVFE_LK_RAW_TEMPORAL;
     const bool reuse = use_reuse && k > 0 && stereo_now && cfg.flow_back && d_tcache_bwd != nullptr;
+    // in a partial step the table decides per stream whether its cache is read (tc_valid)
+    const bool tc_read = partial ? d_tcache != nullptr : tcache_valid;
     if (k > 0)   // bg.TrackLeft / FeatureTrackByLK(prev.gray0, gray0, last_points)
-        DVFE_CHECK(launch_lk(d_groups[ph][semantic ? 1 : 0], B, cap, cfg.lk_max_level, cfg.flow_back, st, lk_back_level[site_t],
-                             lk_fb_thresh[site_t], (tcache_valid ? LK_TCACHE_READ : 0) | (reuse ? LK_TCACHE_WRITE_BWD : 0)));
+        DVFE_CHECK(launch_lk(partial ? d_pgroups[0] : d_groups[ph][semantic ? 1 : 0], B, cap, cfg.lk_max_level, cfg.flow_back, st,
+                             lk_back_level[site_t], lk_fb_thresh[site_t], (tc_read ? LK_TCACHE_READ : 0) | (reuse ? LK_TCACHE_WRITE_BWD : 0)));
     mark(ST_LK_TEMPORAL + 1);
     if (k > 0)   // ReduceVector x4 + track_cnt++
-        DVFE_CHECK(launch_compact(bg, B, cap, st, nullptr, reuse ? d_old_idx : nullptr));
+        DVFE_CHECK(launch_compact(bg, B, cap, st, lane, reuse ? d_old_idx : nullptr));
     mark(ST_COMPACT + 1);
     // discs + goodFeaturesToTrack + ids
-    DVFE_CHECK(launch_gftt(d_jobs[ph][semantic ? (detect_cuda ? 2 : 1) : 0], nullptr, B, W, H, cap, st, with_marks ? &ev[par][ST_GFTT_MASK + 1] : nullptr,
+    DVFE_CHECK(launch_gftt(partial ? d_pjobs : d_jobs[ph][semantic ? (detect_cuda ? 2 : 1) : 0], nullptr, B, W, H, cap, st, with_marks ? &ev[par][ST_GFTT_MASK + 1] : nullptr,
                            stereo_now ? ev_resp[par] : nullptr, use_tma ? tmapL[k % 3] : nullptr,
                            (int)(desc.bytes / (unsigned)desc.lv[0].pitch)));
     if (stereo_now) {
@@ -405,22 +439,23 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
     }
     mark(ST_GFTT_SELECT + 1);
     // UndistortedPts(cam0) + PtsVelocity
-    DVFE_CHECK(launch_left_post(bg, B, cap, cam0, d_dt, nullptr, st));
+    DVFE_CHECK(launch_left_post(bg, B, cap, cam0, d_dt, nullptr, st, lane));
     mark(ST_LEFT_POST + 1);
     if (stereo_now) DVFE_CUDA(cudaStreamWaitEvent(st, ev_rpyr[par], 0));
     if (stereo_now)   // FeatureTrackByLK(gray0, gray1, curr_points) — left points are kept when the match fails
-        DVFE_CHECK(launch_lk(d_groups[ph][2], B, cap, cfg.lk_max_level, cfg.flow_back, st,
+        DVFE_CHECK(launch_lk(partial ? d_pgroups[1] : d_groups[ph][2], B, cap, cfg.lk_max_level, cfg.flow_back, st,
                              lk_back_level[semantic ? DVFE_LK_SEMANTIC_STEREO : DVFE_LK_RAW_STEREO],
                              lk_fb_thresh[semantic ? DVFE_LK_SEMANTIC_STEREO : DVFE_LK_RAW_STEREO],
                              LK_TCACHE_WRITE | (reuse ? LK_TCACHE_READ_BWD : 0), reuse ? lk_back_level[site_t] : -1));
     mark(ST_LK_STEREO + 1);
-    DVFE_CHECK(launch_right_post_pack(bg, B, cap, cam1, d_dt, stereo_now ? 1 : 0, d_obs[par], d_nobs[par], st));
+    DVFE_CHECK(launch_right_post_pack(bg, B, cap, cam1, d_dt, stereo_now ? 1 : 0, d_obs[par], d_nobs[par], st, lane));
     mark(ST_PACK + 1);
     return DVFE_OK;
 }
 
 // Capture and instantiate the graph of the step with buffer phase `ph` and mode `flags` (bit 0 semantic, 2 stereo, 3 not the first
-// frame, 4 forward templates cached, 5 level 0 arrives with its border); `k` = any frame index with k % 6 == ph and (k > 0) as in the flags.  Nothing runs.
+// frame, 4 forward templates cached, 5 level 0 arrives with its border, 6 partial: per-stream flags, bit 4 unused); `k` = any frame
+// index with k % 6 == ph and (k > 0) as in the flags.  Nothing runs.
 int dvfe_tracker::capture_step(int ph, unsigned flags, long k) {
     const unsigned long long before = g_dvfe_launches;
     const bool keep_valid = tcache_valid;
@@ -428,7 +463,7 @@ int dvfe_tracker::capture_step(int ph, unsigned flags, long k) {
     cudaGraph_t g = nullptr;
     DVFE_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
     const int rc = enqueue_compute(nullptr, nullptr, 0, 0, (flags & 1u) != 0, (flags & 32u) ? DVFE_L0_COMPLETE : DVFE_L0_INTERIOR,
-                                   (flags & 4u) != 0, k, false);
+                                   (flags & 4u) != 0, k, false, (flags & 64u) != 0);
     const cudaError_t ce = cudaStreamEndCapture(st, &g);
     tcache_valid = keep_valid;
     const unsigned n_kernels = (unsigned)(g_dvfe_launches - before);
@@ -449,11 +484,20 @@ int dvfe_tracker::capture_step(int ph, unsigned flags, long k) {
 }
 
 int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch,
-                         const double* time0, bool semantic, bool level0_in_place, bool has_right) {
+                         const double* time0, bool semantic, bool level0_in_place, bool has_right, const uint8_t* sflags) {
     const long k = frames;
     const int ph = (int)(k % 6), par = (int)(k % 2);
     const bool stereo_now = cfg.stereo && (d_right != nullptr || (level0_in_place && has_right));
-    for (int s = 0; s < B; s++) h_dt[par][s] = time0[s] - prev_time[s];       // cur_time - prev_time
+    const bool partial = sflags != nullptr;
+    if (partial) {
+        for (int s = 0; s < B; s++) {
+            if (sflags[s] & DVFE_FRAME_RESET) prev_time[s] = 0.0;                  // a new tracker's prev_time
+            h_dt[par][s] = (sflags[s] & DVFE_FRAME_SKIP) ? 0.0 : time0[s] - prev_time[s];
+            h_sflags[par][s] = (uint8_t)(sflags[s] | (tc_valid[s] ? SF_TCACHE_VALID : 0u));
+        }
+    } else {
+        for (int s = 0; s < B; s++) h_dt[par][s] = time0[s] - prev_time[s];       // cur_time - prev_time
+    }
     prof_step[par] = prof;
     // everything step k-1 (background and instances) put on the compute stream lies before this point
     DVFE_CUDA(cudaEventRecord(ev_begin[par], st));
@@ -479,7 +523,8 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
         }
         // level 0 copied by the kernel above arrives with its border; DMA / ingest kernels leave the border to the graph
         const bool l0_complete = !level0_in_place && pyr_level0_writes_border(desc);
-        const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (k > 0 ? 8u : 0u) | (tcache_valid ? 16u : 0u) | (l0_complete ? 32u : 0u);
+        const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (k > 0 ? 8u : 0u) | (tcache_valid && !partial ? 16u : 0u) |
+                               (l0_complete ? 32u : 0u) | (partial ? 64u : 0u);
         const StepKey key(ph, flags);
         if (step_graphs.find(key) == step_graphs.end()) {
             if (step_graphs.size() >= 64) drop_graphs();          // a caller cycling through many modes
@@ -487,7 +532,8 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
             // The first step of a mode also captures the six steady-state graphs it will replay from the next frame on (one per
             // buffer phase), so that instantiation (host time, ~0.3 ms each) never falls into a later, possibly timed, step.
             const bool tc_next = stereo_now && d_tcache != nullptr;
-            const unsigned steady = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | 8u | (tc_next ? 16u : 0u) | (l0_complete ? 32u : 0u);
+            const unsigned steady = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | 8u | (tc_next && !partial ? 16u : 0u) |
+                                    (l0_complete ? 32u : 0u) | (partial ? 64u : 0u);
             for (int p = 0; p < 6; p++)
                 if (step_graphs.find(StepKey(p, steady)) == step_graphs.end()) DVFE_CHECK(capture_step(p, steady, 6 + p));
         }
@@ -496,9 +542,22 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
         g_dvfe_launches += it->second.n_kernels;
     } else {
         DVFE_CHECK(enqueue_compute(d_left, d_right, stream_stride, pitch, semantic, level0_in_place ? DVFE_L0_INTERIOR : DVFE_L0_BUILD,
-                                   stereo_now, k, prof));
+                                   stereo_now, k, prof, partial));
     }
-    tcache_valid = stereo_now && d_tcache != nullptr;
+    // Template-cache validity per stream: a present frame with a stereo step leaves the templates of its points, a frame without
+    // one leaves none (a RESET frame's points are all new), a skipped stream keeps what it had.  A full step reads the cache of
+    // every stream or of none, so it reads it only when every stream's is valid.
+    if (partial) {
+        bool all = true;
+        for (int s = 0; s < B; s++) {
+            if (!(sflags[s] & DVFE_FRAME_SKIP)) tc_valid[s] = stereo_now && d_tcache != nullptr && !(sflags[s] & DVFE_FRAME_NO_RIGHT);
+            all = all && tc_valid[s];
+        }
+        tcache_valid = all;
+    } else {
+        tcache_valid = stereo_now && d_tcache != nullptr;
+        tc_valid.assign(B, tcache_valid ? 1 : 0);
+    }
     // records go home on the download stream so that the next step's kernels do not queue behind the copy
     DVFE_CUDA(cudaEventRecord(ev_packed[par], st));
     DVFE_CUDA(cudaStreamWaitEvent(ds, ev_packed[par], 0));
@@ -507,7 +566,8 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
     DVFE_CUDA(cudaMemcpyAsync(h_obs[par], d_obs[par], (size_t)B * 2 * cap * sizeof(dvfe_obs), cudaMemcpyDeviceToHost, ds));
     if (prof) cudaEventRecord(ev[par][ST_D2H + 1], ds);
     DVFE_CUDA(cudaEventRecord(ev_done[par], ds));
-    for (int s = 0; s < B; s++) prev_time[s] = time0[s];
+    for (int s = 0; s < B; s++)
+        if (!partial || !(sflags[s] & DVFE_FRAME_SKIP)) prev_time[s] = time0[s];
     last_has_right = stereo_now;
     frames++;
     return DVFE_OK;
@@ -687,24 +747,43 @@ static int check_step_args(dvfe_tracker* t, const uint8_t* left, int pitch, cons
     return DVFE_OK;
 }
 
-extern "C" int dvfe_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride,
-                                      int pitch, const double* time0) {
-    DVFE_CHECK(check_step_args(t, left, pitch, time0));
-    if (IS_GROUP(t)) return grp_track_image_async(t, left, right, stream_stride, pitch, time0, false);
+// the raw step of a leaf tracker from host images, enqueued; sflags: per-stream DVFE_FRAME_* (validated) or null
+static int leaf_track_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
+                            const double* time0, const uint8_t* sflags) {
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
     if (t->prep_active()) {
         DVFE_CHECK(t->upload_prepared(left, right, stream_stride, pitch));
-        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr);
+        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr, sflags);
     }
     if (t->staged_upload) {
         const size_t P = (size_t)t->W * t->H;
         const int par = (int)(t->frames % 2);
         DVFE_CHECK(t->upload_staged(left, right, stream_stride, pitch));
         return t->submit(t->d_stage[par], right ? t->d_stage[par] + t->B * P : nullptr, P, t->W, time0, false, false,
-                         right != nullptr);
+                         right != nullptr, sflags);
     }
     DVFE_CHECK(t->upload_in_place(left, right, stream_stride, pitch));
-    return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr);
+    return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr, sflags);
+}
+
+// the same from device-resident images
+static int leaf_track_device_async(dvfe_tracker* t, const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch,
+                                   const double* time0, const uint8_t* sflags) {
+    DVFE_CUDA(cudaSetDevice(t->cfg.device));
+    while (t->frames - t->completed >= 2) DVFE_CHECK(t->wait_one());
+    if (t->prep_active()) {
+        DVFE_CHECK(t->ingest(d_left, stream_stride, pitch, 0, t->st));
+        if (d_right) DVFE_CHECK(t->ingest(d_right, stream_stride, pitch, 1, t->st));
+        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, d_right != nullptr, sflags);
+    }
+    return t->submit(d_left, d_right, stream_stride, pitch, time0, false, false, d_right != nullptr, sflags);
+}
+
+extern "C" int dvfe_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride,
+                                      int pitch, const double* time0) {
+    DVFE_CHECK(check_step_args(t, left, pitch, time0));
+    if (IS_GROUP(t)) return grp_track_image_async(t, left, right, stream_stride, pitch, time0, false);
+    return leaf_track_async(t, left, right, stream_stride, pitch, time0, nullptr);
 }
 
 extern "C" int dvfe_wait(dvfe_tracker* t) {
@@ -744,14 +823,29 @@ extern "C" int dvfe_track_image_device_async(dvfe_tracker* t, const uint8_t* d_l
                                              size_t stream_stride, int pitch, const double* time0) {
     DVFE_CHECK(check_step_args(t, d_left, pitch, time0));
     if (IS_GROUP(t)) return grp_track_image_async(t, d_left, d_right, stream_stride, pitch, time0, true);
-    DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    while (t->frames - t->completed >= 2) DVFE_CHECK(t->wait_one());
-    if (t->prep_active()) {
-        DVFE_CHECK(t->ingest(d_left, stream_stride, pitch, 0, t->st));
-        if (d_right) DVFE_CHECK(t->ingest(d_right, stream_stride, pitch, 1, t->st));
-        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, d_right != nullptr);
-    }
-    return t->submit(d_left, d_right, stream_stride, pitch, time0, false, false, d_right != nullptr);
+    return leaf_track_device_async(t, d_left, d_right, stream_stride, pitch, time0, nullptr);
+}
+
+extern "C" int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
+                                   const double* time0, const uint8_t* stream_flags, unsigned flags) {
+    DVFE_CHECK(check_step_args(t, left, pitch, time0));
+    if (flags & ~DVFE_STEP_DEVICE_INPUT) { dvfe_set_error("track_image_ex: unknown flags 0x%x", flags); return DVFE_ERR_INVALID; }
+    const bool device = (flags & DVFE_STEP_DEVICE_INPUT) != 0;
+    bool any = false;
+    if (stream_flags)
+        for (int s = 0; s < t->B; s++) {
+            const unsigned f = stream_flags[s];
+            if ((f & ~(DVFE_FRAME_SKIP | DVFE_FRAME_NO_RIGHT | DVFE_FRAME_RESET)) ||
+                (f & (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) == (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) {
+                dvfe_set_error("track_image_ex: stream %d: invalid stream flags 0x%x", s, f);
+                return DVFE_ERR_INVALID;
+            }
+            any = any || f != 0;
+        }
+    const uint8_t* sf = any ? stream_flags : nullptr;          // no flag set: exactly the step of the plain entry points
+    if (IS_GROUP(t)) return grp_track_image_ex(t, left, right, stream_stride, pitch, time0, sf, device);
+    return device ? leaf_track_device_async(t, left, right, stream_stride, pitch, time0, sf)
+                  : leaf_track_async(t, left, right, stream_stride, pitch, time0, sf);
 }
 
 extern "C" int dvfe_set_lk_mode_site(dvfe_tracker* t, int site, int back_max_level, double fb_threshold) {
@@ -907,6 +1001,7 @@ extern "C" int dvfe_set_state(dvfe_tracker* t, int stream, const dvfe_state* stt
     DVFE_CUDA(cudaMemcpy(t->d_next_id + stream, &stt->next_id, sizeof(uint32_t), cudaMemcpyHostToDevice));
     t->prev_time[stream] = stt->prev_time;
     t->tcache_valid = false;                 // the cached templates belong to the points that were just replaced
+    t->tc_valid[stream] = 0;
     if (n > 0) {
         DVFE_CUDA(cudaMemcpy(t->bg.ids + o, stt->ids, n * sizeof(uint32_t), cudaMemcpyHostToDevice));
         DVFE_CUDA(cudaMemcpy(t->bg.track_cnt + o, stt->track_cnt, n * sizeof(int32_t), cudaMemcpyHostToDevice));

@@ -72,6 +72,15 @@ struct dvfe_tracker {
     bool tcache_valid = false;                       // the last step ran the stereo LK on the points `bg` holds now
     unsigned* d_tcache_bwd = nullptr;                // backward templates of the temporal call, same layout (stereo only)
     int* d_old_idx = nullptr;                        // [B][cap] index of each point in the temporal call of the step, -1 = new
+    // Per-stream frame presence (dvfe_track_image_ex).  A "partial" step (any stream flag set) runs the same kernels on tables
+    // rebuilt from the stream flags at its start; steps without flags never touch any of this.
+    uint8_t* h_sflags[2] = {nullptr, nullptr};       // pinned [B] per in-flight step: DVFE_FRAME_* | SF_TCACHE_VALID
+    uint8_t* d_sflags = nullptr;                     // [B] the flags of the step on the compute stream
+    uint8_t* d_lane = nullptr;                       // [B] 0 = skipped, else LANE_PRESENT | LANE_STEREO (compact, left/right post)
+    LkGroup* d_pgroups[2] = {nullptr, nullptr};      // [B] partial temporal / stereo LK tables
+    GfttJob* d_pjobs = nullptr;                      // [B] partial GFTT jobs
+    int* d_zero = nullptr;                           // the point count of a stream an LK table leaves out
+    std::vector<uint8_t> tc_valid;                   // per stream: d_tcache holds the forward templates of its current points
     // backward LK maxLevel / forward-backward threshold per call site [DVFE_LK_*]: the CPU FeatureTrackByLK pair
     // (feature_utils.cpp:51,57: 1, 0.5) everywhere except TrackSemanticImage's right image, which the reference tracks with
     // the cv::cuda call pattern (TrackRightGPU, background_tracker.cpp:801: 3 levels, 1.0 px)
@@ -89,7 +98,7 @@ struct dvfe_tracker {
     void drop_graphs();
     int capture_step(int ph, unsigned flags, long k);
     int enqueue_compute(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch, bool semantic,
-                        int level0_mode, bool stereo_now, long k, bool with_marks);
+                        int level0_mode, bool stereo_now, long k, bool with_marks, bool partial = false);
 
     // per-stage device timers (one event set per in-flight step)
     enum { ST_PYRAMID, ST_LK_TEMPORAL, ST_COMPACT, ST_GFTT_MASK, ST_GFTT_DISCS, ST_GFTT_RESPONSE, ST_GFTT_SELECT, ST_LEFT_POST,
@@ -125,8 +134,9 @@ struct dvfe_tracker {
     int upload_in_place(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch);
     int upload_staged(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch);
     // enqueue one frame step (no host synchronisation); at most two steps are in flight
+    // sflags (nullable): per-stream DVFE_FRAME_* of a raw step (dvfe_track_image_ex), already validated
     int submit(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch, const double* time0,
-               bool semantic, bool level0_in_place, bool has_right);
+               bool semantic, bool level0_in_place, bool has_right, const uint8_t* sflags = nullptr);
     // TrackSemanticImage of one frame, enqueued only (uploads on the copy stream, mask erosion + the frame step)
     // flags: DVFE_DYN_DEVICE_INPUT (the three pointers are device memory, nothing is uploaded), DVFE_DYN_LABELS (the mask is a
     // label image: the region is everything no instance bit is set on)

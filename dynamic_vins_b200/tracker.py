@@ -125,22 +125,44 @@ class BatchTracker:
             assert m1.shape == (self.H, self.W, 2) and m2.shape == (self.H, self.W)
         L.check(L.lib().dvfe_set_undistort_maps(self._h, cam, L.ptr(m1), L.ptr(m2)))
 
-    def track_image(self, left: np.ndarray, right: Optional[np.ndarray], time0) -> None:
-        """left/right: (B,H,W) or (H,W) uint8 host arrays."""
+    def _stream_flags(self, stream_flags) -> Optional[np.ndarray]:
+        """per-stream L.FRAME_* bytes of dvfe_track_image_ex (None: the plain entry points)"""
+        if stream_flags is None:
+            return None
+        f = np.ascontiguousarray(stream_flags, np.uint8)
+        if f.shape != (self.B,):
+            raise ValueError(f"stream_flags: one flag byte per stream expected ({self.B}), got shape {f.shape}")
+        return f
+
+    def track_image(self, left: np.ndarray, right: Optional[np.ndarray], time0, stream_flags=None) -> None:
+        """left/right: (B,H,W) or (H,W) uint8 host arrays.  stream_flags: None, or B bytes of FRAME_SKIP / FRAME_NO_RIGHT /
+        FRAME_RESET (per-stream frame presence, include/dvfe.h dvfe_track_image_ex)."""
         self._leave_naive()
+        f = self._stream_flags(stream_flags)
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
-        L.check(L.lib().dvfe_track_image(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
+        if f is None:
+            L.check(L.lib().dvfe_track_image(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
+            return
+        L.check(L.lib().dvfe_track_image_ex(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t),
+                                            L.ptr(f), 0))
+        self.wait()          # at most two steps are in flight: the second wait returns at once unless an earlier async step was
+        self.wait()          # still pending, and then completes this one
 
-    def track_image_async(self, left: np.ndarray, right: Optional[np.ndarray], time0) -> None:
+    def track_image_async(self, left: np.ndarray, right: Optional[np.ndarray], time0, stream_flags=None) -> None:
         """pipelined: enqueue the step and return; the arrays must stay alive until the matching wait()"""
         self._leave_naive()
+        f = self._stream_flags(stream_flags)
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
         self._keep = (l, r, t, getattr(self, "_keep", None) and self._keep[:3])
-        L.check(L.lib().dvfe_track_image_async(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
+        if f is None:
+            L.check(L.lib().dvfe_track_image_async(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
+            return
+        L.check(L.lib().dvfe_track_image_ex(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t),
+                                            L.ptr(f), 0))
 
     def wait(self) -> None:
         """block until the oldest in-flight step is finished; features() then returns its records"""
@@ -153,12 +175,18 @@ class BatchTracker:
         L.check(L.lib().dvfe_track_image_device(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
                                                 stream_stride, pitch, L.ptr(t)))
 
-    def track_image_device_async(self, d_left: int, d_right: int, stream_stride: int, pitch: int, time0) -> None:
+    def track_image_device_async(self, d_left: int, d_right: int, stream_stride: int, pitch: int, time0,
+                                 stream_flags=None) -> None:
         self._leave_naive()
+        f = self._stream_flags(stream_flags)
         t = self._times(time0)
         self._keep_t = (t, getattr(self, "_keep_t", (None,))[0])
-        L.check(L.lib().dvfe_track_image_device_async(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
-                                                      stream_stride, pitch, L.ptr(t)))
+        if f is None:
+            L.check(L.lib().dvfe_track_image_device_async(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
+                                                          stream_stride, pitch, L.ptr(t)))
+            return
+        L.check(L.lib().dvfe_track_image_ex(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
+                                            stream_stride, pitch, L.ptr(t), L.ptr(f), L.STEP_DEVICE_INPUT))
 
     LK_RAW_TEMPORAL, LK_RAW_STEREO, LK_SEMANTIC_TEMPORAL, LK_SEMANTIC_STEREO = 0, 1, 2, 3
 

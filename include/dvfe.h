@@ -161,6 +161,27 @@ int dvfe_track_image_device(dvfe_tracker* t, const uint8_t* d_left, const uint8_
 int dvfe_track_image_device_async(dvfe_tracker* t, const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride,
                                   int pitch, const double* time0);
 
+/* Per-stream frame presence: one TrackImage step (enqueued, pair with dvfe_wait) in which every stream s gets exactly what a
+ * single-stream tracker fed only that stream's frames would get.  stream_flags[s] (NULL = all 0):
+ *   0                    the stream's frame as dvfe_track_image_async / dvfe_track_image_device_async (same graph, same launches
+ *                        when every flag is 0)
+ *   DVFE_FRAME_SKIP      no frame for this stream: FeatureTracker::TrackImage is not called.  Points, ids, next_id, track_cnt,
+ *                        both velocity maps, prev_time and the previous-frame pyramid stay as they were; dvfe_get_features
+ *                        returns 0 records; time0[s] is not read (NaN is fine)
+ *   DVFE_FRAME_NO_RIGHT  left image only (TrackImage with an empty gray1, background_tracker.cpp:107): left points kept, no
+ *                        cam-1 records, right_prev_* unchanged
+ *   DVFE_FRAME_RESET     the stream starts over: before the frame it gets the state of a newly created tracker (n = 0,
+ *                        next_id = 1, prev_time = 0) and the frame runs as a first frame; may be combined with NO_RIGHT
+ * Unknown bits, SKIP|RESET and unknown `flags` bits return DVFE_ERR_INVALID and change nothing.  With right != NULL all B
+ * slots of both images must be readable; the pixels of a skipped stream, and of a NO_RIGHT stream's right image, affect no
+ * result.  right == NULL makes every stream mono.  flags: DVFE_STEP_DEVICE_INPUT = left / right are device pointers. */
+#define DVFE_FRAME_SKIP 1u
+#define DVFE_FRAME_NO_RIGHT 2u
+#define DVFE_FRAME_RESET 4u
+#define DVFE_STEP_DEVICE_INPUT 1u
+int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
+                        const double* time0, const uint8_t* stream_flags, unsigned flags);
+
 /* Backward-pass depth and forward-backward threshold of the LK at each of the reference's four call sites.  The
  * reference uses two pairs: the CPU FeatureTrackByLK (front_end/feature_utils.cpp:35-69: backward maxLevel 1, round
  * trip <= 0.5 px) and the cv::cuda call pattern of FeatureTrackByLKGpu (:83-163 with the objects created at

@@ -428,6 +428,16 @@ public:
         if (dvfe_track_image_async(h_, left, right, stream_stride, step, time0.data()) != DVFE_OK)
             throw std::runtime_error(dvfe_last_error(h_));
     }
+    // The same with per-stream frame presence: stream_flags[s] is 0 or DVFE_FRAME_SKIP / DVFE_FRAME_NO_RIGHT / DVFE_FRAME_RESET
+    // (dvfe_track_image_ex); a skipped stream's time0 is not read.  `device`: left / right are device pointers.
+    void TrackImageAsync(const uint8_t* left, const uint8_t* right, size_t stream_stride, int step, const std::vector<double>& time0,
+                         const std::vector<uint8_t>& stream_flags, bool device = false) {
+        check(time0);
+        if ((int)stream_flags.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one stream flag per stream expected");
+        if (dvfe_track_image_ex(h_, left, right, stream_stride, step, time0.data(), stream_flags.data(),
+                                device ? DVFE_STEP_DEVICE_INPUT : 0u) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
     // TrackSemanticImage + InstsTrack of all cameras, enqueued (dynamic mode; FeatureTrack() in system/main.cpp:247-254)
     void TrackDynamicAsync(const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask, size_t stream_stride, int step,
                            const std::vector<int>& exist_inst, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,

@@ -49,18 +49,6 @@ static int grp_of(const dvfe_tracker* t, int stream, int* local) {
     return -1;
 }
 
-int grp_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
-                          const double* time0, bool device) {
-    for (size_t g = 0; g < t->groups.size(); g++) {
-        const size_t off = (size_t)t->group_first[g] * stride;
-        const uint8_t* l = left + off;
-        const uint8_t* r = right ? right + off : nullptr;
-        DVFE_CHECK(device ? dvfe_track_image_device_async(t->groups[g], l, r, stride, pitch, time0 + t->group_first[g])
-                          : dvfe_track_image_async(t->groups[g], l, r, stride, pitch, time0 + t->group_first[g]));
-    }
-    return DVFE_OK;
-}
-
 // every group submits a step, also one whose streams are all skipped, so that each dvfe_wait still pairs with one step per group
 int grp_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
                        const double* time0, const uint8_t* stream_flags, bool device) {

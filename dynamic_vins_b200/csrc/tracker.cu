@@ -33,8 +33,6 @@ void dvfe_set_error(const char* fmt, ...) {
 // groups.cu
 int grp_create(const dvfe_config* cfg, dvfe_tracker** out);
 void grp_destroy(dvfe_tracker* t);
-int grp_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
-                          const double* time0, bool device);
 int grp_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stride, int pitch,
                        const double* time0, const uint8_t* stream_flags, bool device);
 int grp_wait(dvfe_tracker* t);
@@ -240,11 +238,9 @@ int dvfe_tracker::init() {
     // pitched host->device DMA straight into the padded level 0 runs at full PCIe rate only for rows that are a
     // multiple of 64 bytes; other widths go through a dense staging buffer (one linear copy) and the copy kernel
     staged_upload = (W % 64) != 0;
-    if (const char* e = getenv("DVFE_STAGED_UPLOAD")) staged_upload = atoi(e) != 0;      // experiment / override
     if (const char* e = getenv("DVFE_GRAPHS")) use_graphs = atoi(e) != 0;                // A/B: 0 = plain launches
     if (const char* e = getenv("DVFE_REUSE")) use_reuse = atoi(e) != 0;
-    if (staged_upload)
-        for (int p = 0; p < 2; p++) DVFE_CHECK(dmalloc(&d_stage[p], 2 * B * P));
+    DVFE_CHECK(size_stage());
 
     if (cfg.stereo) {
         DVFE_CHECK(dmalloc(&d_tcache, (size_t)B * cap * DVFE_MAX_PYR_LEVELS * LK_TCACHE_WORDS));
@@ -343,8 +339,7 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
         if (t->ev_done[p]) cudaEventDestroy(t->ev_done[p]);
         for (int i = 0; i <= dvfe_tracker::ST_COUNT; i++) if (t->ev[p][i]) cudaEventDestroy(t->ev[p][i]);
     }
-    cudaFree(t->d_stage[0]); cudaFree(t->d_stage[1]);
-    for (int i = 0; i < 2; i++) { cudaFree(t->d_raw[i]); cudaFree(t->d_map1[i]); cudaFree(t->d_map2[i]); }
+    for (int i = 0; i < 2; i++) { cudaFree(t->d_stage[i]); cudaFree(t->d_map1[i]); cudaFree(t->d_map2[i]); }
     cudaFree(t->d_region); cudaFree(t->d_region_tmp); cudaFree(t->d_exist);
     for (int p = 0; p < 2; p++) {
         cudaFree(t->d_labels[p]);
@@ -406,7 +401,7 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
     set.src_stride = stream_stride; set.dst_stride = desc.bytes; set.per_set = B;
     DVFE_CHECK(launch_build_pyramids(set, B, desc, pitch, st, level0_mode));
     // A skipped stream's "current" pyramid becomes its previous one again.  Nothing else touches either slot meanwhile: the
-    // upload of step k+1 writes slot (k+1) % 3, and the uploads (upload_*, the device-input copy in submit) wait for step k-2,
+    // upload of step k+1 writes slot (k+1) % 3, and the uploads (place_input, the device-input copy in submit) wait for step k-2,
     // the last reader of that slot, before they write it; slots k % 3 and (k+2) % 3 are read only by this step's kernels.
     if (partial) DVFE_CHECK(launch_carry_pyramids(left_slot(k), left_slot(k + 2), desc.bytes, d_sflags, B, st));
     mark(ST_PYRAMID + 1);
@@ -483,11 +478,10 @@ int dvfe_tracker::capture_step(int ph, unsigned flags, long k) {
     return DVFE_OK;
 }
 
-int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch,
-                         const double* time0, bool semantic, bool level0_in_place, bool has_right, const uint8_t* sflags) {
+int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic, const uint8_t* sflags) {
     const long k = frames;
     const int ph = (int)(k % 6), par = (int)(k % 2);
-    const bool stereo_now = cfg.stereo && (d_right != nullptr || (level0_in_place && has_right));
+    const bool stereo_now = cfg.stereo && in.has_right;
     const bool partial = sflags != nullptr;
     if (partial) {
         for (int s = 0; s < B; s++) {
@@ -505,24 +499,24 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
         // The captured step never sees the caller's image pointers: device-resident input is copied into level 0 here,
         // left on the compute stream, right on its own stream behind the last readers of that slot (the stereo LKs of step
         // k-2, all of which precede the start of step k-1), and the graph runs as if level 0 had arrived in place.
-        if (!level0_in_place) {
+        if (!in.in_place) {
             PyrImgSet set;
-            set.src[0] = d_left; set.src[1] = nullptr; set.dst[0] = left_slot(k); set.dst[1] = nullptr;
-            set.src_stride = stream_stride; set.dst_stride = desc.bytes; set.per_set = B;
-            DVFE_CHECK(launch_pyr_level0(set, B, desc, pitch, st));
+            set.src[0] = in.left; set.src[1] = nullptr; set.dst[0] = left_slot(k); set.dst[1] = nullptr;
+            set.src_stride = in.stride; set.dst_stride = desc.bytes; set.per_set = B;
+            DVFE_CHECK(launch_pyr_level0(set, B, desc, in.pitch, st));
             if (stereo_now) {
-                set.src[0] = d_right; set.dst[0] = right_slot(k);
+                set.src[0] = in.right; set.dst[0] = right_slot(k);
                 if (k >= 1) DVFE_CUDA(cudaStreamWaitEvent(rs, ev_begin[1 - par], 0));
                 // ... and behind the upload of this step when the source is the tracker's own staging buffer (widths whose rows
                 // are not a multiple of 64 bytes); for caller-resident images the event is an old, completed one
                 DVFE_CUDA(cudaStreamWaitEvent(rs, ev_up[par], 0));
-                DVFE_CHECK(launch_pyr_level0(set, B, desc, pitch, rs));
+                DVFE_CHECK(launch_pyr_level0(set, B, desc, in.pitch, rs));
                 DVFE_CUDA(cudaEventRecord(ev_r0[par], rs));
                 DVFE_CUDA(cudaStreamWaitEvent(st, ev_r0[par], 0));
             }
         }
         // level 0 copied by the kernel above arrives with its border; DMA / ingest kernels leave the border to the graph
-        const bool l0_complete = !level0_in_place && pyr_level0_writes_border(desc);
+        const bool l0_complete = !in.in_place && pyr_level0_writes_border(desc);
         const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (k > 0 ? 8u : 0u) | (tcache_valid && !partial ? 16u : 0u) |
                                (l0_complete ? 32u : 0u) | (partial ? 64u : 0u);
         const StepKey key(ph, flags);
@@ -541,7 +535,7 @@ int dvfe_tracker::submit(const uint8_t* d_left, const uint8_t* d_right, size_t s
         DVFE_CUDA(cudaGraphLaunch(it->second.exec, st));
         g_dvfe_launches += it->second.n_kernels;
     } else {
-        DVFE_CHECK(enqueue_compute(d_left, d_right, stream_stride, pitch, semantic, level0_in_place ? DVFE_L0_INTERIOR : DVFE_L0_BUILD,
+        DVFE_CHECK(enqueue_compute(in.left, in.right, in.stride, in.pitch, semantic, in.in_place ? DVFE_L0_INTERIOR : DVFE_L0_BUILD,
                                    stereo_now, k, prof, partial));
     }
     // Template-cache validity per stream: a present frame with a stereo step leaves the templates of its points, a frame without
@@ -604,104 +598,105 @@ int dvfe_tracker::wait_all() {
     return DVFE_OK;
 }
 
-// Host images -> level 0 of the pyramids of the NEXT step, one pitched 3-D copy per camera on the upload stream
-// (no staging buffer, no copy kernel).  The target slots were last read two steps ago.
-int dvfe_tracker::upload_in_place(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch) {
-    const long k = frames;
-    const int par = (int)(k % 2);
-    while (frames - completed >= 2) DVFE_CHECK(wait_one());      // slot reuse: step k-2 must be finished
-    const PyrLevel& L0 = desc.lv[0];
-    const size_t inner = L0.offset + (size_t)DVFE_PADY * L0.pitch + DVFE_PADX;
-    for (int cam = 0; cam < 2; cam++) {
-        const uint8_t* src = cam ? right : left;
-        if (!src) continue;
-        uint8_t* dst = (cam ? right_slot(k) : left_slot(k)) + inner;
-        if (stream_stride % (size_t)pitch == 0) {
-            cudaMemcpy3DParms p;
-            memset(&p, 0, sizeof(p));
-            p.srcPtr = make_cudaPitchedPtr((void*)src, (size_t)pitch, (size_t)W, stream_stride / (size_t)pitch);
-            p.dstPtr = make_cudaPitchedPtr((void*)dst, (size_t)L0.pitch, (size_t)W, desc.bytes / (size_t)L0.pitch);
-            p.extent = make_cudaExtent((size_t)W, (size_t)H, (size_t)B);
-            p.kind = cudaMemcpyHostToDevice;
-            DVFE_CUDA(cudaMemcpy3DAsync(&p, cs));
-        } else {
-            for (int s = 0; s < B; s++)
-                DVFE_CUDA(cudaMemcpy2DAsync(dst + (size_t)s * desc.bytes, L0.pitch, src + s * stream_stride, pitch, W,
-                                            (size_t)H, cudaMemcpyHostToDevice, cs));
-        }
-    }
-    DVFE_CUDA(cudaEventRecord(ev_up[par], cs));
-    DVFE_CUDA(cudaStreamWaitEvent(st, ev_up[par], 0));
-    return DVFE_OK;
-}
-
-// Host images -> dense device staging of the NEXT step (upload stream); the copy kernel then builds level 0.
-int dvfe_tracker::upload_staged(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch) {
-    const long k = frames;
-    const int par = (int)(k % 2);
+int dvfe_tracker::wait_slot() {
     while (frames - completed >= 2) DVFE_CHECK(wait_one());
-    const size_t P = (size_t)W * H;
-    for (int cam = 0; cam < 2; cam++) {
-        const uint8_t* src = cam ? right : left;
-        if (!src) continue;
-        uint8_t* dst = d_stage[par] + (size_t)cam * B * P;
-        if (pitch == W && stream_stride == P) {
-            DVFE_CUDA(cudaMemcpyAsync(dst, src, (size_t)B * P, cudaMemcpyHostToDevice, cs));
-        } else {
-            for (int s = 0; s < B; s++)
-                DVFE_CUDA(cudaMemcpy2DAsync(dst + (size_t)s * P, W, src + s * stream_stride, pitch, W, (size_t)H,
-                                            cudaMemcpyHostToDevice, cs));
-        }
-    }
-    DVFE_CUDA(cudaEventRecord(ev_up[par], cs));
-    DVFE_CUDA(cudaStreamWaitEvent(st, ev_up[par], 0));
     return DVFE_OK;
 }
 
-// ---- frame ingest: BGR and/or distorted input -> level 0 on the device ---------------------------------------------
-int dvfe_tracker::ensure_raw() {
-    const size_t need = (size_t)2 * B * W * H * in_ch;
-    for (int p = 0; p < 2; p++) {
-        if (d_raw[p]) continue;
-        DVFE_CUDA(cudaMalloc((void**)&d_raw[p], need));
-    }
-    return DVFE_OK;
+// ---- the step's input: host or device images -> where the step reads them ---------------------------------------------
+uint8_t* dvfe_tracker::level0(int cam) const {
+    const PyrLevel& L0 = desc.lv[0];
+    return (cam ? right_slot(frames) : left_slot(frames)) + L0.offset + (size_t)DVFE_PADY * L0.pitch + DVFE_PADX;
 }
 
 // remap (if camera `cam` has maps) + gray conversion of B device images into level 0 of this step's pyramid slot
 int dvfe_tracker::ingest(const uint8_t* d_src, size_t stream_stride, int pitch, int cam, cudaStream_t s) {
-    const PyrLevel& L0 = desc.lv[0];
     IngestArgs a;
     a.src = d_src; a.src_stride = stream_stride; a.src_pitch = pitch; a.ch = in_ch;
     a.map1 = d_map1[cam]; a.map2 = d_map2[cam];
-    a.dst = (cam ? right_slot(frames) : left_slot(frames)) + L0.offset + (size_t)DVFE_PADY * L0.pitch + DVFE_PADX;
-    a.dst_stride = desc.bytes; a.dst_pitch = L0.pitch;
+    a.dst = level0(cam);
+    a.dst_stride = desc.bytes; a.dst_pitch = desc.lv[0].pitch;
     a.w = W; a.h = H; a.n_img = B; a.keep_channels = 0;
     return launch_ingest(a, s);
 }
 
-// Host images (gray or BGR) -> dense device staging -> ingest kernel on the upload stream -> level 0 of the NEXT step
-int dvfe_tracker::upload_prepared(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch) {
-    const long k = frames;
-    const int par = (int)(k % 2);
-    while (frames - completed >= 2) DVFE_CHECK(wait_one());
-    DVFE_CHECK(ensure_raw());
+// B host images of H rows of `row` bytes -> device memory, on the upload stream.  Into the dense staging: one linear copy
+// when the source is dense too.  Into padded level 0: one pitched 3-D copy when the source's stream stride is a whole
+// number of its rows.  Otherwise one 2-D copy per stream.
+int dvfe_tracker::h2d(uint8_t* dst, size_t dst_pitch, size_t dst_stride, const uint8_t* src, size_t src_pitch, size_t src_stride,
+                      size_t row) {
+    const bool dense = dst_pitch == row && dst_stride == row * H;
+    if (dense && src_pitch == row && src_stride == dst_stride) {
+        DVFE_CUDA(cudaMemcpyAsync(dst, src, (size_t)B * dst_stride, cudaMemcpyHostToDevice, cs));
+    } else if (!dense && src_stride % src_pitch == 0) {
+        cudaMemcpy3DParms p;
+        memset(&p, 0, sizeof(p));
+        p.srcPtr = make_cudaPitchedPtr((void*)src, src_pitch, row, src_stride / src_pitch);
+        p.dstPtr = make_cudaPitchedPtr((void*)dst, dst_pitch, row, dst_stride / dst_pitch);
+        p.extent = make_cudaExtent(row, (size_t)H, (size_t)B);
+        p.kind = cudaMemcpyHostToDevice;
+        DVFE_CUDA(cudaMemcpy3DAsync(&p, cs));
+    } else {
+        for (int s = 0; s < B; s++)
+            DVFE_CUDA(cudaMemcpy2DAsync(dst + s * dst_stride, dst_pitch, src + s * src_stride, src_pitch, row, (size_t)H,
+                                        cudaMemcpyHostToDevice, cs));
+    }
+    return DVFE_OK;
+}
+
+// The route depends on where the images are, whether they need the ingest kernel (BGR or undistortion maps) and the width:
+//   device, gray            the step copies the caller's images into level 0 itself;
+//   device, ingest          the ingest kernel writes level 0 on the compute stream;
+//   host, ingest            dense staging, then the ingest kernel on the upload stream;
+//   host, gray, staged      dense staging, which the step copies into level 0 (pitched DMA of rows that are not a multiple
+//                           of 64 bytes is slow);
+//   host, gray, in place    pitched DMA straight into level 0.
+// Host routes end with ev_up[par] on the upload stream, which the compute stream waits for.  The slots written here were
+// last read by step k-2, which wait_slot() has completed.
+int dvfe_tracker::place_input(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch, bool device,
+                              StepInput* in) {
+    DVFE_CHECK(wait_slot());
+    const bool prep = prep_active();
+    *in = StepInput();
+    in->has_right = right != nullptr;
+    if (device && !prep) {
+        in->left = left; in->right = right; in->stride = stream_stride; in->pitch = pitch;
+        return DVFE_OK;
+    }
+    const uint8_t* src[2] = {left, right};
+    in->in_place = true;
+    if (device) {
+        for (int cam = 0; cam < 2; cam++)
+            if (src[cam]) DVFE_CHECK(ingest(src[cam], stream_stride, pitch, cam, st));
+        return DVFE_OK;
+    }
+    const int par = (int)(frames % 2);
     const size_t row = (size_t)W * in_ch, img = row * H;
     for (int cam = 0; cam < 2; cam++) {
-        const uint8_t* src = cam ? right : left;
-        if (!src) continue;
-        uint8_t* dst = d_raw[par] + (size_t)cam * B * img;
-        if ((size_t)pitch == row && stream_stride == img) {
-            DVFE_CUDA(cudaMemcpyAsync(dst, src, (size_t)B * img, cudaMemcpyHostToDevice, cs));
+        if (!src[cam]) continue;
+        if (prep || staged_upload) {
+            uint8_t* dst = d_stage[par] + (size_t)cam * B * img;
+            DVFE_CHECK(h2d(dst, row, img, src[cam], (size_t)pitch, stream_stride, row));
+            if (prep) DVFE_CHECK(ingest(dst, img, (int)row, cam, cs));
         } else {
-            for (int s = 0; s < B; s++)
-                DVFE_CUDA(cudaMemcpy2DAsync(dst + (size_t)s * img, row, src + s * stream_stride, pitch, row, (size_t)H,
-                                            cudaMemcpyHostToDevice, cs));
+            DVFE_CHECK(h2d(level0(cam), desc.lv[0].pitch, desc.bytes, src[cam], (size_t)pitch, stream_stride, row));
         }
-        DVFE_CHECK(ingest(dst, img, (int)row, cam, cs));
     }
     DVFE_CUDA(cudaEventRecord(ev_up[par], cs));
     DVFE_CUDA(cudaStreamWaitEvent(st, ev_up[par], 0));
+    if (!prep && staged_upload) {
+        in->left = d_stage[par]; in->right = right ? d_stage[par] + B * img : nullptr;
+        in->stride = img; in->pitch = W; in->in_place = false;
+    }
+    return DVFE_OK;
+}
+
+// the staging buffers the host routes of the current input format need: [2 cameras][B][H*W*in_ch] when images are staged or
+// ingested, none when they are DMA'd into level 0
+int dvfe_tracker::size_stage() {
+    for (int p = 0; p < 2; p++) { cudaFree(d_stage[p]); d_stage[p] = nullptr; }
+    if (!staged_upload && !prep_active()) return DVFE_OK;
+    for (int p = 0; p < 2; p++) DVFE_CUDA(cudaMalloc((void**)&d_stage[p], (size_t)2 * B * W * H * in_ch));
     return DVFE_OK;
 }
 
@@ -713,12 +708,9 @@ extern "C" int dvfe_set_input(dvfe_tracker* t, int channels) {
     if (IS_GROUP(t)) return grp_set_input(t, channels);
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
     DVFE_CHECK(t->wait_all());
-    if (channels != t->in_ch) {
-        DVFE_CUDA(cudaStreamSynchronize(t->cs));
-        for (int p = 0; p < 2; p++) { cudaFree(t->d_raw[p]); t->d_raw[p] = nullptr; }
-    }
+    DVFE_CUDA(cudaStreamSynchronize(t->cs));
     t->in_ch = channels;
-    return DVFE_OK;
+    return t->size_stage();
 }
 
 extern "C" int dvfe_set_undistort_maps(dvfe_tracker* t, int cam, const int16_t* map1, const uint16_t* map2) {
@@ -729,13 +721,14 @@ extern "C" int dvfe_set_undistort_maps(dvfe_tracker* t, int cam, const int16_t* 
     DVFE_CUDA(cudaStreamSynchronize(t->cs));
     cudaFree(t->d_map1[cam]); cudaFree(t->d_map2[cam]);
     t->d_map1[cam] = nullptr; t->d_map2[cam] = nullptr;
-    if (!map1) return DVFE_OK;
-    const size_t P = (size_t)t->W * t->H;
-    DVFE_CUDA(cudaMalloc((void**)&t->d_map1[cam], P * 4));
-    DVFE_CUDA(cudaMalloc((void**)&t->d_map2[cam], P * 2));
-    DVFE_CUDA(cudaMemcpy(t->d_map1[cam], map1, P * 4, cudaMemcpyHostToDevice));
-    DVFE_CUDA(cudaMemcpy(t->d_map2[cam], map2, P * 2, cudaMemcpyHostToDevice));
-    return DVFE_OK;
+    if (map1) {
+        const size_t P = (size_t)t->W * t->H;
+        DVFE_CUDA(cudaMalloc((void**)&t->d_map1[cam], P * 4));
+        DVFE_CUDA(cudaMalloc((void**)&t->d_map2[cam], P * 2));
+        DVFE_CUDA(cudaMemcpy(t->d_map1[cam], map1, P * 4, cudaMemcpyHostToDevice));
+        DVFE_CUDA(cudaMemcpy(t->d_map2[cam], map2, P * 2, cudaMemcpyHostToDevice));
+    }
+    return t->size_stage();
 }
 
 static int check_step_args(dvfe_tracker* t, const uint8_t* left, int pitch, const double* time0) {
@@ -747,43 +740,24 @@ static int check_step_args(dvfe_tracker* t, const uint8_t* left, int pitch, cons
     return DVFE_OK;
 }
 
-// the raw step of a leaf tracker from host images, enqueued; sflags: per-stream DVFE_FRAME_* (validated) or null
-static int leaf_track_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
-                            const double* time0, const uint8_t* sflags) {
+// one raw step of a leaf tracker, enqueued; sflags: per-stream DVFE_FRAME_* (validated) or null
+static int leaf_track(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
+                      const double* time0, const uint8_t* sflags, bool device) {
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    if (t->prep_active()) {
-        DVFE_CHECK(t->upload_prepared(left, right, stream_stride, pitch));
-        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr, sflags);
-    }
-    if (t->staged_upload) {
-        const size_t P = (size_t)t->W * t->H;
-        const int par = (int)(t->frames % 2);
-        DVFE_CHECK(t->upload_staged(left, right, stream_stride, pitch));
-        return t->submit(t->d_stage[par], right ? t->d_stage[par] + t->B * P : nullptr, P, t->W, time0, false, false,
-                         right != nullptr, sflags);
-    }
-    DVFE_CHECK(t->upload_in_place(left, right, stream_stride, pitch));
-    return t->submit(nullptr, nullptr, 0, 0, time0, false, true, right != nullptr, sflags);
+    StepInput in;
+    DVFE_CHECK(t->place_input(left, right, stream_stride, pitch, device, &in));
+    return t->submit(in, time0, false, sflags);
 }
 
-// the same from device-resident images
-static int leaf_track_device_async(dvfe_tracker* t, const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch,
-                                   const double* time0, const uint8_t* sflags) {
+static int wait_all_steps(dvfe_tracker* t) {
+    if (IS_GROUP(t)) return grp_wait_all(t);
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    while (t->frames - t->completed >= 2) DVFE_CHECK(t->wait_one());
-    if (t->prep_active()) {
-        DVFE_CHECK(t->ingest(d_left, stream_stride, pitch, 0, t->st));
-        if (d_right) DVFE_CHECK(t->ingest(d_right, stream_stride, pitch, 1, t->st));
-        return t->submit(nullptr, nullptr, 0, 0, time0, false, true, d_right != nullptr, sflags);
-    }
-    return t->submit(d_left, d_right, stream_stride, pitch, time0, false, false, d_right != nullptr, sflags);
+    return t->wait_all();
 }
 
 extern "C" int dvfe_track_image_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride,
                                       int pitch, const double* time0) {
-    DVFE_CHECK(check_step_args(t, left, pitch, time0));
-    if (IS_GROUP(t)) return grp_track_image_async(t, left, right, stream_stride, pitch, time0, false);
-    return leaf_track_async(t, left, right, stream_stride, pitch, time0, nullptr);
+    return dvfe_track_image_ex(t, left, right, stream_stride, pitch, time0, nullptr, 0u);
 }
 
 extern "C" int dvfe_wait(dvfe_tracker* t) {
@@ -795,35 +769,22 @@ extern "C" int dvfe_wait(dvfe_tracker* t) {
 
 extern "C" int dvfe_track_image(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride,
                                 int pitch, const double* time0) {
-    DVFE_CHECK(dvfe_track_image_async(t, left, right, stream_stride, pitch, time0));
-    return IS_GROUP(t) ? grp_wait_all(t) : t->wait_all();
+    DVFE_CHECK(dvfe_track_image_ex(t, left, right, stream_stride, pitch, time0, nullptr, 0u));
+    return wait_all_steps(t);
 }
 
 extern "C" int dvfe_track_image_device(dvfe_tracker* t, const uint8_t* d_left, const uint8_t* d_right,
                                        size_t stream_stride, int pitch, const double* time0) {
     DVFE_CHECK(check_step_args(t, d_left, pitch, time0));
-    if (IS_GROUP(t)) {
-        DVFE_CHECK(grp_wait_all(t));
-        DVFE_CHECK(grp_track_image_async(t, d_left, d_right, stream_stride, pitch, time0, true));
-        return grp_wait_all(t);
-    }
-    DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    DVFE_CHECK(t->wait_all());
-    if (t->prep_active()) {
-        DVFE_CHECK(t->ingest(d_left, stream_stride, pitch, 0, t->st));
-        if (d_right) DVFE_CHECK(t->ingest(d_right, stream_stride, pitch, 1, t->st));
-        DVFE_CHECK(t->submit(nullptr, nullptr, 0, 0, time0, false, true, d_right != nullptr));
-        return t->wait_all();
-    }
-    DVFE_CHECK(t->submit(d_left, d_right, stream_stride, pitch, time0, false, false, d_right != nullptr));
-    return t->wait_all();
+    // an earlier step's capacity error is reported here, before this step is enqueued
+    DVFE_CHECK(wait_all_steps(t));
+    DVFE_CHECK(dvfe_track_image_ex(t, d_left, d_right, stream_stride, pitch, time0, nullptr, DVFE_STEP_DEVICE_INPUT));
+    return wait_all_steps(t);
 }
 
 extern "C" int dvfe_track_image_device_async(dvfe_tracker* t, const uint8_t* d_left, const uint8_t* d_right,
                                              size_t stream_stride, int pitch, const double* time0) {
-    DVFE_CHECK(check_step_args(t, d_left, pitch, time0));
-    if (IS_GROUP(t)) return grp_track_image_async(t, d_left, d_right, stream_stride, pitch, time0, true);
-    return leaf_track_device_async(t, d_left, d_right, stream_stride, pitch, time0, nullptr);
+    return dvfe_track_image_ex(t, d_left, d_right, stream_stride, pitch, time0, nullptr, DVFE_STEP_DEVICE_INPUT);
 }
 
 extern "C" int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
@@ -844,8 +805,7 @@ extern "C" int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const u
         }
     const uint8_t* sf = any ? stream_flags : nullptr;          // no flag set: exactly the step of the plain entry points
     if (IS_GROUP(t)) return grp_track_image_ex(t, left, right, stream_stride, pitch, time0, sf, device);
-    return device ? leaf_track_device_async(t, left, right, stream_stride, pitch, time0, sf)
-                  : leaf_track_async(t, left, right, stream_stride, pitch, time0, sf);
+    return leaf_track(t, left, right, stream_stride, pitch, time0, sf, device);
 }
 
 extern "C" int dvfe_set_lk_mode_site(dvfe_tracker* t, int site, int back_max_level, double fb_threshold) {
@@ -875,7 +835,7 @@ extern "C" int dvfe_set_detect_mode(dvfe_tracker* t, int mode) {
 
 int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask,
                                   size_t stream_stride, int pitch, const int* exist_inst, const double* time0, unsigned flags) {
-    while (frames - completed >= 2) DVFE_CHECK(wait_one());      // buffers of step k-2 are free again
+    DVFE_CHECK(wait_slot());                // before the mask copy: d_inv_in[par] / d_labels[par] are step k-2's until then
     const size_t P = (size_t)W * H;
     const int par = (int)(frames % 2);
     const bool prep = prep_active();
@@ -904,13 +864,9 @@ int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, con
                     DVFE_CUDA(cudaMemcpy2DAsync(dst + s * P, W, mask + s * mask_stride, mask_pitch, W, (size_t)H, cudaMemcpyHostToDevice, cs));
         }
         d_mask = dst; d_mask_stride = P; d_mask_pitch = W;
-        if (prep) DVFE_CHECK(upload_prepared(left, right, stream_stride, pitch));
-        else if (staged_upload) DVFE_CHECK(upload_staged(left, right, stream_stride, pitch));
-        else DVFE_CHECK(upload_in_place(left, right, stream_stride, pitch));          // records ev_up; st waits for it
-    } else if (prep) {
-        DVFE_CHECK(ingest(left, stream_stride, pitch, 0, st));
-        if (right) DVFE_CHECK(ingest(right, stream_stride, pitch, 1, st));
     }
+    StepInput in;                           // a host route's ev_up, recorded after the images, covers the mask copy too
+    DVFE_CHECK(place_input(left, right, stream_stride, pitch, device, &in));
     lab_ptr[par] = labels ? d_mask : nullptr; lab_stride[par] = d_mask_stride; lab_pitch[par] = d_mask_pitch;
     DVFE_CUDA(cudaMemcpyAsync(d_exist, h_exist[par], B * sizeof(int), cudaMemcpyHostToDevice, st));
     // region mask = exist_inst ? erode(inv_merge_mask, mask_morphology_size) : all 255   (:764-772); with a label image
@@ -921,10 +877,7 @@ int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, con
                                      st, labels ? 1 : 0));
     else
         DVFE_CHECK(launch_erode_rect(d_inv_in[par], W, d_region, W, d_region_tmp, W, H, 1, B, P, d_exist, st));   // all 255
-    if (device && !prep) return submit(left, right, stream_stride, pitch, time0, true, false, right != nullptr);
-    if (!device && !prep && staged_upload)
-        return submit(d_stage[par], right ? d_stage[par] + B * P : nullptr, P, W, time0, true, false, right != nullptr);
-    return submit(nullptr, nullptr, 0, 0, time0, true, true, right != nullptr);
+    return submit(in, time0, true);
 }
 
 extern "C" int dvfe_track_semantic_image(dvfe_tracker* t, const uint8_t* left, const uint8_t* right,

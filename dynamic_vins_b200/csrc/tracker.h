@@ -25,6 +25,16 @@ int gftt_cells(int w, int h, float min_dist);
 
 struct InstanceState;   // instances.cu
 
+// Where a frame step finds its images once dvfe_tracker::place_input has put them in place
+struct StepInput {
+    const uint8_t* left = nullptr;                   // device images the step copies into level 0 (null when in_place)
+    const uint8_t* right = nullptr;
+    size_t stride = 0;                               // bytes between the streams' images
+    int pitch = 0;
+    bool in_place = false;                           // level 0 of this step's pyramid slots already holds the images
+    bool has_right = false;
+};
+
 struct dvfe_tracker {
     // A tracker is either a leaf (owns device state for its B streams) or a container of G leaf trackers
     // ("stream groups", dvfe_config::n_groups) that splits every call by stream range.
@@ -119,24 +129,26 @@ struct dvfe_tracker {
     int init();
     int init_instances();
     void free_instances();
-    uint8_t* d_stage[2] = {nullptr, nullptr};       // dense upload staging [2 cameras][B][H*W], one per in-flight step
     bool staged_upload = false;                      // rows that are not a multiple of 64 B make pitched DMA slow
     // frame ingest (dvfe_set_input / dvfe_set_undistort_maps): BGR and/or remapped input goes through a device staging
     // buffer and the ingest kernel, which writes level 0 in place
     int in_ch = 1;
     short* d_map1[2] = {nullptr, nullptr};
     unsigned short* d_map2[2] = {nullptr, nullptr};
-    uint8_t* d_raw[2] = {nullptr, nullptr};          // [2 cameras][B][H*W*in_ch] per in-flight step
+    // dense staging of host images [2 cameras][B][H*W*in_ch], one per in-flight step: the staged upload's copy source, or the
+    // ingest kernel's input; sized by size_stage() whenever the input format changes, never inside a step
+    uint8_t* d_stage[2] = {nullptr, nullptr};
     bool prep_active() const { return in_ch != 1 || d_map1[0] || d_map1[1]; }
-    int ensure_raw();
+    int size_stage();
+    uint8_t* level0(int cam) const;                  // the interior of level 0 of this step's left / right slot
     int ingest(const uint8_t* d_src, size_t stream_stride, int pitch, int cam, cudaStream_t s);
-    int upload_prepared(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch);
-    int upload_in_place(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch);
-    int upload_staged(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch);
+    int h2d(uint8_t* dst, size_t dst_pitch, size_t dst_stride, const uint8_t* src, size_t src_pitch, size_t src_stride, size_t row);
+    int wait_slot();                                 // fewer than two steps in flight: step k-2's buffers are free again
+    // wait_slot, then put this step's images (host or device memory) where the step reads them
+    int place_input(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch, bool device, StepInput* in);
     // enqueue one frame step (no host synchronisation); at most two steps are in flight
     // sflags (nullable): per-stream DVFE_FRAME_* of a raw step (dvfe_track_image_ex), already validated
-    int submit(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch, const double* time0,
-               bool semantic, bool level0_in_place, bool has_right, const uint8_t* sflags = nullptr);
+    int submit(const StepInput& in, const double* time0, bool semantic, const uint8_t* sflags = nullptr);
     // TrackSemanticImage of one frame, enqueued only (uploads on the copy stream, mask erosion + the frame step)
     // flags: DVFE_DYN_DEVICE_INPUT (the three pointers are device memory, nothing is uploaded), DVFE_DYN_LABELS (the mask is a
     // label image: the region is everything no instance bit is set on)

@@ -126,7 +126,7 @@ class BatchTracker:
         L.check(L.lib().dvfe_set_undistort_maps(self._h, cam, L.ptr(m1), L.ptr(m2)))
 
     def _stream_flags(self, stream_flags) -> Optional[np.ndarray]:
-        """per-stream L.FRAME_* bytes of dvfe_track_image_ex (None: the plain entry points)"""
+        """per-stream L.FRAME_* bytes of dvfe_track_image_ex (None: no flag array, the plain step)"""
         if stream_flags is None:
             return None
         f = np.ascontiguousarray(stream_flags, np.uint8)
@@ -142,9 +142,6 @@ class BatchTracker:
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
-        if f is None:
-            L.check(L.lib().dvfe_track_image(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
-            return
         L.check(L.lib().dvfe_track_image_ex(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t),
                                             L.ptr(f), 0))
         self.wait()          # at most two steps are in flight: the second wait returns at once unless an earlier async step was
@@ -158,9 +155,6 @@ class BatchTracker:
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         t = self._times(time0)
         self._keep = (l, r, t, getattr(self, "_keep", None) and self._keep[:3])
-        if f is None:
-            L.check(L.lib().dvfe_track_image_async(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t)))
-            return
         L.check(L.lib().dvfe_track_image_ex(self._h, L.ptr(l), L.ptr(r), self.H * self.W * self.ch, self.W * self.ch, L.ptr(t),
                                             L.ptr(f), 0))
 
@@ -181,10 +175,6 @@ class BatchTracker:
         f = self._stream_flags(stream_flags)
         t = self._times(time0)
         self._keep_t = (t, getattr(self, "_keep_t", (None,))[0])
-        if f is None:
-            L.check(L.lib().dvfe_track_image_device_async(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
-                                                          stream_stride, pitch, L.ptr(t)))
-            return
         L.check(L.lib().dvfe_track_image_ex(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
                                             stream_stride, pitch, L.ptr(t), L.ptr(f), L.STEP_DEVICE_INPUT))
 

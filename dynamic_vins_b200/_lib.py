@@ -79,10 +79,10 @@ SYMBOLS = [
     "dvfe_op_disc_mask", "dvfe_op_erode_rect", "dvfe_op_lift_projective", "dvfe_op_bgr_to_gray", "dvfe_op_merge_masks",
     "dvfe_op_remap", "dvfe_set_input", "dvfe_set_undistort_maps", "dvfe_track_dynamic_async", "dvfe_op_punch_out", "dvfe_insts_table", "dvfe_track_dynamic_ex",
     "dvfe_op_reject_with_f", "dvfe_op_detect_extra_points", "dvfe_op_build_pyramid_bordered", "dvfe_set_detect_mode", "dvfe_op_good_features_cuda",
-    "dvfe_track_image_ex",
+    "dvfe_track_image_ex", "dvfe_track_semantic_ex", "dvfe_track_dynamic_ex2",
 ]
 
-# dvfe_track_image_ex: per-stream frame flags and step flags (include/dvfe.h)
+# dvfe_track_image_ex / _semantic_ex / _dynamic_ex2: per-stream frame flags; dvfe_track_image_ex's step flags (include/dvfe.h)
 FRAME_SKIP, FRAME_NO_RIGHT, FRAME_RESET = 1, 2, 4
 STEP_DEVICE_INPUT = 1
 
@@ -142,6 +142,10 @@ def lib() -> C.CDLL:
         L.dvfe_op_punch_out.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
         L.dvfe_track_dynamic_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
+        L.dvfe_track_dynamic_ex2.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
+        L.dvfe_track_semantic_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_uint]
         L.dvfe_insts_table.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.dvfe_set_input.argtypes = [C.c_void_p, C.c_int]
         L.dvfe_set_undistort_maps.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]

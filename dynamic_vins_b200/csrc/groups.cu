@@ -72,13 +72,13 @@ int grp_wait_all(dvfe_tracker* t) {
 }
 
 int grp_track_semantic(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv, size_t stride, int pitch,
-                       const int* exist, const double* time0) {
+                       const int* exist, const double* time0, const uint8_t* stream_flags, unsigned flags) {
     for (size_t g = 0; g < t->groups.size(); g++) {
         const int f = t->group_first[g];
         const size_t off = (size_t)f * stride;
         const size_t moff = off / (size_t)(t->groups[g]->prep_active() ? t->groups[g]->in_ch : 1);
-        DVFE_CHECK(dvfe_track_semantic_image(t->groups[g], left + off, right ? right + off : nullptr, inv ? inv + moff : nullptr,
-                                             stride, pitch, exist + f, time0 + f));
+        DVFE_CHECK(dvfe_track_semantic_ex(t->groups[g], left + off, right ? right + off : nullptr, inv ? inv + moff : nullptr,
+                                          stride, pitch, exist + f, time0 + f, stream_flags ? stream_flags + f : nullptr, flags));
     }
     return DVFE_OK;
 }
@@ -100,17 +100,18 @@ int grp_insts_track_batch(dvfe_tracker* t, const dvfe_inst_in* boxes, const int*
     return DVFE_OK;
 }
 
+// as grp_track_image_ex: every group submits a step, also one whose streams are all skipped
 int grp_track_dynamic_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv, size_t stride,
                             int pitch, const int* exist, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0,
-                            unsigned flags) {
+                            const uint8_t* stream_flags, unsigned flags) {
     size_t boff = 0;
     for (size_t g = 0; g < t->groups.size(); g++) {
         const int f = t->group_first[g];
         const size_t off = (size_t)f * stride;
         const size_t moff = off / (size_t)(t->groups[g]->prep_active() ? t->groups[g]->in_ch : 1);
-        DVFE_CHECK(dvfe_track_dynamic_ex(t->groups[g], left + off, right ? right + off : nullptr, inv ? inv + moff : nullptr,
-                                         stride, pitch, exist ? exist + f : nullptr, boxes ? boxes + boff : nullptr, n_boxes + f,
-                                         time0 + f, flags));
+        DVFE_CHECK(dvfe_track_dynamic_ex2(t->groups[g], left + off, right ? right + off : nullptr, inv ? inv + moff : nullptr,
+                                          stride, pitch, exist ? exist + f : nullptr, boxes ? boxes + boff : nullptr, n_boxes + f,
+                                          time0 + f, stream_flags ? stream_flags + f : nullptr, flags));
         for (int s = f; s < t->group_first[g + 1]; s++) boff += (size_t)n_boxes[s];
     }
     return DVFE_OK;

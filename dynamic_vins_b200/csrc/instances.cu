@@ -107,6 +107,7 @@ struct InstCall {
     Staged<ErodeJob> erode;
     Staged<GfttJob> gftt;
     Staged<uint8_t> act_track, act_vis, clear_flags;    // indexed by set
+    Staged<uint8_t> lane;                // per set, after a step with stream flags: LANE_PRESENT | LANE_STEREO of its stream
     Staged<double> dt;
     Staged<float2> offs;
     Staged<uint32_t> inst_id;
@@ -150,8 +151,7 @@ int dvfe_tracker::init_instances() {
     I.full = make_pyr_desc(W, H, cfg.lk_max_level > 3 ? cfg.lk_max_level : 3);
     const size_t NS = (size_t)B * I.MI;
     I.streams.resize(B);
-    for (auto& s : I.streams)
-        for (int k = I.MI - 1; k >= 0; k--) s.free_slots.push_back(k);
+    for (int s = 0; s < B; s++) reset_instances(s);
     DVFE_CHECK(alloc_point_sets(&I.pts, (int)NS, I.cap));
     DVFE_CHECK(dmalloc(&I.roi_gray, NS * 2 * I.P));
     DVFE_CHECK(dmalloc(&I.roi_mask, NS * I.P));
@@ -169,7 +169,7 @@ int dvfe_tracker::init_instances() {
         DVFE_CUDA(cudaMallocHost((void**)&C.h_n, (NS + 1) * sizeof(int)));
         memset(C.h_n, 0, (NS + 1) * sizeof(int));
         DVFE_CHECK(C.arena.alloc(NS * (sizeof(CropJob) + 2 * sizeof(PyrJob) + 2 * sizeof(LkGroup) + sizeof(ErodeJob) +
-                                       sizeof(GfttJob) + 3 + sizeof(double) + sizeof(float2) + sizeof(uint32_t)) + 4096));
+                                       sizeof(GfttJob) + 4 + sizeof(double) + sizeof(float2) + sizeof(uint32_t)) + 4096));
         C.arena.take(C.crop, (int)NS);
         C.arena.take(C.pyr, 2 * (int)NS);
         C.arena.take(C.lk_t, (int)NS);
@@ -179,6 +179,7 @@ int dvfe_tracker::init_instances() {
         C.arena.take(C.act_track, (int)NS);
         C.arena.take(C.act_vis, (int)NS);
         C.arena.take(C.clear_flags, (int)NS);
+        C.arena.take(C.lane, (int)NS);
         C.arena.take(C.dt, (int)NS);
         C.arena.take(C.offs, (int)NS);
         C.arena.take(C.inst_id, (int)NS);
@@ -210,6 +211,16 @@ void dvfe_tracker::free_instances() {
     inst = nullptr;
 }
 
+// a newly created InstsFeatManager for `stream` (DVFE_FRAME_RESET): no instances, every slot free, last_time = 0.  A slot's
+// point count is cleared when an instance takes it; Output() of the last completed call stays readable.
+void dvfe_tracker::reset_instances(int stream) {
+    InstStream& S = inst->streams[stream];
+    S.insts.clear();
+    S.free_slots.clear();
+    for (int k = inst->MI - 1; k >= 0; k--) S.free_slots.push_back(k);
+    S.last_time = 0.0;
+}
+
 // InstsFeatManager::ManageInstances (front_end/dynamic_tracker.cpp:499-514)
 static void manage_instances(InstStream& S) {
     for (auto it = S.insts.begin(); it != S.insts.end();) {
@@ -227,14 +238,22 @@ static void manage_instances(InstStream& S) {
     }
 }
 
-// Every box inside the image with a mask, and enough free slots for the new track ids: checked before anything is changed
-// (and, for the pipelined call, before the background step is enqueued), so a bad call leaves the tracker untouched.
-static int insts_validate(dvfe_tracker* t, int s0, int s1, const dvfe_inst_in* const* boxes_of, const int* n_of, bool labels = false) {
+// Every box inside the image with a mask, no box for a skipped stream, and enough free slots for the new track ids: checked before
+// anything is changed (and, for the pipelined call, before the background step is enqueued), so a bad call leaves the tracker
+// untouched.  sflags (nullable, [B]): the stream flags of the frame; a RESET stream's instance table counts as empty.
+static int insts_validate(dvfe_tracker* t, int s0, int s1, const dvfe_inst_in* const* boxes_of, const int* n_of, bool labels,
+                          const uint8_t* sflags) {
     InstanceState& I = *t->inst;
     const int W = t->W, H = t->H;
     for (int stream = s0; stream < s1; stream++) {
         const InstStream& S = I.streams[stream];
         const dvfe_inst_in* boxes = boxes_of[stream - s0];
+        const unsigned sf = sflags ? sflags[stream] : 0u;
+        if ((sf & DVFE_FRAME_SKIP) && n_of[stream - s0] > 0) {
+            dvfe_set_error("insts_track: stream %d skips this frame but has %d boxes", stream, n_of[stream - s0]);
+            return DVFE_ERR_INVALID;
+        }
+        const bool fresh_table = (sf & DVFE_FRAME_RESET) != 0;
         std::vector<uint32_t> fresh;
         for (int b = 0; b < n_of[stream - s0]; b++) {
             const dvfe_inst_in& bx = boxes[b];
@@ -245,10 +264,11 @@ static int insts_validate(dvfe_tracker* t, int s0, int s1, const dvfe_inst_in* c
                                stream, b, bx.x, bx.y, bx.w, bx.h, W, H);
                 return DVFE_ERR_INVALID;
             }
-            if (S.insts.find(bx.track_id) == S.insts.end() && std::find(fresh.begin(), fresh.end(), bx.track_id) == fresh.end())
+            if ((fresh_table || S.insts.find(bx.track_id) == S.insts.end()) &&
+                std::find(fresh.begin(), fresh.end(), bx.track_id) == fresh.end())
                 fresh.push_back(bx.track_id);
         }
-        if (fresh.size() > S.free_slots.size()) {
+        if (fresh.size() > (fresh_table ? (size_t)I.MI : S.free_slots.size())) {
             dvfe_set_error("insts_track: more than max_instances=%d live instances in stream %d", I.MI, stream);
             return DVFE_ERR_CAPACITY;
         }
@@ -263,10 +283,14 @@ static int insts_validate(dvfe_tracker* t, int s0, int s1, const dvfe_inst_in* c
 // dvfe_tracker::wait_one() finishes the call (finish_instances).  Nothing on the host side depends on device results.
 // labels: the ROI masks are cut out of the label images the background step of this frame received (DVFE_DYN_LABELS) on the
 // device, inside the erosion that reads them; no mask bytes cross the bus.
+// The stream flags of the last background step apply: a skipped stream is not touched (no per-frame reset, no lost_num change,
+// no ManageInstances, last_time kept), a NO_RIGHT stream runs mono, a RESET stream's table was cleared by that step.
 static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_in* const* boxes_of, const int* n_of,
                                const double* time_of, bool defer, bool labels = false) {
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    if (!defer) DVFE_CHECK(insts_validate(t, s0, s1, boxes_of, n_of, labels));      // deferred: done before the background step
+    const uint8_t* sflags = t->last_sflags.data();
+    // deferred: validated before the background step
+    if (!defer) DVFE_CHECK(insts_validate(t, s0, s1, boxes_of, n_of, labels, sflags));
     if (!defer) DVFE_CHECK(t->wait_all());
     InstanceState& I = *t->inst;
     const int par = (int)((t->frames - 1) % 2);          // the step these instances belong to
@@ -278,16 +302,20 @@ static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_
     // the frame uploaded by the last background step
     const PyrLevel& L0 = t->desc.lv[0];
     const bool stereo_now = t->cfg.stereo && t->last_has_right;
+    bool partial = false;
+    for (int stream = s0; stream < s1; stream++) partial = partial || sflags[stream] != 0;
 
     memset(C.act_track.h, 0, NS); memset(C.act_vis.h, 0, NS); memset(C.clear_flags.h, 0, NS);
     size_t mask_used = 0;
-    int nv = 0, n_track = 0, max_rw = 1, max_rh = 1, max_pw = 1, max_ph = 1, max_lv = 1;
+    int nv = 0, n_track = 0, n_stereo = 0, max_rw = 1, max_rh = 1, max_pw = 1, max_ph = 1, max_lv = 1;
     bool any_clear = false;
     std::vector<char> exist(s1 - s0, 0);
     C.s0 = s0; C.s1 = s1; C.plan.clear(); C.has_records = false;
     C.h_n[NS] = 0;
 
     for (int stream = s0; stream < s1; stream++) {
+        if (sflags[stream] & DVFE_FRAME_SKIP) continue;                  // InstsTrack is not called for this stream
+        const bool stereo = stereo_now && !(sflags[stream] & DVFE_FRAME_NO_RIGHT);
         InstStream& S = I.streams[stream];
         const dvfe_inst_in* boxes = boxes_of[stream - s0];
         const int n_boxes = n_of[stream - s0];
@@ -357,6 +385,7 @@ static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_
             c.dst = I.roi_gray + (set * 2 + in.cur_buf) * P;
             max_rw = std::max(max_rw, in.w); max_rh = std::max(max_rh, in.h);
             C.act_vis.h[set] = 1;
+            C.lane.h[set] = (uint8_t)(LANE_PRESENT | (stereo ? LANE_STEREO : 0u));
             C.dt.h[set] = time0 - S.last_time;                         // curr_time - last_time
             C.offs.h[set] = make_float2((float)in.x, (float)in.y);       // box2d->rect.tl()
             C.inst_id.h[set] = in.track_id;
@@ -401,7 +430,8 @@ static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_
             J.disc_radius = t->cfg.min_dynamic_dist; J.min_dist = (float)t->cfg.min_dynamic_dist; J.quality = 0.01;
             J.err = t->d_err + par;
             // stereo job: TrackRightByPad — full images, points offset by rect.tl()
-            LkGroup& R = C.lk_s.h[j];
+            if (!stereo) continue;
+            LkGroup& R = C.lk_s.h[n_stereo++];
             memset(&R, 0, sizeof(R));
             R.pyrA = left_pyr; R.pyrB = right_pyr; R.desc = t->desc;
             R.ptsA = I.pts.pts + set * cap; R.ptsB = I.pts.rpts + set * cap; R.status = I.pts.rstatus + set * cap;
@@ -437,9 +467,9 @@ static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_
         // UndistortedPointsWithAddOffset(cam0) + PtsVelocity(curr_time - last_time) (:448-457)
         DVFE_CHECK(launch_left_post(V, n_sets, cap, t->cam0, C.dt.d + set0, C.offs.d + set0, st, C.act_vis.d + set0));
         // TrackRightByPad + RightUndistortedPts + RightPtsVelocity (:462-471), then the Output() records
-        if (stereo_now) DVFE_CHECK(launch_lk(C.lk_s.d, nv, cap, t->cfg.lk_max_level, t->cfg.flow_back, st));
+        if (n_stereo > 0) DVFE_CHECK(launch_lk(C.lk_s.d, n_stereo, cap, t->cfg.lk_max_level, t->cfg.flow_back, st));
         DVFE_CHECK(launch_inst_post_pack(V, n_sets, cap, t->cam1, C.dt.d + set0, C.act_vis.d + set0, stereo_now ? 1 : 0,
-                                         C.inst_id.d + set0, C.d_out + o, C.d_n + set0, st));
+                                         partial ? C.lane.d + set0 : nullptr, C.inst_id.d + set0, C.d_out + o, C.d_n + set0, st));
         C.has_records = true;
     }
     if (any_clear) DVFE_CHECK(launch_clear_sets(I.pts.n + set0, C.clear_flags.d + set0, n_sets, st));
@@ -516,7 +546,7 @@ int dvfe_tracker::finish_instances(int par) {
 
 int grp_track_dynamic_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv, size_t stride,
                             int pitch, const int* exist, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0,
-                            unsigned flags);
+                            const uint8_t* stream_flags, unsigned flags);
 int grp_insts_track(dvfe_tracker* t, int stream, const dvfe_inst_in* boxes, int n, double time0);
 int grp_insts_track_batch(dvfe_tracker* t, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0);
 int grp_route(dvfe_tracker* t, int stream, dvfe_tracker** leaf, int* local);
@@ -566,18 +596,22 @@ extern "C" int dvfe_insts_track_batch(dvfe_tracker* t, const dvfe_inst_in* boxes
 extern "C" int dvfe_track_dynamic_async(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask,
                                         size_t stream_stride, int pitch, const int* exist_inst, const dvfe_inst_in* boxes,
                                         const int* n_boxes, const double* time0) {
-    return dvfe_track_dynamic_ex(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, boxes, n_boxes, time0, 0u);
+    return dvfe_track_dynamic_ex2(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, boxes, n_boxes, time0, nullptr, 0u);
 }
 
 extern "C" int dvfe_track_dynamic_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* mask,
                                      size_t stream_stride, int pitch, const int* exist_inst, const dvfe_inst_in* boxes,
                                      const int* n_boxes, const double* time0, unsigned flags) {
+    return dvfe_track_dynamic_ex2(t, left, right, mask, stream_stride, pitch, exist_inst, boxes, n_boxes, time0, nullptr, flags);
+}
+
+extern "C" int dvfe_track_dynamic_ex2(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* mask,
+                                      size_t stream_stride, int pitch, const int* exist_inst, const dvfe_inst_in* boxes,
+                                      const int* n_boxes, const double* time0, const uint8_t* stream_flags, unsigned flags) {
     const bool labels = (flags & DVFE_DYN_LABELS) != 0;
     if (!t || !left || !time0 || !n_boxes || (!exist_inst && !labels)) { dvfe_set_error("track_dynamic: null argument"); return DVFE_ERR_INVALID; }
-    if (!t->groups.empty())
-        return grp_track_dynamic_async(t, left, right, mask, stream_stride, pitch, exist_inst, boxes, n_boxes, time0, flags);
-    if (!t->inst) { dvfe_set_error("track_dynamic_async: max_instances must be > 0 at create"); return DVFE_ERR_INVALID; }
-    if (pitch < t->W * t->in_ch) { dvfe_set_error("track_dynamic_async: bad pitch"); return DVFE_ERR_INVALID; }
+    const uint8_t* sf = nullptr;
+    DVFE_CHECK(check_stream_flags(stream_flags, t->B, "track_dynamic", &sf));
     std::vector<const dvfe_inst_in*> of(t->B);
     size_t off = 0;
     for (int s = 0; s < t->B; s++) {
@@ -585,11 +619,24 @@ extern "C" int dvfe_track_dynamic_ex(dvfe_tracker* t, const uint8_t* left, const
         of[s] = boxes + off;
         off += (size_t)n_boxes[s];
     }
+    if (!t->groups.empty()) {
+        // every group's boxes are checked before the first group enqueues anything
+        for (size_t g = 0; g < t->groups.size(); g++) {
+            dvfe_tracker* leaf = t->groups[g];
+            const int f = t->group_first[g];
+            if (leaf->inst) DVFE_CHECK(insts_validate(leaf, 0, leaf->B, of.data() + f, n_boxes + f, labels, sf ? sf + f : nullptr));
+        }
+        return grp_track_dynamic_async(t, left, right, mask, stream_stride, pitch, exist_inst, boxes, n_boxes, time0, sf, flags);
+    }
+    if (!t->inst) { dvfe_set_error("track_dynamic_async: max_instances must be > 0 at create"); return DVFE_ERR_INVALID; }
+    if (pitch < t->W * t->in_ch) { dvfe_set_error("track_dynamic_async: bad pitch"); return DVFE_ERR_INVALID; }
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    DVFE_CHECK(insts_validate(t, 0, t->B, of.data(), n_boxes, labels));
+    DVFE_CHECK(insts_validate(t, 0, t->B, of.data(), n_boxes, labels, sf));
+    // SetMaskAndRoi: exist_inst = !boxes2d.empty(); a skipped stream's exist_inst is not read
     std::vector<int> exist(t->B);
-    for (int s = 0; s < t->B; s++) exist[s] = labels ? (n_boxes[s] > 0 ? 1 : 0) : exist_inst[s];     // SetMaskAndRoi: exist_inst = !boxes2d.empty()
-    DVFE_CHECK(t->semantic_submit(left, right, mask, stream_stride, pitch, exist.data(), time0, flags));
+    for (int s = 0; s < t->B; s++)
+        exist[s] = (sf && (sf[s] & DVFE_FRAME_SKIP)) ? 0 : labels ? (n_boxes[s] > 0 ? 1 : 0) : exist_inst[s];
+    DVFE_CHECK(t->semantic_submit(left, right, mask, stream_stride, pitch, exist.data(), time0, flags, sf));
     return insts_track_streams(t, 0, t->B, of.data(), n_boxes, time0, true, labels);
 }
 

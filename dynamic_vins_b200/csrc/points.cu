@@ -227,12 +227,14 @@ int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const C
 
 // ---- instances: RightUndistortedPts + RightPtsVelocity + InstsFeatManager::Output record -----------------------
 // (front_end/dynamic_tracker.cpp:462-471, 521-577).  One record per point at out[set*cap + i]; ids ascend with i.
+// lanes (nullable, per set): whether the set's stream had a right image (LANE_STEREO) in place of stereo_all for every set.
 __global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int cap, CamParams cam1, const double* __restrict__ dt,
-                                                        const uint8_t* __restrict__ active, int stereo_now,
-                                                        const uint32_t* __restrict__ inst_id, dvfe_inst_obs* __restrict__ out,
-                                                        int* __restrict__ n_out) {
+                                                        const uint8_t* __restrict__ active, int stereo_all,
+                                                        const uint8_t* __restrict__ lanes, const uint32_t* __restrict__ inst_id,
+                                                        dvfe_inst_obs* __restrict__ out, int* __restrict__ n_out) {
     const int set = blockIdx.y;
     if (!active[set]) return;
+    const int stereo_now = lanes != nullptr ? (lanes[set] & LANE_STEREO) != 0 : stereo_all;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     // the record count of this call, snapshotted into the call's own buffer: S.n is rewritten by the next step while the
     // download stream may still be reading
@@ -269,11 +271,11 @@ __global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int ca
 }
 
 int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
-                          const uint8_t* d_active, int stereo_now, const uint32_t* d_inst_id, dvfe_inst_obs* out,
-                          int* d_n_out, cudaStream_t st) {
+                          const uint8_t* d_active, int stereo_now, const uint8_t* d_lane, const uint32_t* d_inst_id,
+                          dvfe_inst_obs* out, int* d_n_out, cudaStream_t st) {
     if (n_sets <= 0) return DVFE_OK;
     dim3 grid((cap + 127) / 128, n_sets);
-    DVFE_LAUNCH(k_inst_post_pack, grid, 128, 0, st, S, cap, cam1, d_dt, d_active, stereo_now, d_inst_id, out, d_n_out);
+    DVFE_LAUNCH(k_inst_post_pack, grid, 128, 0, st, S, cap, cam1, d_dt, d_active, stereo_now, d_lane, d_inst_id, out, d_n_out);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }

@@ -38,7 +38,7 @@ int grp_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* righ
 int grp_wait(dvfe_tracker* t);
 int grp_wait_all(dvfe_tracker* t);
 int grp_track_semantic(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv, size_t stride, int pitch,
-                       const int* exist, const double* time0);
+                       const int* exist, const double* time0, const uint8_t* stream_flags, unsigned flags);
 int grp_route(dvfe_tracker* t, int stream, dvfe_tracker** leaf, int* local);
 int grp_set_lk_mode(dvfe_tracker* t, int site, int back_max_level, double fb);
 int grp_set_detect_mode(dvfe_tracker* t, int mode);
@@ -198,6 +198,7 @@ int dvfe_tracker::init() {
     DVFE_CHECK(dmalloc(&d_err, (size_t)2));
     prev_time.assign(B, 0.0);
     tc_valid.assign(B, 0);
+    last_sflags.assign(B, 0);
     DVFE_CHECK(dmalloc(&d_sflags, (size_t)B));
     DVFE_CHECK(dmalloc(&d_lane, (size_t)B));
     DVFE_CHECK(dmalloc(&d_pgroups[0], (size_t)B));
@@ -372,8 +373,8 @@ void dvfe_tracker::drop_graphs() {
 // The kernels of one frame step on the compute stream `st` (+ the right pyramid on `rs`, forked and joined by events).
 // No host-dependent state is read: the same call with the same arguments enqueues the same work, which is what lets
 // submit() capture it into a graph.
-// partial: the step of dvfe_track_image_ex with some stream flag set (raw mode only).  The same kernels run on the partial tables
-// (presence.cu), which k_partial_tables derives from the flags copied here; skipped streams' previous pyramids are carried.
+// partial: a step with some stream flag set.  The same kernels run on the partial tables (presence.cu), which k_partial_tables
+// derives from the flags copied here and the tables of this phase and mode; skipped streams' previous pyramids are carried.
 int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right, size_t stream_stride, int pitch, bool semantic,
                                   int level0_mode, bool stereo_now, long k, bool with_marks, bool partial) {
     const int ph = (int)(k % 6), par = (int)(k % 2);
@@ -387,7 +388,8 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
     if (partial) {
         DVFE_CUDA(cudaMemcpyAsync(d_sflags, h_sflags[par], (size_t)B, cudaMemcpyHostToDevice, st));
         PartialTables pt;
-        pt.full_temporal = d_groups[ph][0]; pt.full_stereo = d_groups[ph][2]; pt.full_jobs = d_jobs[ph][0];
+        pt.full_temporal = d_groups[ph][semantic ? 1 : 0]; pt.full_stereo = d_groups[ph][2];
+        pt.full_jobs = d_jobs[ph][semantic ? (detect_cuda ? 2 : 1) : 0];
         pt.temporal = d_pgroups[0]; pt.stereo = d_pgroups[1]; pt.jobs = d_pjobs; pt.lane = d_lane;
         pt.zero = d_zero; pt.n = bg.n; pt.next_id = d_next_id;
         DVFE_CHECK(launch_partial_tables(pt, d_sflags, B, stereo_now ? 1 : 0, st));     // also RESET: n = 0, next_id = 1
@@ -563,6 +565,8 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
     for (int s = 0; s < B; s++)
         if (!partial || !(sflags[s] & DVFE_FRAME_SKIP)) prev_time[s] = time0[s];
     last_has_right = stereo_now;
+    if (partial) last_sflags.assign(sflags, sflags + B);
+    else last_sflags.assign(B, 0);
     frames++;
     return DVFE_OK;
 }
@@ -787,23 +791,29 @@ extern "C" int dvfe_track_image_device_async(dvfe_tracker* t, const uint8_t* d_l
     return dvfe_track_image_ex(t, d_left, d_right, stream_stride, pitch, time0, nullptr, DVFE_STEP_DEVICE_INPUT);
 }
 
+int check_stream_flags(const uint8_t* stream_flags, int B, const char* who, const uint8_t** out) {
+    bool any = false;
+    if (stream_flags)
+        for (int s = 0; s < B; s++) {
+            const unsigned f = stream_flags[s];
+            if ((f & ~(DVFE_FRAME_SKIP | DVFE_FRAME_NO_RIGHT | DVFE_FRAME_RESET)) ||
+                (f & (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) == (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) {
+                dvfe_set_error("%s: stream %d: invalid stream flags 0x%x", who, s, f);
+                return DVFE_ERR_INVALID;
+            }
+            any = any || f != 0;
+        }
+    *out = any ? stream_flags : nullptr;                       // no flag set: exactly the step of the plain entry points
+    return DVFE_OK;
+}
+
 extern "C" int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
                                    const double* time0, const uint8_t* stream_flags, unsigned flags) {
     DVFE_CHECK(check_step_args(t, left, pitch, time0));
     if (flags & ~DVFE_STEP_DEVICE_INPUT) { dvfe_set_error("track_image_ex: unknown flags 0x%x", flags); return DVFE_ERR_INVALID; }
     const bool device = (flags & DVFE_STEP_DEVICE_INPUT) != 0;
-    bool any = false;
-    if (stream_flags)
-        for (int s = 0; s < t->B; s++) {
-            const unsigned f = stream_flags[s];
-            if ((f & ~(DVFE_FRAME_SKIP | DVFE_FRAME_NO_RIGHT | DVFE_FRAME_RESET)) ||
-                (f & (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) == (DVFE_FRAME_SKIP | DVFE_FRAME_RESET)) {
-                dvfe_set_error("track_image_ex: stream %d: invalid stream flags 0x%x", s, f);
-                return DVFE_ERR_INVALID;
-            }
-            any = any || f != 0;
-        }
-    const uint8_t* sf = any ? stream_flags : nullptr;          // no flag set: exactly the step of the plain entry points
+    const uint8_t* sf = nullptr;
+    DVFE_CHECK(check_stream_flags(stream_flags, t->B, "track_image_ex", &sf));
     if (IS_GROUP(t)) return grp_track_image_ex(t, left, right, stream_stride, pitch, time0, sf, device);
     return leaf_track(t, left, right, stream_stride, pitch, time0, sf, device);
 }
@@ -834,7 +844,8 @@ extern "C" int dvfe_set_detect_mode(dvfe_tracker* t, int mode) {
 }
 
 int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask,
-                                  size_t stream_stride, int pitch, const int* exist_inst, const double* time0, unsigned flags) {
+                                  size_t stream_stride, int pitch, const int* exist_inst, const double* time0, unsigned flags,
+                                  const uint8_t* sflags) {
     DVFE_CHECK(wait_slot());                // before the mask copy: d_inv_in[par] / d_labels[par] are step k-2's until then
     const size_t P = (size_t)W * H;
     const int par = (int)(frames % 2);
@@ -843,11 +854,13 @@ int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, con
     // the region mask / label image is one byte per pixel whatever the image format
     const size_t mask_stride = prep ? stream_stride / (size_t)in_ch : stream_stride;
     const int mask_pitch = prep ? pitch / in_ch : pitch;
+    // a skipped stream counts as one without instances: its mask is neither copied nor eroded
     bool all = true;
     for (int s = 0; s < B; s++) {
-        h_exist[par][s] = exist_inst[s] ? 1 : 0;
-        all = all && exist_inst[s];
-        if (exist_inst[s] && !mask) { dvfe_set_error("track_semantic_image: exist_inst set but no mask"); return DVFE_ERR_INVALID; }
+        const bool ex = !(sflags && (sflags[s] & DVFE_FRAME_SKIP)) && exist_inst[s];
+        h_exist[par][s] = ex ? 1 : 0;
+        all = all && ex;
+        if (ex && !mask) { dvfe_set_error("track_semantic_image: exist_inst set but no mask"); return DVFE_ERR_INVALID; }
     }
     const uint8_t* d_mask = mask;            // where the erosion reads the mask / label image from
     size_t d_mask_stride = mask_stride;
@@ -860,7 +873,7 @@ int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, con
             DVFE_CUDA(cudaMemcpyAsync(dst, mask, (size_t)B * P, cudaMemcpyHostToDevice, cs));
         } else {
             for (int s = 0; s < B; s++)
-                if (exist_inst[s])
+                if (h_exist[par][s])
                     DVFE_CUDA(cudaMemcpy2DAsync(dst + s * P, W, mask + s * mask_stride, mask_pitch, W, (size_t)H, cudaMemcpyHostToDevice, cs));
         }
         d_mask = dst; d_mask_stride = P; d_mask_pitch = W;
@@ -877,19 +890,32 @@ int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, con
                                      st, labels ? 1 : 0));
     else
         DVFE_CHECK(launch_erode_rect(d_inv_in[par], W, d_region, W, d_region_tmp, W, H, 1, B, P, d_exist, st));   // all 255
-    return submit(in, time0, true);
+    if (sflags && inst)
+        for (int s = 0; s < B; s++)
+            if (sflags[s] & DVFE_FRAME_RESET) reset_instances(s);
+    return submit(in, time0, true, sflags);
+}
+
+extern "C" int dvfe_track_semantic_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask,
+                                      size_t stream_stride, int pitch, const int* exist_inst, const double* time0,
+                                      const uint8_t* stream_flags, unsigned flags) {
+    DVFE_CHECK(check_step_args(t, left, pitch, time0));
+    if (!exist_inst) { dvfe_set_error("track_semantic_image: exist_inst is null"); return DVFE_ERR_INVALID; }
+    if (flags & ~DVFE_DYN_DEVICE_INPUT) { dvfe_set_error("track_semantic_ex: unknown flags 0x%x", flags); return DVFE_ERR_INVALID; }
+    const uint8_t* sf = nullptr;
+    DVFE_CHECK(check_stream_flags(stream_flags, t->B, "track_semantic_ex", &sf));
+    if (IS_GROUP(t)) return grp_track_semantic(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0, sf, flags);
+    DVFE_CUDA(cudaSetDevice(t->cfg.device));
+    return t->semantic_submit(left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0, flags, sf);
 }
 
 extern "C" int dvfe_track_semantic_image(dvfe_tracker* t, const uint8_t* left, const uint8_t* right,
                                          const uint8_t* inv_merge_mask, size_t stream_stride, int pitch,
                                          const int* exist_inst, const double* time0) {
     DVFE_CHECK(check_step_args(t, left, pitch, time0));
-    if (!exist_inst) { dvfe_set_error("track_semantic_image: exist_inst is null"); return DVFE_ERR_INVALID; }
-    if (IS_GROUP(t)) return grp_track_semantic(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0);
-    DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    DVFE_CHECK(t->wait_all());
-    DVFE_CHECK(t->semantic_submit(left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0));
-    return t->wait_all();
+    DVFE_CHECK(wait_all_steps(t));
+    DVFE_CHECK(dvfe_track_semantic_ex(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0, nullptr, 0u));
+    return wait_all_steps(t);
 }
 
 extern "C" int dvfe_get_features(dvfe_tracker* t, int stream, dvfe_obs* out, int cap, int* n_out) {

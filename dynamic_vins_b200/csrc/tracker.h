@@ -22,6 +22,9 @@ int alloc_gftt_scratch(GfttScratch* sc, int n_jobs, int w, int h, float min_dist
 void free_gftt_scratch(GfttScratch* sc);
 void gftt_job_bind_scratch(GfttJob* J, const GfttScratch& sc, int j);
 int gftt_cells(int w, int h, float min_dist);
+// Checks per-stream DVFE_FRAME_* bytes (nullable) of a tracker with B streams; *out = stream_flags, or null when no flag is set (the
+// step is then the plain one).  DVFE_ERR_INVALID for unknown bits and SKIP|RESET.
+int check_stream_flags(const uint8_t* stream_flags, int B, const char* who, const uint8_t** out);
 
 struct InstanceState;   // instances.cu
 
@@ -56,6 +59,8 @@ struct dvfe_tracker {
     long frames = 0;                                 // steps submitted
     long completed = 0;                              // steps whose outputs have been waited for
     bool last_has_right = false;                     // the last submitted frame had a right image
+    std::vector<uint8_t> last_sflags;                // [B] DVFE_FRAME_* of the last submitted step (all 0 for a full step): the
+                                                     // InstsTrack of the same frame follows them
     PointSetArrays bg{};                             // background point sets, one per stream
     uint32_t* d_next_id = nullptr;                   // [B] InstFeat::global_id_count per stream
     double* d_dt = nullptr;
@@ -147,13 +152,15 @@ struct dvfe_tracker {
     // wait_slot, then put this step's images (host or device memory) where the step reads them
     int place_input(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch, bool device, StepInput* in);
     // enqueue one frame step (no host synchronisation); at most two steps are in flight
-    // sflags (nullable): per-stream DVFE_FRAME_* of a raw step (dvfe_track_image_ex), already validated
+    // sflags (nullable): per-stream DVFE_FRAME_* (dvfe_track_image_ex / _semantic_ex / _dynamic_ex2), already validated
     int submit(const StepInput& in, const double* time0, bool semantic, const uint8_t* sflags = nullptr);
     // TrackSemanticImage of one frame, enqueued only (uploads on the copy stream, mask erosion + the frame step)
     // flags: DVFE_DYN_DEVICE_INPUT (the three pointers are device memory, nothing is uploaded), DVFE_DYN_LABELS (the mask is a
-    // label image: the region is everything no instance bit is set on)
+    // label image: the region is everything no instance bit is set on).  sflags: as submit; a skipped stream's exist_inst and
+    // mask are not read, a RESET stream's instance manager starts over too
     int semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
-                        int pitch, const int* exist_inst, const double* time0, unsigned flags = 0);
+                        int pitch, const int* exist_inst, const double* time0, unsigned flags = 0, const uint8_t* sflags = nullptr);
+    void reset_instances(int stream);                // instances.cu: a newly created InstsFeatManager for one stream
     uint8_t* d_labels[2] = {nullptr, nullptr};       // uploaded label images, one per in-flight step (allocated on first use)
     const uint8_t* lab_ptr[2] = {nullptr, nullptr};  // the label images of the in-flight steps (device), for the ROI masks
     size_t lab_stride[2] = {0, 0};

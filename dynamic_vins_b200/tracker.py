@@ -126,7 +126,7 @@ class BatchTracker:
         L.check(L.lib().dvfe_set_undistort_maps(self._h, cam, L.ptr(m1), L.ptr(m2)))
 
     def _stream_flags(self, stream_flags) -> Optional[np.ndarray]:
-        """per-stream L.FRAME_* bytes of dvfe_track_image_ex (None: no flag array, the plain step)"""
+        """per-stream L.FRAME_* bytes of dvfe_track_image_ex / _semantic_ex / _dynamic_ex2 (None: no flag array, the plain step)"""
         if stream_flags is None:
             return None
         f = np.ascontiguousarray(stream_flags, np.uint8)
@@ -213,25 +213,35 @@ class BatchTracker:
             L.check(L.lib().dvfe_set_detect_mode(self._h, 1 if self._detect_cuda else 0))
             self._naive = False
 
-    def track_image_naive(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
+    def track_image_naive(self, left, right, inv_merge_mask, exist_inst, time0, stream_flags=None) -> None:
         """FeatureTracker::TrackImageNaive (front_end/background_tracker.cpp:400-516): the semantic step with the cv::cuda call
         pattern (3, 1.0) at both semantic LK sites and the cv::cuda detector's threshold.  The modes of the other entry points
-        (set_lk_mode, set_detect_mode) are left as they were."""
+        (set_lk_mode, set_detect_mode) are left as they were.  stream_flags: as track_semantic_image."""
+        f = self._stream_flags(stream_flags)
         self._enter_naive()
-        self._semantic(left, right, inv_merge_mask, exist_inst, time0)
+        self._semantic(left, right, inv_merge_mask, exist_inst, time0, f)
 
-    def track_semantic_image(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
+    def track_semantic_image(self, left, right, inv_merge_mask, exist_inst, time0, stream_flags=None) -> None:
+        """stream_flags: None, or B bytes of FRAME_SKIP / FRAME_NO_RIGHT / FRAME_RESET (per-stream frame presence, include/dvfe.h
+        dvfe_track_semantic_ex); a following insts_track_batch of the same frame obeys them"""
+        f = self._stream_flags(stream_flags)
         self._leave_naive()
-        self._semantic(left, right, inv_merge_mask, exist_inst, time0)
+        self._semantic(left, right, inv_merge_mask, exist_inst, time0, f)
 
-    def _semantic(self, left, right, inv_merge_mask, exist_inst, time0) -> None:
+    def _semantic(self, left, right, inv_merge_mask, exist_inst, time0, f) -> None:
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         m = self._batch(inv_merge_mask, self.B, self.H, self.W)
         e = np.ascontiguousarray(np.broadcast_to(np.asarray(exist_inst, np.int32), (self.B,)))
         t = self._times(time0)
-        L.check(L.lib().dvfe_track_semantic_image(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch,
-                                                  self.W * self.ch, L.ptr(e), L.ptr(t)))
+        if f is None:
+            L.check(L.lib().dvfe_track_semantic_image(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch,
+                                                      self.W * self.ch, L.ptr(e), L.ptr(t)))
+            return
+        L.check(L.lib().dvfe_track_semantic_ex(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch, self.W * self.ch,
+                                               L.ptr(e), L.ptr(t), L.ptr(f), 0))
+        self.wait()          # as track_image: the second wait completes this step when an earlier async step was still pending
+        self.wait()
 
     def insts_track(self, stream: int, boxes: Sequence[dict], time0: float, disp=None) -> None:
         """boxes: [{track_id, rect=(x,y,w,h), mask (h,w) uint8}] (SemanticImage::boxes2d); disp: SemanticImage::disp of the
@@ -273,8 +283,11 @@ class BatchTracker:
         t = self._times(time0)
         L.check(L.lib().dvfe_insts_track_batch(self._h, arr, L.ptr(counts), L.ptr(t)))
 
-    def track_dynamic_async(self, left, right, inv_merge_mask, exist_inst, boxes_per_stream, time0) -> None:
-        """TrackSemanticImage + InstsTrack of one frame for all streams, pipelined; results after the matching wait()"""
+    def track_dynamic_async(self, left, right, inv_merge_mask, exist_inst, boxes_per_stream, time0, stream_flags=None) -> None:
+        """TrackSemanticImage + InstsTrack of one frame for all streams, pipelined; results after the matching wait().
+        stream_flags: None, or B bytes of FRAME_SKIP / FRAME_NO_RIGHT / FRAME_RESET (include/dvfe.h dvfe_track_dynamic_ex2); a
+        skipped stream has no boxes"""
+        f = self._stream_flags(stream_flags)
         self._leave_naive()
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
@@ -284,8 +297,12 @@ class BatchTracker:
         assert len(counts) == self.B
         t = self._times(time0)
         self._keep = (l, r, m, e, arr, counts, keep, t, getattr(self, "_keep", None) and self._keep[:8])
-        L.check(L.lib().dvfe_track_dynamic_async(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch,
-                                                 self.W * self.ch, L.ptr(e), arr, L.ptr(counts), L.ptr(t)))
+        if f is None:
+            L.check(L.lib().dvfe_track_dynamic_async(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch,
+                                                     self.W * self.ch, L.ptr(e), arr, L.ptr(counts), L.ptr(t)))
+        else:
+            L.check(L.lib().dvfe_track_dynamic_ex2(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch,
+                                                   self.W * self.ch, L.ptr(e), arr, L.ptr(counts), L.ptr(t), L.ptr(f), 0))
 
     # ---- outputs -------------------------------------------------------------------------------
     def features(self, stream: int = 0) -> np.ndarray:
@@ -301,10 +318,13 @@ class BatchTracker:
 
     DYN_DEVICE_INPUT, DYN_LABELS = 1, 2
 
-    def track_dynamic_labels_async(self, left, right, labels, boxes_per_stream, time0, device: bool = False) -> None:
+    def track_dynamic_labels_async(self, left, right, labels, boxes_per_stream, time0, device: bool = False,
+                                   stream_flags=None) -> None:
         """SemanticImage::SetMaskAndRoi on the device: `labels` holds one u8 label image per stream (bit b = the instance whose
         box has label_bit == b).  Host arrays, or (device=True) device addresses `left`, `right`, `labels` of dense
-        [B][H][W] buffers.  Pipelined like track_dynamic_async; results after the matching wait()."""
+        [B][H][W] buffers.  Pipelined like track_dynamic_async; results after the matching wait().  stream_flags: as
+        track_dynamic_async."""
+        f = self._stream_flags(stream_flags)
         self._leave_naive()
         arr, counts, keep = boxes_per_stream if isinstance(boxes_per_stream, tuple) else self.marshal_boxes(boxes_per_stream)
         assert len(counts) == self.B
@@ -313,15 +333,21 @@ class BatchTracker:
         if device:
             l, r, m = C.c_void_p(left), (C.c_void_p(right) if right else None), C.c_void_p(labels)
             self._keep = (arr, counts, keep, t, getattr(self, "_keep", None) and self._keep[:4])
-            L.check(L.lib().dvfe_track_dynamic_ex(self._h, l, r, m, self.H * self.W * self.ch, self.W * self.ch, None, arr,
-                                                  L.ptr(counts), L.ptr(t), flags))
+            self._dynamic_ex(l, r, m, arr, counts, t, f, flags)
             return
         l = self._batch(left, self.B, self.H, self.W, self.ch)
         r = self._batch(right, self.B, self.H, self.W, self.ch)
         m = self._batch(labels, self.B, self.H, self.W)
         self._keep = (l, r, m, arr, counts, keep, t, getattr(self, "_keep", None) and self._keep[:7])
-        L.check(L.lib().dvfe_track_dynamic_ex(self._h, L.ptr(l), L.ptr(r), L.ptr(m), self.H * self.W * self.ch, self.W * self.ch,
-                                              None, arr, L.ptr(counts), L.ptr(t), flags))
+        self._dynamic_ex(L.ptr(l), L.ptr(r), L.ptr(m), arr, counts, t, f, flags)
+
+    def _dynamic_ex(self, l, r, m, arr, counts, t, f, flags) -> None:
+        if f is None:
+            L.check(L.lib().dvfe_track_dynamic_ex(self._h, l, r, m, self.H * self.W * self.ch, self.W * self.ch, None, arr,
+                                                  L.ptr(counts), L.ptr(t), flags))
+        else:
+            L.check(L.lib().dvfe_track_dynamic_ex2(self._h, l, r, m, self.H * self.W * self.ch, self.W * self.ch, None, arr,
+                                                   L.ptr(counts), L.ptr(t), L.ptr(f), flags))
 
     def insts_table(self, stream: int = 0) -> list:
         """InstsFeatManager::instances after the last InstsTrack: [(track_id, lost_num, is_curr_visible, has_box, rect)]"""

@@ -221,6 +221,18 @@ int dvfe_track_semantic_image(dvfe_tracker* t, const uint8_t* left, const uint8_
                               const uint8_t* inv_merge_mask, size_t stream_stride, int pitch,
                               const int* exist_inst, const double* time0);
 
+/* Per-stream frame presence for TrackSemanticImage (and TrackImageNaive, see dvfe_set_detect_mode): one step, enqueued (pair with
+ * dvfe_wait), in which every stream s gets exactly what a single-stream tracker fed only that stream's frames would get.
+ * stream_flags[s] as for dvfe_track_image_ex (NULL or all 0: the step dvfe_track_semantic_image enqueues, same graph, same
+ * launches); a skipped stream's exist_inst[s], mask and time0[s] are not read.  DVFE_FRAME_RESET also starts the stream's
+ * instance manager over (as dvfe_track_dynamic_ex2).  A following dvfe_insts_track / dvfe_insts_track_batch of the same frame
+ * obeys the flags: a skipped stream must have 0 boxes and is left untouched, a DVFE_FRAME_NO_RIGHT stream's instances run mono.
+ * flags: DVFE_DYN_DEVICE_INPUT (left / right / mask are device pointers) only.  Invalid stream flags and unknown `flags` bits
+ * return DVFE_ERR_INVALID and change nothing.  dvfe_track_semantic_image == wait for all steps + this with NULL flags + wait. */
+int dvfe_track_semantic_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask,
+                           size_t stream_stride, int pitch, const int* exist_inst, const double* time0,
+                           const uint8_t* stream_flags, unsigned flags);
+
 /* InstsFeatManager::InstsTrack(SemanticImage) preceded by the caller's per-frame instance reset and
  * AddViodeInstances (system/main.cpp:198-210, front_end/dynamic_tracker.cpp:348-493,585-605), for ONE stream.
  * Uses the gray0/gray1 uploaded by the last dvfe_track_semantic_image call of that stream. */
@@ -243,6 +255,22 @@ int dvfe_insts_track_batch(dvfe_tracker* t, const dvfe_inst_in* insts, const int
 int dvfe_track_dynamic_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
                           int pitch, const int* exist_inst, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0,
                           unsigned flags);
+
+/* dvfe_track_dynamic_ex with per-stream frame presence (dvfe_track_dynamic_ex and dvfe_track_dynamic_async are this with
+ * stream_flags = NULL).  stream_flags[s] (NULL or all 0: the plain step, same graph, same launches):
+ *   DVFE_FRAME_SKIP      neither TrackSemanticImage nor InstsTrack is called for the stream: the background as for
+ *                        dvfe_track_image_ex; no per-frame instance reset, no lost_num change, no ManageInstances, last_time and the
+ *                        ROI buffers kept; dvfe_get_features and dvfe_insts_output return 0 records, dvfe_insts_table is unchanged.
+ *                        n_boxes[s] must be 0; the stream's pixels, mask / label image, exist_inst[s] and time0[s] are not read
+ *   DVFE_FRAME_NO_RIGHT  a mono frame for the stream: no cam-1 records for the background or the instances, no TrackRightByPad,
+ *                        the right velocity maps kept
+ *   DVFE_FRAME_RESET     a newly created FeatureTracker and InstsFeatManager for the stream (no points, next_id = 1 before the
+ *                        background detection, prev_time = 0; no instances, every slot free, last_time = 0); boxes allowed (they are
+ *                        the new manager's first frame); may be combined with NO_RIGHT
+ * Unknown bits, SKIP|RESET and boxes for a skipped stream return DVFE_ERR_INVALID and change nothing. */
+int dvfe_track_dynamic_ex2(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
+                           int pitch, const int* exist_inst, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0,
+                           const uint8_t* stream_flags, unsigned flags);
 
 /* FeatureBackground of stream s of the last step: n_out records, sorted by (id, cam). */
 int dvfe_get_features(dvfe_tracker* t, int stream, dvfe_obs* out, int cap, int* n_out);

@@ -442,24 +442,15 @@ public:
     void TrackDynamicAsync(const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask, size_t stream_stride, int step,
                            const std::vector<int>& exist_inst, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,
                            const std::vector<double>& time0) {
-        check(time0);
-        if ((int)exist_inst.size() != cfg_.n_streams || (int)boxes2d.size() != cfg_.n_streams)
-            throw std::runtime_error("BatchFeatureTracker: one exist_inst / box list per stream expected");
-        std::vector<dvfe_inst_in> in;
-        std::vector<int> n(boxes2d.size());
-        for (size_t s = 0; s < boxes2d.size(); s++) {
-            n[s] = (int)boxes2d[s].size();
-            for (const Box2D::Ptr& b : boxes2d[s]) {
-                dvfe_inst_in d{};
-                d.track_id = (uint32_t)b->track_id;
-                d.x = (int)b->rect.x; d.y = (int)b->rect.y; d.w = (int)b->rect.width; d.h = (int)b->rect.height;
-                d.mask = b->roi ? b->roi->mask_cv.data : nullptr; d.mask_pitch = b->roi ? b->roi->mask_cv.step : 0;
-                in.push_back(d);
-            }
-        }
-        if (dvfe_track_dynamic_async(h_, left, right, inv_merge_mask, stream_stride, step, exist_inst.data(),
-                                     in.empty() ? nullptr : in.data(), n.data(), time0.data()) != DVFE_OK)
-            throw std::runtime_error(dvfe_last_error(h_));
+        dynamic(left, right, inv_merge_mask, stream_stride, step, exist_inst, boxes2d, time0, nullptr);
+    }
+    // The same with per-stream frame presence: stream_flags[s] is 0 or DVFE_FRAME_SKIP / DVFE_FRAME_NO_RIGHT / DVFE_FRAME_RESET
+    // (dvfe_track_dynamic_ex2); a skipped stream has an empty box list, and its time0 and exist_inst are not read.
+    void TrackDynamicAsync(const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask, size_t stream_stride, int step,
+                           const std::vector<int>& exist_inst, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,
+                           const std::vector<double>& time0, const std::vector<uint8_t>& stream_flags) {
+        if ((int)stream_flags.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one stream flag per stream expected");
+        dynamic(left, right, inv_merge_mask, stream_stride, step, exist_inst, boxes2d, time0, stream_flags.data());
     }
     // the oldest enqueued frame is finished: Features() / InstsOutput() return its results
     void Wait() {
@@ -497,6 +488,28 @@ public:
     }
 
 private:
+    void dynamic(const uint8_t* left, const uint8_t* right, const uint8_t* inv_merge_mask, size_t stream_stride, int step,
+                 const std::vector<int>& exist_inst, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,
+                 const std::vector<double>& time0, const uint8_t* stream_flags) {
+        check(time0);
+        if ((int)exist_inst.size() != cfg_.n_streams || (int)boxes2d.size() != cfg_.n_streams)
+            throw std::runtime_error("BatchFeatureTracker: one exist_inst / box list per stream expected");
+        std::vector<dvfe_inst_in> in;
+        std::vector<int> n(boxes2d.size());
+        for (size_t s = 0; s < boxes2d.size(); s++) {
+            n[s] = (int)boxes2d[s].size();
+            for (const Box2D::Ptr& b : boxes2d[s]) {
+                dvfe_inst_in d{};
+                d.track_id = (uint32_t)b->track_id;
+                d.x = (int)b->rect.x; d.y = (int)b->rect.y; d.w = (int)b->rect.width; d.h = (int)b->rect.height;
+                d.mask = b->roi ? b->roi->mask_cv.data : nullptr; d.mask_pitch = b->roi ? b->roi->mask_cv.step : 0;
+                in.push_back(d);
+            }
+        }
+        if (dvfe_track_dynamic_ex2(h_, left, right, inv_merge_mask, stream_stride, step, exist_inst.data(),
+                                   in.empty() ? nullptr : in.data(), n.data(), time0.data(), stream_flags, 0u) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
     void check(const std::vector<double>& time0) const {
         if ((int)time0.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one time0 per stream expected");
     }

@@ -1,7 +1,8 @@
 // dvfe_config_from_yaml — replaces fe_para::SetParameters (dynamic_vins/src/front_end/front_end_parameters.cpp:17-40),
 // the cfg keys the path reads (dynamic_vins/src/utils/parameters.cpp:19-147: num_of_cam, image_width/height,
 // cam0_calib, cam1_calib) and the camodocal PINHOLE yaml reader
-// (/root/reference/camera_models/src/camera_models/PinholeCamera.cc:80-140, readFromYamlFile).
+// (/root/reference/camera_models/src/camera_models/PinholeCamera.cc:80-140, readFromYamlFile), which dvfe_camera_from_yaml
+// exposes on its own for per-stream calibrations.
 // The reference parses with cv::FileStorage; the files are flat "key: value" yaml (OpenCV "%YAML:1.0" dialect)
 // with at most one level of nesting and unique leaf names, which is all this reader supports.
 #include <stdio.h>
@@ -77,6 +78,14 @@ int read_camera(const std::string& path, dvfe_camera* cam) {
     return DVFE_OK;
 }
 }  // namespace
+
+extern "C" int dvfe_camera_from_yaml(const char* path, dvfe_camera* cam) {
+    if (!path || !cam) { dvfe_set_error("camera_from_yaml: null argument"); return DVFE_ERR_INVALID; }
+    dvfe_camera c;
+    const int rc = read_camera(path, &c);
+    if (rc == DVFE_OK) *cam = c;
+    return rc;
+}
 
 extern "C" int dvfe_config_from_yaml(const char* config_path, dvfe_config* cfg) {
     if (!config_path || !cfg) { dvfe_set_error("config_from_yaml: null argument"); return DVFE_ERR_INVALID; }

@@ -134,6 +134,18 @@ int grp_set_maps(dvfe_tracker* t, int cam, const int16_t* map1, const uint16_t* 
     return DVFE_OK;
 }
 
+int grp_set_stream_camera(dvfe_tracker* t, int stream, const dvfe_camera* cam0, const dvfe_camera* cam1) {
+    dvfe_tracker* leaf; int local;
+    DVFE_CHECK(grp_route(t, stream, &leaf, &local));
+    return dvfe_set_stream_camera(leaf, local, cam0, cam1);
+}
+
+int grp_set_stream_maps(dvfe_tracker* t, int stream, int cam, const int16_t* map1, const uint16_t* map2) {
+    dvfe_tracker* leaf; int local;
+    DVFE_CHECK(grp_route(t, stream, &leaf, &local));
+    return dvfe_set_stream_undistort_maps(leaf, local, cam, map1, map2);
+}
+
 int grp_set_lk_mode(dvfe_tracker* t, int site, int back_max_level, double fb) {
     for (dvfe_tracker* g : t->groups) DVFE_CHECK(dvfe_set_lk_mode_site(g, site, back_max_level, fb));
     return DVFE_OK;

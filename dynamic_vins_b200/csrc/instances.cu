@@ -464,11 +464,12 @@ static int insts_track_streams(dvfe_tracker* t, int s0, int s1, const dvfe_inst_
         // ErodeMask(roi mask, 5) + discs(min_dynamic_dist) + goodFeaturesToTrack on the ROI + ids (:418-446)
         DVFE_CHECK(launch_erode_jobs(C.erode.d, nv, max_rw, max_rh, st));
         DVFE_CHECK(launch_gftt(C.gftt.d, nullptr, nv, max_rw, max_rh, cap, st));
-        // UndistortedPointsWithAddOffset(cam0) + PtsVelocity(curr_time - last_time) (:448-457)
-        DVFE_CHECK(launch_left_post(V, n_sets, cap, t->cam0, C.dt.d + set0, C.offs.d + set0, st, C.act_vis.d + set0));
+        // UndistortedPointsWithAddOffset(cam0) + PtsVelocity(curr_time - last_time) (:448-457), each stream with the cameras of
+        // its background step: the camera table is only rewritten ahead of the next step's kernels
+        DVFE_CHECK(launch_left_post(V, n_sets, cap, t->d_cam + s0, MI, C.dt.d + set0, C.offs.d + set0, st, C.act_vis.d + set0));
         // TrackRightByPad + RightUndistortedPts + RightPtsVelocity (:462-471), then the Output() records
         if (n_stereo > 0) DVFE_CHECK(launch_lk(C.lk_s.d, n_stereo, cap, t->cfg.lk_max_level, t->cfg.flow_back, st));
-        DVFE_CHECK(launch_inst_post_pack(V, n_sets, cap, t->cam1, C.dt.d + set0, C.act_vis.d + set0, stereo_now ? 1 : 0,
+        DVFE_CHECK(launch_inst_post_pack(V, n_sets, cap, t->d_cam + B + s0, MI, C.dt.d + set0, C.act_vis.d + set0, stereo_now ? 1 : 0,
                                          partial ? C.lane.d + set0 : nullptr, C.inst_id.d + set0, C.d_out + o, C.d_n + set0, st));
         C.has_records = true;
     }

@@ -56,7 +56,13 @@ struct IngestArgs {
     int w, h, n_img;
     int keep_channels;           // 1: plain cv::remap of all channels (seam op); 0: output gray
 };
-int launch_ingest(const IngestArgs& a, cudaStream_t st);
+// The maps of one image (per-stream undistortion): map1 == null = not remapped, only copied / converted to gray
+struct IngestMaps {
+    const short* map1;
+    const unsigned short* map2;
+};
+// d_maps (nullable): [n_img] per-image maps in place of a.map1 / a.map2 (gray output only)
+int launch_ingest(const IngestArgs& a, cudaStream_t st, const IngestMaps* d_maps = nullptr);
 
 int launch_build_pyramids_jobs(const PyrJob* d_jobs, int n_jobs, int max_w, int max_h, int max_levels, cudaStream_t st);
 int launch_crop_jobs(const CropJob* d_jobs, int n_jobs, int max_w, int max_h, cudaStream_t st);

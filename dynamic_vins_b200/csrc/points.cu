@@ -115,7 +115,10 @@ int launch_compact(const PointSetArrays& S, int n_sets, int cap, cudaStream_t st
 }
 
 // ---- UndistortedPts + PtsVelocity for the left image; un[] holds prev_id_pts on entry, curr on exit ------
-__global__ void __launch_bounds__(128) k_left_post(PointSetArrays S, int cap, CamParams cam, const double* __restrict__ dt,
+// cams: the camera of each stream; set `set` belongs to stream set / sets_per_cam (1 for the background, max_instances for the
+// instance sets)
+__global__ void __launch_bounds__(128) k_left_post(PointSetArrays S, int cap, const CamParams* __restrict__ cams, int sets_per_cam,
+                                                   const double* __restrict__ dt,
                                                    const float2* __restrict__ offset /* nullable, per set */,
                                                    const uint8_t* __restrict__ active) {
     const int set = blockIdx.y;
@@ -125,6 +128,7 @@ __global__ void __launch_bounds__(128) k_left_post(PointSetArrays S, int cap, Ca
     const size_t k = (size_t)set * cap + i;
     const float2 p = S.pts[k];
     const float2 off = offset ? offset[set] : make_float2(0.f, 0.f);
+    const CamParams cam = cams[set / sets_per_cam];
     const float2 un = lift_projective(cam, p.x + off.x, p.y + off.y);
     float2 vel = make_float2(0.f, 0.f);
     if (S.track_cnt[k] > 1) {          // id is in prev_id_pts  <=>  the point was tracked from the last frame
@@ -139,11 +143,11 @@ __global__ void __launch_bounds__(128) k_left_post(PointSetArrays S, int cap, Ca
     S.vel[k] = vel;
 }
 
-int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam, const double* d_dt,
+int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams, int sets_per_cam, const double* d_dt,
                      const float2* d_offset, cudaStream_t st, const uint8_t* d_active) {
     if (n_sets <= 0) return DVFE_OK;
     dim3 grid((cap + 127) / 128, n_sets);
-    DVFE_LAUNCH(k_left_post, grid, 128, 0, st, S, cap, cam, d_dt, d_offset, d_active);
+    DVFE_LAUNCH(k_left_post, grid, 128, 0, st, S, cap, d_cams, sets_per_cam, d_dt, d_offset, d_active);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }
@@ -153,7 +157,9 @@ int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamPara
 // ascending id order (survivors keep their order, new ids are appended).
 // lanes (nullable, per set): 0 = the set had no frame in this step (no records, nothing written), else LANE_PRESENT and
 // LANE_STEREO when it had a right image; null = every set present, with a right image iff stereo_now.
-__global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int cap, CamParams cam1, const double* __restrict__ dt,
+// cams1: the right camera of each set (one set per stream).
+__global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int cap, const CamParams* __restrict__ cams1,
+                                                         const double* __restrict__ dt,
                                                          int stereo_all, const uint8_t* __restrict__ lanes,
                                                          dvfe_obs* __restrict__ obs, int* __restrict__ n_obs) {
     __shared__ int s_warp[8];
@@ -176,6 +182,7 @@ __global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int c
         float2 run = make_float2(0, 0), rvel = run, rp = run;
         if (has_r) {
             rp = S.rpts[o + i];
+            const CamParams cam1 = cams1[set];
             run = lift_projective(cam1, rp.x, rp.y);
             if (S.rprev_valid[o + i]) {
                 const float2 prev = S.rprev_un[o + i];
@@ -217,10 +224,10 @@ __global__ void __launch_bounds__(256) k_right_post_pack(PointSetArrays S, int c
     if (tid == 0) n_obs[set] = n + s_base;
 }
 
-int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
+int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, const double* d_dt,
                            int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st, const uint8_t* d_lane) {
     if (n_sets <= 0) return DVFE_OK;
-    DVFE_LAUNCH(k_right_post_pack, n_sets, 256, 0, st, S, cap, cam1, d_dt, stereo_now, d_lane, obs, n_obs);
+    DVFE_LAUNCH(k_right_post_pack, n_sets, 256, 0, st, S, cap, d_cams1, d_dt, stereo_now, d_lane, obs, n_obs);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }
@@ -228,7 +235,9 @@ int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const C
 // ---- instances: RightUndistortedPts + RightPtsVelocity + InstsFeatManager::Output record -----------------------
 // (front_end/dynamic_tracker.cpp:462-471, 521-577).  One record per point at out[set*cap + i]; ids ascend with i.
 // lanes (nullable, per set): whether the set's stream had a right image (LANE_STEREO) in place of stereo_all for every set.
-__global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int cap, CamParams cam1, const double* __restrict__ dt,
+// cams1: the right camera of each stream, set `set` belonging to stream set / sets_per_cam.
+__global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int cap, const CamParams* __restrict__ cams1,
+                                                        int sets_per_cam, const double* __restrict__ dt,
                                                         const uint8_t* __restrict__ active, int stereo_all,
                                                         const uint8_t* __restrict__ lanes, const uint32_t* __restrict__ inst_id,
                                                         dvfe_inst_obs* __restrict__ out, int* __restrict__ n_out) {
@@ -245,6 +254,7 @@ __global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int ca
     float2 run = make_float2(0, 0), rvel = run;
     if (has_r) {
         const float2 rp = S.rpts[k];
+        const CamParams cam1 = cams1[set / sets_per_cam];
         run = lift_projective(cam1, rp.x, rp.y);
         if (S.rprev_valid[k]) {
             const float2 prev = S.rprev_un[k];
@@ -270,12 +280,12 @@ __global__ void __launch_bounds__(128) k_inst_post_pack(PointSetArrays S, int ca
     out[k] = r;
 }
 
-int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
-                          const uint8_t* d_active, int stereo_now, const uint8_t* d_lane, const uint32_t* d_inst_id,
-                          dvfe_inst_obs* out, int* d_n_out, cudaStream_t st) {
+int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, int sets_per_cam,
+                          const double* d_dt, const uint8_t* d_active, int stereo_now, const uint8_t* d_lane,
+                          const uint32_t* d_inst_id, dvfe_inst_obs* out, int* d_n_out, cudaStream_t st) {
     if (n_sets <= 0) return DVFE_OK;
     dim3 grid((cap + 127) / 128, n_sets);
-    DVFE_LAUNCH(k_inst_post_pack, grid, 128, 0, st, S, cap, cam1, d_dt, d_active, stereo_now, d_lane, d_inst_id, out, d_n_out);
+    DVFE_LAUNCH(k_inst_post_pack, grid, 128, 0, st, S, cap, d_cams1, sets_per_cam, d_dt, d_active, stereo_now, d_lane, d_inst_id, out, d_n_out);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }

@@ -53,7 +53,8 @@ __global__ void __launch_bounds__(256) k_merge_masks(const uint8_t* __restrict__
 // w = {(32-fx)(32-fy), fx(32-fy), (32-fx)fy, fx fy} * 32 (exact shorts, sum 2^15), taps outside the source = 0,
 // dst = (sum w * tap + 2^14) >> 15 per channel == (sum (w/32) * tap + 512) >> 10.  One thread = 4 consecutive output
 // pixels of up to INGEST_SPT streams: the map entries are loaded once and reused across streams (the maps are shared
-// by all streams and stay in L2), the source taps are gathers served by L1/L2.
+// by all streams and stay in L2), the source taps are gathers served by L1/L2.  Streams with their own maps
+// (dvfe_set_stream_undistort_maps) go through k_ingest_remap_each, which decodes each image's maps for that image.
 #define INGEST_SPT 8
 
 // taps of one output pixel whose 2 x 2 footprint is not fully inside the source (border pixels only)
@@ -115,7 +116,36 @@ __device__ __forceinline__ unsigned gray_of(unsigned b, unsigned g, unsigned r) 
     return (b * 3735u + g * 19235u + r * 9798u + 16384u) >> 15;
 }
 
-// Unmapped images (gray copy / BGR -> gray): 4 consecutive output pixels per thread, word loads, one 32-bit store.
+// Unmapped images (gray copy / BGR -> gray): 4 consecutive output pixels x0.. of row y of image s (n of them inside the row),
+// word loads, one 32-bit store.
+template <int CH, bool KEEP>
+__device__ __forceinline__ void ingest_rows_px(const IngestArgs& a, int s, int x0, int y, int n) {
+    const uint8_t* __restrict__ row = a.src + (size_t)s * a.src_stride + (size_t)y * a.src_pitch + x0 * CH;
+    uint8_t* d = a.dst + (size_t)s * a.dst_stride + (size_t)y * a.dst_pitch + x0 * (KEEP ? CH : 1);
+    if (KEEP) {
+        for (int i = 0; i < n * CH; i++) d[i] = __ldg(row + i);
+        return;
+    }
+    unsigned packed = 0;
+    if (n == 4 && ((uintptr_t)row & 3) == 0) {
+        const unsigned* p = reinterpret_cast<const unsigned*>(row);
+        if (CH == 3) {
+            const unsigned w0 = __ldg(p), w1 = __ldg(p + 1), w2 = __ldg(p + 2);   // B G R B | G R B G | R B G R
+            packed = gray_of(w0 & 255, (w0 >> 8) & 255, (w0 >> 16) & 255) |
+                     gray_of(w0 >> 24, w1 & 255, (w1 >> 8) & 255) << 8 |
+                     gray_of((w1 >> 16) & 255, w1 >> 24, w2 & 255) << 16 |
+                     gray_of((w2 >> 8) & 255, (w2 >> 16) & 255, w2 >> 24) << 24;
+        } else {
+            packed = __ldg(p);
+        }
+    } else {
+        for (int i = 0; i < n; i++)
+            packed |= (CH == 3 ? gray_of(__ldg(row + 3 * i), __ldg(row + 3 * i + 1), __ldg(row + 3 * i + 2)) : __ldg(row + i)) << (8 * i);
+    }
+    if (n == 4 && ((uintptr_t)d & 3) == 0) *reinterpret_cast<unsigned*>(d) = packed;
+    else for (int i = 0; i < n; i++) d[i] = (uint8_t)(packed >> (8 * i));
+}
+
 template <int CH, bool KEEP>
 __global__ void __launch_bounds__(256) k_ingest_rows(IngestArgs a) {
     const int x0 = (blockIdx.x * 32 + threadIdx.x) * 4;
@@ -123,31 +153,72 @@ __global__ void __launch_bounds__(256) k_ingest_rows(IngestArgs a) {
     if (x0 >= a.w || y >= a.h) return;
     const int n = min(4, a.w - x0);
     const int s_end = min(a.n_img, (int)(blockIdx.z + 1) * INGEST_SPT);
-    for (int s = blockIdx.z * INGEST_SPT; s < s_end; s++) {
-        const uint8_t* __restrict__ row = a.src + (size_t)s * a.src_stride + (size_t)y * a.src_pitch + x0 * CH;
-        uint8_t* d = a.dst + (size_t)s * a.dst_stride + (size_t)y * a.dst_pitch + x0 * (KEEP ? CH : 1);
-        if (KEEP) {
-            for (int i = 0; i < n * CH; i++) d[i] = __ldg(row + i);
-            continue;
-        }
-        unsigned packed = 0;
-        if (n == 4 && ((uintptr_t)row & 3) == 0) {
-            const unsigned* p = reinterpret_cast<const unsigned*>(row);
-            if (CH == 3) {
-                const unsigned w0 = __ldg(p), w1 = __ldg(p + 1), w2 = __ldg(p + 2);   // B G R B | G R B G | R B G R
-                packed = gray_of(w0 & 255, (w0 >> 8) & 255, (w0 >> 16) & 255) |
-                         gray_of(w0 >> 24, w1 & 255, (w1 >> 8) & 255) << 8 |
-                         gray_of((w1 >> 16) & 255, w1 >> 24, w2 & 255) << 16 |
-                         gray_of((w2 >> 8) & 255, (w2 >> 16) & 255, w2 >> 24) << 24;
-            } else {
-                packed = __ldg(p);
+    for (int s = blockIdx.z * INGEST_SPT; s < s_end; s++) ingest_rows_px<CH, KEEP>(a, s, x0, y, n);
+}
+
+// The body of k_ingest_remap (below) for the maps (map1, map2) and the images [s_begin, s_end): the per-image kernel's remap.
+// k_ingest_remap keeps its own copy of these lines: written as a call of this function it compiles to 4-11 more registers.
+template <int CH, bool KEEP>
+__device__ __forceinline__ void remap_images(const IngestArgs& a, const short* map1, const unsigned short* map2,
+                                             int xb, int y, int s_begin, int s_end) {
+    int off[4], wa[4], wb[4];          // byte offset of tap (0,0); weights packed w00 | w01 << 16, w10 | w11 << 16
+    short sxs[4], sys[4];
+    unsigned inside = 0;
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int x = xb + 32 * i;
+        off[i] = 0; wa[i] = 0; wb[i] = 0; sxs[i] = 0; sys[i] = 0;
+        if (x < a.w) {
+            const size_t m = (size_t)y * a.w + x;
+            const unsigned xy = __ldg(reinterpret_cast<const unsigned*>(map1) + m);
+            const unsigned f = __ldg(map2 + m);
+            const int sx = (short)(xy & 0xffff), sy = (short)(xy >> 16);
+            const int fx = f & 31, fy = (f >> 5) & 31;
+            sxs[i] = (short)sx; sys[i] = (short)sy;
+            wa[i] = ((32 - fx) * (32 - fy)) | (fx * (32 - fy)) << 16;
+            wb[i] = ((32 - fx) * fy) | (fx * fy) << 16;
+            // inside = the 2 x 2 footprint is in the image AND (3 channels) the 12 aligned bytes the word path reads around
+            // each 6-byte row stay inside the image buffer; everything else takes the bounds-checked path
+            if ((unsigned)sx < (unsigned)(a.w - 1) && (unsigned)sy < (unsigned)(a.h - 1) &&
+                (CH != 3 || (sy + 1) * a.src_pitch + sx * CH + 12 <= a.h * a.src_pitch)) {
+                inside |= 1u << i;
+                off[i] = sy * a.src_pitch + sx * CH;
             }
-        } else {
-            for (int i = 0; i < n; i++)
-                packed |= (CH == 3 ? gray_of(__ldg(row + 3 * i), __ldg(row + 3 * i + 1), __ldg(row + 3 * i + 2)) : __ldg(row + i)) << (8 * i);
         }
-        if (n == 4 && ((uintptr_t)d & 3) == 0) *reinterpret_cast<unsigned*>(d) = packed;
-        else for (int i = 0; i < n; i++) d[i] = (uint8_t)(packed >> (8 * i));
+    }
+    for (int s = s_begin; s < s_end; s++) {
+        const uint8_t* __restrict__ img = a.src + (size_t)s * a.src_stride;
+        uint8_t* drow = a.dst + (size_t)s * a.dst_stride + (size_t)y * a.dst_pitch;
+        unsigned res[4][CH];
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            if (xb + 32 * i >= a.w) break;
+            const int w00 = wa[i] & 0xffff, w01 = wa[i] >> 16, w10 = wb[i] & 0xffff, w11 = wb[i] >> 16;
+            if (inside >> i & 1) {
+                const uint8_t* p = img + off[i];
+                if (CH == 3) {
+                    remap_bgr_words(p, a.src_pitch, wa[i], wb[i], res[i]);
+                } else {
+#pragma unroll
+                    for (int c = 0; c < CH; c++)
+                        res[i][c] = (unsigned)(w00 * __ldg(p + c) + w01 * __ldg(p + CH + c) + w10 * __ldg(p + a.src_pitch + c) +
+                                               w11 * __ldg(p + a.src_pitch + CH + c) + 512) >> 10;
+                }
+            } else {
+                remap_taps_border<CH>(img, a.src_pitch, a.w, a.h, sxs[i], sys[i], w00, w01, w10, w11, res[i]);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const int x = xb + 32 * i;
+            if (x >= a.w) break;
+            if (KEEP) {
+#pragma unroll
+                for (int c = 0; c < CH; c++) drow[x * CH + c] = (uint8_t)res[i][c];
+            } else {
+                drow[x] = (uint8_t)(CH == 3 ? gray_of(res[i][0], res[i][1], res[i][2]) : res[i][0]);
+            }
+        }
     }
 }
 
@@ -224,11 +295,35 @@ __global__ void __launch_bounds__(256) k_ingest_remap(IngestArgs a) {
     }
 }
 
-int launch_ingest(const IngestArgs& a, cudaStream_t st) {
+// Per-image maps (streams with their own undistortion maps): image blockIdx.z is remapped with maps[blockIdx.z], decoded for that
+// image alone; an image without maps gets the pixels of k_ingest_rows.  The same tile of output pixels per block as the two
+// kernels above, and the same arithmetic, so every image gets the bytes the shared-map kernel (or k_ingest_rows) writes for its maps.
+template <int CH>
+__global__ void __launch_bounds__(256) k_ingest_remap_each(IngestArgs a, const IngestMaps* __restrict__ maps) {
+    const int s = blockIdx.z;
+    const int y = blockIdx.y * 8 + threadIdx.y;
+    const IngestMaps m = maps[s];
+    if (m.map1 == nullptr) {
+        const int x0 = (blockIdx.x * 32 + threadIdx.x) * 4;
+        if (x0 >= a.w || y >= a.h) return;
+        ingest_rows_px<CH, false>(a, s, x0, y, min(4, a.w - x0));
+        return;
+    }
+    const int xb = blockIdx.x * 128 + threadIdx.x;
+    if (xb >= a.w || y >= a.h) return;
+    remap_images<CH, false>(a, m.map1, m.map2, xb, y, s, s + 1);
+}
+
+int launch_ingest(const IngestArgs& a, cudaStream_t st, const IngestMaps* d_maps) {
     if (a.n_img <= 0) return DVFE_OK;
     const int nz = (a.n_img + INGEST_SPT - 1) / INGEST_SPT;
     dim3 blk(32, 8), grid((a.w + 127) / 128, (a.h + 7) / 8, nz);
-    if (a.map1) {
+    if (d_maps) {
+        if (a.keep_channels) { dvfe_set_error("ingest: per-image maps write gray images only"); return DVFE_ERR_INVALID; }
+        const dim3 grid_each(grid.x, grid.y, a.n_img);
+        if (a.ch == 3) DVFE_LAUNCH((k_ingest_remap_each<3>), grid_each, blk, 0, st, a, d_maps);
+        else DVFE_LAUNCH((k_ingest_remap_each<1>), grid_each, blk, 0, st, a, d_maps);
+    } else if (a.map1) {
         if (a.ch == 3 && a.keep_channels) DVFE_LAUNCH((k_ingest_remap<3, true>), grid, blk, 0, st, a);
         else if (a.ch == 3) DVFE_LAUNCH((k_ingest_remap<3, false>), grid, blk, 0, st, a);
         else DVFE_LAUNCH((k_ingest_remap<1, false>), grid, blk, 0, st, a);

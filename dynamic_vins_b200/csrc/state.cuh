@@ -21,11 +21,12 @@ struct PointSetArrays {
 int launch_compact(const PointSetArrays& S, int n_sets, int cap, cudaStream_t st, const uint8_t* d_active = nullptr,
                    int* d_old_idx = nullptr);
 struct CamParams;
-int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam, const double* d_dt,
+// d_cams / d_cams1: device camera table, one entry per stream; set s uses entry s / sets_per_cam
+int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams, int sets_per_cam, const double* d_dt,
                      const float2* d_offset, cudaStream_t st, const uint8_t* d_active = nullptr);
-int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
-                          const uint8_t* d_active, int stereo_now, const uint8_t* d_lane, const uint32_t* d_inst_id,
-                          dvfe_inst_obs* out, int* d_n_out, cudaStream_t st);
+int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, int sets_per_cam,
+                          const double* d_dt, const uint8_t* d_active, int stereo_now, const uint8_t* d_lane,
+                          const uint32_t* d_inst_id, dvfe_inst_obs* out, int* d_n_out, cudaStream_t st);
 int launch_clear_sets(int* d_n, const uint8_t* d_flags, int n_sets, cudaStream_t st);
-int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams& cam1, const double* d_dt,
+int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, const double* d_dt,
                            int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st, const uint8_t* d_lane = nullptr);

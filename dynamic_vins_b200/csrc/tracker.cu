@@ -3,6 +3,7 @@
 // 757-837) and the seam-level operators.  Host code only orchestrates launches; no pixel or point
 // arithmetic happens on the CPU and there is no fallback when no CUDA device is present.
 #include <limits.h>
+#include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -162,8 +163,8 @@ extern "C" int dvfe_create(const dvfe_config* cfg, dvfe_tracker** out) {
     t->B = cfg->n_streams; t->W = cfg->width; t->H = cfg->height; t->cap = cfg->max_cnt;
     // levels for the forward maxLevel, the backward call's maxLevel 1 and the cv::cuda call pattern's 3 (dvfe_set_lk_mode)
     t->desc = make_pyr_desc(t->W, t->H, cfg->lk_max_level > 3 ? cfg->lk_max_level : 3);
-    t->cam0 = make_cam(cfg->cam0);
-    t->cam1 = make_cam(cfg->cam1);
+    t->cams.assign((size_t)2 * t->B, make_cam(cfg->cam0));          // every stream with the config's cameras
+    for (int s = 0; s < t->B; s++) t->cams[(size_t)t->B + s] = make_cam(cfg->cam1);
     int rc = t->init();
     if (rc != DVFE_OK) { dvfe_destroy(t); return rc; }
     *out = t;
@@ -205,6 +206,15 @@ int dvfe_tracker::init() {
     DVFE_CHECK(dmalloc(&d_pgroups[1], (size_t)B));
     DVFE_CHECK(dmalloc(&d_pjobs, (size_t)B));
     DVFE_CHECK(dmalloc(&d_zero, (size_t)1));
+    DVFE_CHECK(dmalloc(&d_cam, cams.size()));
+    DVFE_CUDA(cudaMemcpy(d_cam, cams.data(), cams.size() * sizeof(CamParams), cudaMemcpyHostToDevice));
+    for (int p = 0; p < 2; p++) DVFE_CUDA(cudaMallocHost((void**)&h_cam[p], cams.size() * sizeof(CamParams)));
+    for (int cam = 0; cam < 2; cam++) {
+        own_maps[cam].assign(B, 0);
+        s_map1[cam].assign(B, nullptr);
+        s_map2[cam].assign(B, nullptr);
+        DVFE_CHECK(dmalloc(&d_imaps[cam], (size_t)B));          // all null: no maps
+    }
     for (int p = 0; p < 2; p++) {
         DVFE_CUDA(cudaMallocHost((void**)&h_sflags[p], (size_t)B));
         memset(h_sflags[p], 0, (size_t)B);
@@ -327,8 +337,15 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     cudaFree(t->d_old_idx);
     cudaFree(t->d_sflags); cudaFree(t->d_lane); cudaFree(t->d_pgroups[0]); cudaFree(t->d_pgroups[1]); cudaFree(t->d_pjobs);
     cudaFree(t->d_zero);
+    cudaFree(t->d_cam);
+    for (int cam = 0; cam < 2; cam++) {
+        cudaFree(t->d_imaps[cam]);
+        for (short* m : t->s_map1[cam]) cudaFree(m);
+        for (unsigned short* m : t->s_map2[cam]) cudaFree(m);
+    }
     for (int p = 0; p < 2; p++) {
         cudaFreeHost(t->h_sflags[p]);
+        cudaFreeHost(t->h_cam[p]);
         cudaFree(t->d_obs[p]); cudaFree(t->d_nobs[p]);
         if (t->ev_packed[p]) cudaEventDestroy(t->ev_packed[p]);
         if (t->ev_resp[p]) cudaEventDestroy(t->ev_resp[p]);
@@ -435,8 +452,8 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
         DVFE_CUDA(cudaEventRecord(ev_rpyr[par], rs));
     }
     mark(ST_GFTT_SELECT + 1);
-    // UndistortedPts(cam0) + PtsVelocity
-    DVFE_CHECK(launch_left_post(bg, B, cap, cam0, d_dt, nullptr, st, lane));
+    // UndistortedPts(cam0) + PtsVelocity, each stream with its own cam0
+    DVFE_CHECK(launch_left_post(bg, B, cap, d_cam, 1, d_dt, nullptr, st, lane));
     mark(ST_LEFT_POST + 1);
     if (stereo_now) DVFE_CUDA(cudaStreamWaitEvent(st, ev_rpyr[par], 0));
     if (stereo_now)   // FeatureTrackByLK(gray0, gray1, curr_points) — left points are kept when the match fails
@@ -445,7 +462,7 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
                              lk_fb_thresh[semantic ? DVFE_LK_SEMANTIC_STEREO : DVFE_LK_RAW_STEREO],
                              LK_TCACHE_WRITE | (reuse ? LK_TCACHE_READ_BWD : 0), reuse ? lk_back_level[site_t] : -1));
     mark(ST_LK_STEREO + 1);
-    DVFE_CHECK(launch_right_post_pack(bg, B, cap, cam1, d_dt, stereo_now ? 1 : 0, d_obs[par], d_nobs[par], st, lane));
+    DVFE_CHECK(launch_right_post_pack(bg, B, cap, d_cam + B, d_dt, stereo_now ? 1 : 0, d_obs[par], d_nobs[par], st, lane));
     mark(ST_PACK + 1);
     return DVFE_OK;
 }
@@ -495,6 +512,13 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
         for (int s = 0; s < B; s++) h_dt[par][s] = time0[s] - prev_time[s];       // cur_time - prev_time
     }
     prof_step[par] = prof;
+    if (cam_dirty) {
+        // the calibration of this step (dvfe_set_stream_camera), ahead of its kernels and behind those of every earlier step.
+        // h_cam[par] was last the source of step k-2's copy, which has completed (wait_slot).
+        memcpy(h_cam[par], cams.data(), cams.size() * sizeof(CamParams));
+        DVFE_CUDA(cudaMemcpyAsync(d_cam, h_cam[par], cams.size() * sizeof(CamParams), cudaMemcpyHostToDevice, st));
+        cam_dirty = false;
+    }
     // everything step k-1 (background and instances) put on the compute stream lies before this point
     DVFE_CUDA(cudaEventRecord(ev_begin[par], st));
     if (use_graphs && !prof) {
@@ -613,15 +637,29 @@ uint8_t* dvfe_tracker::level0(int cam) const {
     return (cam ? right_slot(frames) : left_slot(frames)) + L0.offset + (size_t)DVFE_PADY * L0.pitch + DVFE_PADX;
 }
 
-// remap (if camera `cam` has maps) + gray conversion of B device images into level 0 of this step's pyramid slot
+// remap (if camera `cam` has maps) + gray conversion of B device images into level 0 of this step's pyramid slot: the
+// shared-map kernel when every stream of the camera uses the same maps (or none), the per-image kernel otherwise
 int dvfe_tracker::ingest(const uint8_t* d_src, size_t stream_stride, int pitch, int cam, cudaStream_t s) {
     IngestArgs a;
     a.src = d_src; a.src_stride = stream_stride; a.src_pitch = pitch; a.ch = in_ch;
-    a.map1 = d_map1[cam]; a.map2 = d_map2[cam];
+    a.map1 = maps_uniform[cam] ? stream_map1(cam, 0) : nullptr;
+    a.map2 = maps_uniform[cam] ? stream_map2(cam, 0) : nullptr;
     a.dst = level0(cam);
     a.dst_stride = desc.bytes; a.dst_pitch = desc.lv[0].pitch;
     a.w = W; a.h = H; a.n_img = B; a.keep_channels = 0;
-    return launch_ingest(a, s);
+    return launch_ingest(a, s, maps_uniform[cam] ? nullptr : d_imaps[cam]);
+}
+
+int dvfe_tracker::update_maps(int cam) {
+    std::vector<IngestMaps> m(B);
+    bool uniform = true;
+    for (int s = 0; s < B; s++) {
+        m[s].map1 = stream_map1(cam, s); m[s].map2 = stream_map2(cam, s);
+        uniform = uniform && m[s].map1 == m[0].map1;
+    }
+    maps_uniform[cam] = uniform;
+    DVFE_CUDA(cudaMemcpy(d_imaps[cam], m.data(), B * sizeof(IngestMaps), cudaMemcpyHostToDevice));
+    return DVFE_OK;
 }
 
 // B host images of H rows of `row` bytes -> device memory, on the upload stream.  Into the dense staging: one linear copy
@@ -706,6 +744,8 @@ int dvfe_tracker::size_stage() {
 
 int grp_set_input(dvfe_tracker* t, int channels);
 int grp_set_maps(dvfe_tracker* t, int cam, const int16_t* map1, const uint16_t* map2);
+int grp_set_stream_camera(dvfe_tracker* t, int stream, const dvfe_camera* cam0, const dvfe_camera* cam1);
+int grp_set_stream_maps(dvfe_tracker* t, int stream, int cam, const int16_t* map1, const uint16_t* map2);
 
 extern "C" int dvfe_set_input(dvfe_tracker* t, int channels) {
     if (!t || (channels != 1 && channels != 3)) { dvfe_set_error("set_input: channels must be 1 (gray) or 3 (BGR)"); return DVFE_ERR_INVALID; }
@@ -732,7 +772,73 @@ extern "C" int dvfe_set_undistort_maps(dvfe_tracker* t, int cam, const int16_t* 
         DVFE_CUDA(cudaMemcpy(t->d_map1[cam], map1, P * 4, cudaMemcpyHostToDevice));
         DVFE_CUDA(cudaMemcpy(t->d_map2[cam], map2, P * 2, cudaMemcpyHostToDevice));
     }
+    for (int s = 0; s < t->B; s++) {                 // every stream follows the shared maps again
+        cudaFree(t->s_map1[cam][s]); cudaFree(t->s_map2[cam][s]);
+        t->s_map1[cam][s] = nullptr; t->s_map2[cam][s] = nullptr;
+        t->own_maps[cam][s] = 0;
+    }
+    DVFE_CHECK(t->update_maps(cam));
     return t->size_stage();
+}
+
+// Per-stream maps live in device memory the call allocates, so no step may be in flight; the call does not wait for one itself,
+// which would take the records of the earlier steps from the caller's later dvfe_wait calls.
+extern "C" int dvfe_set_stream_undistort_maps(dvfe_tracker* t, int stream, int cam, const int16_t* map1, const uint16_t* map2) {
+    if (!t || cam < 0 || cam > 1 || (map1 != nullptr) != (map2 != nullptr)) {
+        dvfe_set_error("set_stream_undistort_maps: bad argument");
+        return DVFE_ERR_INVALID;
+    }
+    if (IS_GROUP(t)) return grp_set_stream_maps(t, stream, cam, map1, map2);
+    if (stream < 0 || stream >= t->B) { dvfe_set_error("set_stream_undistort_maps: bad stream index %d", stream); return DVFE_ERR_INVALID; }
+    if (t->completed < t->frames) {
+        dvfe_set_error("set_stream_undistort_maps: %ld step(s) in flight; wait for them first", t->frames - t->completed);
+        return DVFE_ERR_INVALID;
+    }
+    DVFE_CUDA(cudaSetDevice(t->cfg.device));
+    DVFE_CUDA(cudaStreamSynchronize(t->st));
+    DVFE_CUDA(cudaStreamSynchronize(t->cs));
+    short* m1 = nullptr;
+    unsigned short* m2 = nullptr;
+    if (map1) {
+        const size_t P = (size_t)t->W * t->H;
+        cudaError_t e = cudaMalloc((void**)&m1, P * 4);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&m2, P * 2);
+        if (e == cudaSuccess) e = cudaMemcpy(m1, map1, P * 4, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaMemcpy(m2, map2, P * 2, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            cudaFree(m1); cudaFree(m2);
+            dvfe_set_error("set_stream_undistort_maps: %s", cudaGetErrorString(e));
+            return DVFE_ERR_CUDA;
+        }
+    }
+    cudaFree(t->s_map1[cam][stream]); cudaFree(t->s_map2[cam][stream]);
+    t->s_map1[cam][stream] = m1; t->s_map2[cam][stream] = m2;
+    t->own_maps[cam][stream] = 1;
+    DVFE_CHECK(t->update_maps(cam));
+    return t->size_stage();
+}
+
+static bool camera_ok(const dvfe_camera* c) {
+    const double v[8] = {c->fx, c->fy, c->cx, c->cy, c->k1, c->k2, c->p1, c->p2};
+    for (double x : v)
+        if (!isfinite(x)) return false;
+    return c->fx != 0.0 && c->fy != 0.0;
+}
+
+// The calibration of the next step submitted; steps already submitted keep theirs (submit() uploads the table).  No tracking state
+// is touched.
+extern "C" int dvfe_set_stream_camera(dvfe_tracker* t, int stream, const dvfe_camera* cam0, const dvfe_camera* cam1) {
+    if (!t || !cam0) { dvfe_set_error("set_stream_camera: null argument"); return DVFE_ERR_INVALID; }
+    if (!camera_ok(cam0) || (cam1 && !camera_ok(cam1))) {
+        dvfe_set_error("set_stream_camera: camera parameters must be finite, with fx and fy non-zero");
+        return DVFE_ERR_INVALID;
+    }
+    if (IS_GROUP(t)) return grp_set_stream_camera(t, stream, cam0, cam1);
+    if (stream < 0 || stream >= t->B) { dvfe_set_error("set_stream_camera: bad stream index %d", stream); return DVFE_ERR_INVALID; }
+    t->cams[stream] = make_cam(*cam0);
+    t->cams[(size_t)t->B + stream] = make_cam(cam1 ? *cam1 : *cam0);
+    t->cam_dirty = true;
+    return DVFE_OK;
 }
 
 static int check_step_args(dvfe_tracker* t, const uint8_t* left, int pitch, const double* time0) {

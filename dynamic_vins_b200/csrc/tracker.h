@@ -51,7 +51,13 @@ struct dvfe_tracker {
     cudaStream_t rs = nullptr;                       // right-image pyramid stream: fills the SMs the selection kernel leaves idle
     bool own_stream = true;
     PyrDesc desc{};
-    CamParams cam0{}, cam1{};
+    // Per-stream calibration (dvfe_set_stream_camera): the post kernels read d_cam[cam * B + stream].  The host table is the
+    // calibration of the next step; submit() uploads it on the compute stream, ahead of that step's kernels, when it changed.
+    // The device pointer never changes, so captured graphs stay valid.
+    std::vector<CamParams> cams;                     // [2][B] cam0 of every stream, then cam1
+    CamParams* d_cam = nullptr;                      // [2][B]
+    CamParams* h_cam[2] = {nullptr, nullptr};        // pinned copy source, one per in-flight step
+    bool cam_dirty = false;                          // `cams` differs from what the last uploaded table holds
     // Pyramids: 3 left slots (current / previous / being uploaded) and 2 right slots.  Step k uses
     // left[k % 3] (previous = left[(k + 2) % 3]) and right[k % 2]; "phase" = k % 6 selects the descriptor set.
     uint8_t* pyrL[3] = {nullptr, nullptr, nullptr};
@@ -138,12 +144,27 @@ struct dvfe_tracker {
     // frame ingest (dvfe_set_input / dvfe_set_undistort_maps): BGR and/or remapped input goes through a device staging
     // buffer and the ingest kernel, which writes level 0 in place
     int in_ch = 1;
-    short* d_map1[2] = {nullptr, nullptr};
+    short* d_map1[2] = {nullptr, nullptr};           // the maps of every stream of camera cam (dvfe_set_undistort_maps)
     unsigned short* d_map2[2] = {nullptr, nullptr};
+    // per-stream maps (dvfe_set_stream_undistort_maps): own_maps[cam][s] = the stream's own maps (or none) replace the shared ones
+    std::vector<uint8_t> own_maps[2];
+    std::vector<short*> s_map1[2];                   // [B], null = no maps
+    std::vector<unsigned short*> s_map2[2];
+    IngestMaps* d_imaps[2] = {nullptr, nullptr};     // [B] the maps each image of camera cam is remapped with (ingest kernel)
+    bool maps_uniform[2] = {true, true};             // every stream of camera cam uses the same maps: the shared-map kernel
+    const short* stream_map1(int cam, int s) const { return own_maps[cam][s] ? s_map1[cam][s] : d_map1[cam]; }
+    const unsigned short* stream_map2(int cam, int s) const { return own_maps[cam][s] ? s_map2[cam][s] : d_map2[cam]; }
+    int update_maps(int cam);                        // recompute maps_uniform[cam] and upload d_imaps[cam] (no step in flight)
     // dense staging of host images [2 cameras][B][H*W*in_ch], one per in-flight step: the staged upload's copy source, or the
     // ingest kernel's input; sized by size_stage() whenever the input format changes, never inside a step
     uint8_t* d_stage[2] = {nullptr, nullptr};
-    bool prep_active() const { return in_ch != 1 || d_map1[0] || d_map1[1]; }
+    bool prep_active() const {                       // any stream of either camera has maps, or BGR input
+        if (in_ch != 1) return true;
+        for (int cam = 0; cam < 2; cam++)
+            for (int s = 0; s < B; s++)
+                if (stream_map1(cam, s)) return true;
+        return false;
+    }
     int size_stage();
     uint8_t* level0(int cam) const;                  // the interior of level 0 of this step's left / right slot
     int ingest(const uint8_t* d_src, size_t stream_stride, int pitch, int cam, cudaStream_t s);

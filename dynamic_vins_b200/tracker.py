@@ -17,6 +17,24 @@ import numpy as np
 from . import _lib as L
 
 
+CAMERA_KEYS = ("fx", "fy", "cx", "cy", "k1", "k2", "p1", "p2")
+
+
+def make_camera(cam: dict) -> L.Camera:
+    """a camera dict (fx, fy, cx, cy, k1, k2, p1, p2) -> dvfe_camera"""
+    c = L.Camera()
+    for k in CAMERA_KEYS:
+        setattr(c, k, float(cam[k]))
+    return c
+
+
+def camera_from_yaml(path: str) -> dict:
+    """one camodocal PINHOLE calibration file -> the camera dict make_config and BatchTracker.set_stream_camera take"""
+    c = L.Camera()
+    L.check(L.lib().dvfe_camera_from_yaml(path.encode(), C.byref(c)))
+    return {k: getattr(c, k) for k in CAMERA_KEYS}
+
+
 def make_config(width: int, height: int, max_cnt: int, min_dist: int, cam0: dict, cam1: Optional[dict] = None,
                 stereo: bool = True, n_streams: int = 1, max_dynamic_cnt: int = 50, min_dynamic_dist: int = 5,
                 flow_back: int = 1, use_mask_morphology: int = 0, mask_morphology_size: int = 5,
@@ -30,10 +48,7 @@ def make_config(width: int, height: int, max_cnt: int, min_dist: int, cam0: dict
     c.use_mask_morphology, c.mask_morphology_size = use_mask_morphology, mask_morphology_size
     c.lk_max_level, c.max_instances, c.device = lk_max_level, max_instances, device
     c.n_groups = n_groups
-    cam1 = cam1 if cam1 is not None else cam0
-    for dst, src in ((c.cam0, cam0), (c.cam1, cam1)):
-        for k in ("fx", "fy", "cx", "cy", "k1", "k2", "p1", "p2"):
-            setattr(dst, k, float(src[k]))
+    c.cam0, c.cam1 = make_camera(cam0), make_camera(cam1 if cam1 is not None else cam0)
     return c
 
 
@@ -124,6 +139,22 @@ class BatchTracker:
         if m1 is not None:
             assert m1.shape == (self.H, self.W, 2) and m2.shape == (self.H, self.W)
         L.check(L.lib().dvfe_set_undistort_maps(self._h, cam, L.ptr(m1), L.ptr(m2)))
+
+    def set_stream_undistort_maps(self, stream: int, cam: int, map1: Optional[np.ndarray], map2: Optional[np.ndarray]) -> None:
+        """maps of camera cam for one stream only (None, None: that stream's images of camera cam are not remapped); no step may
+        be in flight (wait() for async steps first).  set_undistort_maps gives every stream the shared maps again."""
+        m1 = None if map1 is None else np.ascontiguousarray(map1, np.int16)
+        m2 = None if map2 is None else np.ascontiguousarray(map2, np.uint16)
+        if m1 is not None:
+            assert m1.shape == (self.H, self.W, 2) and m2.shape == (self.H, self.W)
+        L.check(L.lib().dvfe_set_stream_undistort_maps(self._h, int(stream), int(cam), L.ptr(m1), L.ptr(m2)))
+
+    def set_stream_camera(self, stream: int, cam0: dict, cam1: Optional[dict] = None) -> None:
+        """the calibration (camera dicts as make_config takes them; cam1 None = cam0) of one stream from the next step on; the
+        stream's tracking state is kept (add FRAME_RESET on its next step when the slot now serves another camera)"""
+        c0 = make_camera(cam0)
+        c1 = None if cam1 is None else make_camera(cam1)
+        L.check(L.lib().dvfe_set_stream_camera(self._h, int(stream), C.byref(c0), None if c1 is None else C.byref(c1)))
 
     def _stream_flags(self, stream_flags) -> Optional[np.ndarray]:
         """per-stream L.FRAME_* bytes of dvfe_track_image_ex / _semantic_ex / _dynamic_ex2 (None: no flag array, the plain step)"""

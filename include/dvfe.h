@@ -7,8 +7,10 @@
  * sizes only; no C++/torch types cross this boundary; nothing throws — the
  * reference's exception cases come back as negative codes.
  *
- * One `dvfe_tracker` owns B independent camera streams of identical geometry on
- * one GPU ("stream-sharded replicas", SURVEY.md §8e).  B = 1 is the reference's
+ * One `dvfe_tracker` owns B independent camera streams of identical geometry (image
+ * size and front-end parameters) on one GPU ("stream-sharded replicas", SURVEY.md §8e);
+ * each stream may have its own calibration and undistortion maps
+ * (dvfe_set_stream_camera, dvfe_set_stream_undistort_maps).  B = 1 is the reference's
  * single `FeatureTracker` + `InstsFeatManager` pair.  All device state (pyramids,
  * point sets, ids, velocities) stays resident in HBM between calls.
  */
@@ -115,6 +117,11 @@ void dvfe_destroy(dvfe_tracker* t);
 /* fe_para::SetParameters(config_path) + the cfg keys of utils/parameters.cpp + the two camodocal yaml files
  * named by cam0_calib / cam1_calib (front_end/front_end_parameters.cpp:17-40).  Fills *cfg; n_streams = 1. */
 int dvfe_config_from_yaml(const char* config_path, dvfe_config* cfg);
+
+/* camodocal PinholeCamera::readFromYamlFile of one calibration file (the reader dvfe_config_from_yaml uses for cam0_calib /
+ * cam1_calib), e.g. for dvfe_set_stream_camera.  DVFE_ERR_CONFIG for a bad path or a model_type other than PINHOLE.  Needs no
+ * device. */
+int dvfe_camera_from_yaml(const char* path, dvfe_camera* cam);
 
 const char* dvfe_last_error(const dvfe_tracker* t);   /* t may be NULL: last error of dvfe_create / ops */
 const char* dvfe_version(void);
@@ -398,6 +405,24 @@ int dvfe_track_dynamic_async(dvfe_tracker* t, const uint8_t* left, const uint8_t
  * and stays one byte per pixel: with a 3-channel input its row pitch is pitch / 3 and its stream stride stream_stride / 3. */
 int dvfe_set_input(dvfe_tracker* t, int channels);
 int dvfe_set_undistort_maps(dvfe_tracker* t, int cam, const int16_t* map1, const uint16_t* map2);
+
+/* ---- per-stream calibration ----------------------------------------------------------------------------------
+ * dvfe_set_stream_camera: the cam_t.cam0 / cam_t.cam1 of stream `stream` (cam1 == NULL: cam1 = cam0, as dvfe_config_from_yaml
+ * without cam1_calib); until then every stream uses dvfe_config::cam0 / cam1.  It is the PinholeCamera::liftProjective of the
+ * stream's x, y, vx, vy (background, instances with their ROI offset through cam0, instance right points through cam1).  The call
+ * does not wait: it applies from the next step submitted through any entry point (steps already submitted keep the calibration
+ * they were submitted with; a skipped stream picks it up at its next present frame; the InstsTrack of a frame uses the calibration
+ * of that frame's background step).  No tracking state is reset: the next velocities compare the previous frame's points, lifted
+ * with the old calibration, with the new lift.  A caller that gives a stream slot to another physical camera adds
+ * DVFE_FRAME_RESET on that stream's next step.  The calibration belongs to the slot: DVFE_FRAME_RESET and dvfe_set_state leave
+ * it.  DVFE_ERR_INVALID (nothing changed) for a stream out of range, cam0 == NULL, a non-finite field or fx / fy == 0.
+ * dvfe_set_stream_undistort_maps: the maps of camera `cam` for stream `stream` alone, in the format of dvfe_set_undistort_maps
+ * (6 bytes per pixel of device memory per stream and camera); (NULL, NULL) = that stream's images of camera `cam` are not
+ * remapped, even when the other streams' are.  dvfe_set_undistort_maps gives every stream of `cam` the shared maps again (per-stream
+ * maps of `cam` are dropped).  The call allocates device memory: with a step in flight (not yet waited for) it returns
+ * DVFE_ERR_INVALID and changes nothing.  With stream groups both calls go to the group that holds the stream. */
+int dvfe_set_stream_camera(dvfe_tracker* t, int stream, const dvfe_camera* cam0, const dvfe_camera* cam1);
+int dvfe_set_stream_undistort_maps(dvfe_tracker* t, int stream, int cam, const int16_t* map1, const uint16_t* map2);
 
 /* ---- epipolar outlier rejection and extra points (SURVEY.md §8f N4) --------------------------------------
  * InstsFeatManager::RejectWithF (front_end/dynamic_tracker.cpp:831-849; FeatureTracker::RejectWithF,

@@ -422,6 +422,17 @@ public:
     const dvfe_config& config() const { return cfg_; }
     dvfe_tracker* handle() { return h_; }
 
+    // The calibration of one stream (cam_t.cam0 / cam1 of that stream's rig, e.g. dvfe_camera_from_yaml of its calibration
+    // files; cam1 == nullptr: cam1 = cam0), from the next step on; the stream's tracking state is kept (dvfe_set_stream_camera)
+    void SetStreamCamera(int stream, const dvfe_camera& cam0, const dvfe_camera* cam1 = nullptr) {
+        if (dvfe_set_stream_camera(h_, stream, &cam0, cam1) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+    }
+    // The undistortion maps of camera `cam` for one stream (CV_16SC2 + CV_16UC1; both null: not remapped); no step may be in
+    // flight (dvfe_set_stream_undistort_maps)
+    void SetStreamUndistortMaps(int stream, int cam, const int16_t* map1, const uint16_t* map2) {
+        if (dvfe_set_stream_undistort_maps(h_, stream, cam, map1, map2) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+    }
+
     // TrackImage of all cameras, enqueued; `time0` has one entry per stream; the images stay valid until the matching Wait()
     void TrackImageAsync(const uint8_t* left, const uint8_t* right, size_t stream_stride, int step, const std::vector<double>& time0) {
         check(time0);

@@ -81,6 +81,7 @@ SYMBOLS = [
     "dvfe_op_reject_with_f", "dvfe_op_detect_extra_points", "dvfe_op_build_pyramid_bordered", "dvfe_set_detect_mode", "dvfe_op_good_features_cuda",
     "dvfe_track_image_ex", "dvfe_track_semantic_ex", "dvfe_track_dynamic_ex2",
     "dvfe_set_stream_camera", "dvfe_set_stream_undistort_maps", "dvfe_camera_from_yaml",
+    "dvfe_export_stream", "dvfe_import_stream",
 ]
 
 # dvfe_track_image_ex / _semantic_ex / _dynamic_ex2: per-stream frame flags; dvfe_track_image_ex's step flags (include/dvfe.h)
@@ -153,6 +154,8 @@ def lib() -> C.CDLL:
         L.dvfe_set_stream_camera.argtypes = [C.c_void_p, C.c_int, C.POINTER(Camera), C.POINTER(Camera)]
         L.dvfe_set_stream_undistort_maps.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         L.dvfe_camera_from_yaml.argtypes = [C.c_char_p, C.POINTER(Camera)]
+        L.dvfe_export_stream.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
+        L.dvfe_import_stream.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_size_t]
         L.dvfe_op_merge_masks.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         L.dvfe_set_detect_mode.argtypes = [C.c_void_p, C.c_int]
         L.dvfe_op_build_pyramid_bordered.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]

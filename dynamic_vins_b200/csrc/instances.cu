@@ -221,6 +221,42 @@ void dvfe_tracker::reset_instances(int stream) {
     S.last_time = 0.0;
 }
 
+// The previous ROI crop of an instance is in the buffer its last crop went to (cur_buf); an imported one goes to buffer 0.
+void dvfe_tracker::insts_export(int stream, std::vector<SnapInst>* recs, std::vector<SnapInstDev>* dev, double* last_time) const {
+    const InstStream& S = inst->streams[stream];
+    for (const auto& kv : S.insts) {
+        const InstHost& in = kv.second;
+        recs->push_back(SnapInst{in.track_id, in.lost_num, in.visible ? 1 : 0, in.has_box ? 1 : 0, in.x, in.y, in.w, in.h,
+                                 in.prev_w, in.prev_h});
+        const size_t set = (size_t)stream * inst->MI + in.slot;
+        dev->push_back(SnapInstDev{set, inst->roi_gray + (set * 2 + in.cur_buf) * inst->P});
+    }
+    *last_time = S.last_time;
+}
+
+void dvfe_tracker::insts_import(int stream, const std::vector<SnapInst>& recs, double last_time, std::vector<SnapInstDev>* dev) {
+    reset_instances(stream);
+    InstStream& S = inst->streams[stream];
+    S.last_time = last_time;
+    S.out.clear();
+    for (const SnapInst& r : recs) {
+        InstHost in;
+        in.track_id = r.track_id;
+        in.slot = S.free_slots.back();
+        S.free_slots.pop_back();
+        in.lost_num = r.lost_num; in.visible = r.visible != 0; in.has_box = r.has_box != 0;
+        in.x = r.x; in.y = r.y; in.w = r.w; in.h = r.h;
+        in.prev_w = r.prev_w; in.prev_h = r.prev_h;
+        in.roi_w = r.prev_w; in.roi_h = r.prev_h;
+        in.cur_buf = 0;
+        S.insts.emplace(r.track_id, in);
+        const size_t set = (size_t)stream * inst->MI + in.slot;
+        dev->push_back(SnapInstDev{set, inst->roi_gray + set * 2 * inst->P});
+    }
+}
+
+const PointSetArrays& dvfe_tracker::inst_points() const { return inst->pts; }
+
 // InstsFeatManager::ManageInstances (front_end/dynamic_tracker.cpp:499-514)
 static void manage_instances(InstStream& S) {
     for (auto it = S.insts.begin(); it != S.insts.end();) {

@@ -200,6 +200,7 @@ int dvfe_tracker::init() {
     prev_time.assign(B, 0.0);
     tc_valid.assign(B, 0);
     last_sflags.assign(B, 0);
+    had_frame.assign(B, 0);
     DVFE_CHECK(dmalloc(&d_sflags, (size_t)B));
     DVFE_CHECK(dmalloc(&d_lane, (size_t)B));
     DVFE_CHECK(dmalloc(&d_pgroups[0], (size_t)B));
@@ -338,6 +339,7 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     cudaFree(t->d_sflags); cudaFree(t->d_lane); cudaFree(t->d_pgroups[0]); cudaFree(t->d_pgroups[1]); cudaFree(t->d_pjobs);
     cudaFree(t->d_zero);
     cudaFree(t->d_cam);
+    cudaFree(t->d_snap);
     for (int cam = 0; cam < 2; cam++) {
         cudaFree(t->d_imaps[cam]);
         for (short* m : t->s_map1[cam]) cudaFree(m);
@@ -502,6 +504,8 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
     const int ph = (int)(k % 6), par = (int)(k % 2);
     const bool stereo_now = cfg.stereo && in.has_right;
     const bool partial = sflags != nullptr;
+    // the frame index the compute part runs as: frame 6 has the buffer phase of frame 0 and is not a first frame (prev_loaded)
+    const long kc = (k == 0 && prev_loaded) ? 6 : k;
     if (partial) {
         for (int s = 0; s < B; s++) {
             if (sflags[s] & DVFE_FRAME_RESET) prev_time[s] = 0.0;                  // a new tracker's prev_time
@@ -543,12 +547,12 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
         }
         // level 0 copied by the kernel above arrives with its border; DMA / ingest kernels leave the border to the graph
         const bool l0_complete = !in.in_place && pyr_level0_writes_border(desc);
-        const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (k > 0 ? 8u : 0u) | (tcache_valid && !partial ? 16u : 0u) |
+        const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (kc > 0 ? 8u : 0u) | (tcache_valid && !partial ? 16u : 0u) |
                                (l0_complete ? 32u : 0u) | (partial ? 64u : 0u);
         const StepKey key(ph, flags);
         if (step_graphs.find(key) == step_graphs.end()) {
             if (step_graphs.size() >= 64) drop_graphs();          // a caller cycling through many modes
-            DVFE_CHECK(capture_step(ph, flags, k));
+            DVFE_CHECK(capture_step(ph, flags, kc));
             // The first step of a mode also captures the six steady-state graphs it will replay from the next frame on (one per
             // buffer phase), so that instantiation (host time, ~0.3 ms each) never falls into a later, possibly timed, step.
             const bool tc_next = stereo_now && d_tcache != nullptr;
@@ -562,7 +566,7 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
         g_dvfe_launches += it->second.n_kernels;
     } else {
         DVFE_CHECK(enqueue_compute(in.left, in.right, in.stride, in.pitch, semantic, in.in_place ? DVFE_L0_INTERIOR : DVFE_L0_BUILD,
-                                   stereo_now, k, prof, partial));
+                                   stereo_now, kc, prof, partial));
     }
     // Template-cache validity per stream: a present frame with a stereo step leaves the templates of its points, a frame without
     // one leaves none (a RESET frame's points are all new), a skipped stream keeps what it had.  A full step reads the cache of
@@ -587,7 +591,7 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
     if (prof) cudaEventRecord(ev[par][ST_D2H + 1], ds);
     DVFE_CUDA(cudaEventRecord(ev_done[par], ds));
     for (int s = 0; s < B; s++)
-        if (!partial || !(sflags[s] & DVFE_FRAME_SKIP)) prev_time[s] = time0[s];
+        if (!partial || !(sflags[s] & DVFE_FRAME_SKIP)) { prev_time[s] = time0[s]; had_frame[s] = 1; }
     last_has_right = stereo_now;
     if (partial) last_sflags.assign(sflags, sflags + B);
     else last_sflags.assign(B, 0);

@@ -28,6 +28,20 @@ int check_stream_flags(const uint8_t* stream_flags, int B, const char* who, cons
 
 struct InstanceState;   // instances.cu
 
+// One instance of a stream snapshot (snapshot.cu, dvfe_export_stream): the host bookkeeping of InstsFeatManager::instances that the
+// next frame reads.  Stored in the blob as is.
+struct SnapInst {
+    uint32_t track_id;
+    int32_t lost_num, visible, has_box;
+    int32_t x, y, w, h;                              // the box of the last frame the instance was seen in
+    int32_t prev_w, prev_h;                          // size of the previous ROI crop (0: none)
+};
+// Where that instance's device state lives: its point set in InstanceState::pts and its previous ROI crop (dense prev_w x prev_h)
+struct SnapInstDev {
+    size_t set;
+    uint8_t* crop;
+};
+
 // Where a frame step finds its images once dvfe_tracker::place_input has put them in place
 struct StepInput {
     const uint8_t* left = nullptr;                   // device images the step copies into level 0 (null when in_place)
@@ -67,6 +81,11 @@ struct dvfe_tracker {
     bool last_has_right = false;                     // the last submitted frame had a right image
     std::vector<uint8_t> last_sflags;                // [B] DVFE_FRAME_* of the last submitted step (all 0 for a full step): the
                                                      // InstsTrack of the same frame follows them
+    std::vector<uint8_t> had_frame;                  // [B] the stream has had a frame: the previous left slot holds its last image
+    // dvfe_import_stream put a previous left image into a tracker that has run no step: its first step is then run in the
+    // "not the first frame" form (temporal LK + compaction), which is exact for every stream that never had a frame (n = 0)
+    bool prev_loaded = false;
+    uint8_t* d_snap = nullptr;                       // stream snapshot staging (snapshot.cu), allocated on first use at its largest
     PointSetArrays bg{};                             // background point sets, one per stream
     uint32_t* d_next_id = nullptr;                   // [B] InstFeat::global_id_count per stream
     double* d_dt = nullptr;
@@ -182,6 +201,11 @@ struct dvfe_tracker {
     int semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
                         int pitch, const int* exist_inst, const double* time0, unsigned flags = 0, const uint8_t* sflags = nullptr);
     void reset_instances(int stream);                // instances.cu: a newly created InstsFeatManager for one stream
+    // instances.cu, for stream snapshots: the instance table of `stream` in ascending track id with where each instance's device state
+    // lives, and its last_time; insts_import replaces the table (slots from the free list) and says where the device state goes
+    void insts_export(int stream, std::vector<SnapInst>* recs, std::vector<SnapInstDev>* dev, double* last_time) const;
+    void insts_import(int stream, const std::vector<SnapInst>& recs, double last_time, std::vector<SnapInstDev>* dev);
+    const PointSetArrays& inst_points() const;
     uint8_t* d_labels[2] = {nullptr, nullptr};       // uploaded label images, one per in-flight step (allocated on first use)
     const uint8_t* lab_ptr[2] = {nullptr, nullptr};  // the label images of the in-flight steps (device), for the ROI masks
     size_t lab_stride[2] = {0, 0};

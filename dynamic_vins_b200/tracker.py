@@ -418,6 +418,21 @@ class BatchTracker:
         L.check(L.lib().dvfe_set_state(self._h, stream, C.byref(st)))
 
 
+    # ---- stream snapshots ----------------------------------------------------------------------
+    def export_stream(self, stream: int) -> bytes:
+        """everything the next step of `stream` reads from earlier frames, as one blob (include/dvfe.h dvfe_export_stream); no step
+        may be in flight (wait() for async steps first)"""
+        n = C.c_size_t(0)
+        L.check(L.lib().dvfe_export_stream(self._h, int(stream), None, 0, C.byref(n)))
+        buf = C.create_string_buffer(n.value)
+        L.check(L.lib().dvfe_export_stream(self._h, int(stream), buf, n.value, C.byref(n)))
+        return buf.raw[:n.value]
+
+    def import_stream(self, stream: int, blob: bytes) -> None:
+        """replace the whole state of slot `stream` with an exported stream's (dvfe_import_stream): the slot then continues as the
+        source stream would have; undistortion maps and the LK / detector modes are not part of the blob"""
+        L.check(L.lib().dvfe_import_stream(self._h, int(stream), bytes(blob), len(blob)))
+
 class FeatureTracker:
     """Single-stream tracker with the reference's method names (front_end/background_tracker.h:44-49).
     `img` is any object with the SemanticImage fields the path reads: gray0, gray1 (or None), time0 and, for

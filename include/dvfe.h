@@ -316,6 +316,30 @@ typedef struct dvfe_state {
 int dvfe_get_state(dvfe_tracker* t, int stream, dvfe_state* st, int cap);
 int dvfe_set_state(dvfe_tracker* t, int stream, const dvfe_state* st);
 
+/* ---- stream snapshots: move one camera stream to another slot, tracker or GPU, or checkpoint it -------------------
+ * dvfe_export_stream writes everything the next step of `stream` reads from earlier frames into `blob` (host memory, `cap` bytes):
+ * the background point set (n, next_id — the id counter the stream's instances share —, prev_time, ids, track_cnt, last points,
+ * prev_un, right_prev_un, right_prev_valid), whether the stream has had a frame and then its last left image, the stream's cam0 / cam1
+ * as the tracker lifts with them, and with max_instances > 0 the instance table (last_time; per instance in ascending track id:
+ * lost_num, visibility, box, previous ROI crop and point set).  *n_bytes = the blob's size; blob == NULL only asks for it.  cap too
+ * small: DVFE_ERR_CAPACITY, *n_bytes set, nothing written.  A pure read: every stream continues bit for bit, with no added launches.
+ * dvfe_import_stream replaces the whole state of slot `stream` with the blob's: every later step gives that slot the records the
+ * source stream would have had, bit for bit, through any entry point.  The destination may have another n_streams, n_groups, device,
+ * slot index, frame count (also none: the usual target of a migration) and buffer phase.  Its calibration is applied as
+ * dvfe_set_stream_camera does; the template caches of the slot are dropped.
+ * Not carried: undistortion maps (6 bytes per pixel and camera: the caller sets them on the destination slot with
+ * dvfe_set_stream_undistort_maps) and the tracker-wide modes of dvfe_set_lk_mode* / dvfe_set_detect_mode (the continuation is exact
+ * under the same modes).  Dynamic mode: take a snapshot between frames, after the frame's InstsTrack if the frame has one (the
+ * library cannot tell whether a caller still means to call dvfe_insts_track for the last background step).
+ * The blob is host-endian and read only by a library of the same snapshot format version (layout: DESIGN.md §2).  Both calls return
+ * DVFE_ERR_INVALID and change nothing with a step of the stream's group in flight (not yet waited for), a bad stream index or a NULL
+ * pointer; import also for a bad magic number, format version or CRC-32, a truncated blob, a front-end field (width, height, stereo,
+ * max_cnt, min_dist, max_dynamic_cnt, min_dynamic_dist, flow_back, use_mask_morphology, mask_morphology_size, lk_max_level) that
+ * differs from the destination's, or more instances than its max_instances.  With stream groups both go to the group that holds
+ * the stream.  dvfe_get_state / dvfe_set_state stay the teacher-forced exchange of the background point arrays. */
+int dvfe_export_stream(dvfe_tracker* t, int stream, void* blob, size_t cap, size_t* n_bytes);
+int dvfe_import_stream(dvfe_tracker* t, int stream, const void* blob, size_t n_bytes);
+
 /* ---- seam-level operators (unit parity; each replaces one OpenCV/camodocal call of the path) ---- */
 
 /* cv::buildOpticalFlowPyramid(img, pyr, Size(21,21), max_level) as used inside calcOpticalFlowPyrLK.

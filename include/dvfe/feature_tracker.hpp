@@ -433,6 +433,19 @@ public:
         if (dvfe_set_stream_undistort_maps(h_, stream, cam, map1, map2) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
     }
 
+    // Everything the next step of one stream reads from earlier frames, as one blob (dvfe_export_stream); no step may be in flight
+    std::vector<uint8_t> ExportStream(int stream) {
+        size_t n = 0;
+        if (dvfe_export_stream(h_, stream, nullptr, 0, &n) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+        std::vector<uint8_t> blob(n);
+        if (dvfe_export_stream(h_, stream, blob.data(), blob.size(), &n) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+        return blob;
+    }
+    // The whole state of slot `stream` from an exported blob (dvfe_import_stream): the slot continues as the source stream would have
+    void ImportStream(int stream, const std::vector<uint8_t>& blob) {
+        if (dvfe_import_stream(h_, stream, blob.data(), blob.size()) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+    }
+
     // TrackImage of all cameras, enqueued; `time0` has one entry per stream; the images stay valid until the matching Wait()
     void TrackImageAsync(const uint8_t* left, const uint8_t* right, size_t stream_stride, int step, const std::vector<double>& time0) {
         check(time0);

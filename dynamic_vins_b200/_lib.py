@@ -64,6 +64,12 @@ class InstInfo(C.Structure):
                 ("x", C.c_int32), ("y", C.c_int32), ("w", C.c_int32), ("h", C.c_int32)]
 
 
+class FrameDesc(C.Structure):
+    """dvfe_frame: one camera's images of a step (dvfe_track_frames)"""
+    _fields_ = [("left", C.c_void_p), ("right", C.c_void_p), ("mask", C.c_void_p), ("pitch", C.c_int32), ("mask_pitch", C.c_int32),
+                ("exist_inst", C.c_int32), ("flags", C.c_uint32), ("time0", C.c_double)]
+
+
 class State(C.Structure):
     _fields_ = [("n", C.c_int), ("next_id", C.c_uint32), ("prev_time", C.c_double),
                 ("ids", C.c_void_p), ("track_cnt", C.c_void_p), ("last_points", C.c_void_p),
@@ -82,6 +88,7 @@ SYMBOLS = [
     "dvfe_track_image_ex", "dvfe_track_semantic_ex", "dvfe_track_dynamic_ex2",
     "dvfe_set_stream_camera", "dvfe_set_stream_undistort_maps", "dvfe_camera_from_yaml",
     "dvfe_export_stream", "dvfe_import_stream",
+    "dvfe_track_frames", "dvfe_track_semantic_frames", "dvfe_track_dynamic_frames",
 ]
 
 # dvfe_track_image_ex / _semantic_ex / _dynamic_ex2: per-stream frame flags; dvfe_track_image_ex's step flags (include/dvfe.h)
@@ -156,6 +163,9 @@ def lib() -> C.CDLL:
         L.dvfe_camera_from_yaml.argtypes = [C.c_char_p, C.POINTER(Camera)]
         L.dvfe_export_stream.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.POINTER(C.c_size_t)]
         L.dvfe_import_stream.argtypes = [C.c_void_p, C.c_int, C.c_char_p, C.c_size_t]
+        L.dvfe_track_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_uint]
+        L.dvfe_track_semantic_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_uint]
+        L.dvfe_track_dynamic_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
         L.dvfe_op_merge_masks.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         L.dvfe_set_detect_mode.argtypes = [C.c_void_p, C.c_int]
         L.dvfe_op_build_pyramid_bordered.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]

@@ -667,14 +667,25 @@ extern "C" int dvfe_track_dynamic_ex2(dvfe_tracker* t, const uint8_t* left, cons
     }
     if (!t->inst) { dvfe_set_error("track_dynamic_async: max_instances must be > 0 at create"); return DVFE_ERR_INVALID; }
     if (pitch < t->W * t->in_ch) { dvfe_set_error("track_dynamic_async: bad pitch"); return DVFE_ERR_INVALID; }
-    DVFE_CUDA(cudaSetDevice(t->cfg.device));
     DVFE_CHECK(insts_validate(t, 0, t->B, of.data(), n_boxes, labels, sf));
+    return leaf_track_dynamic(t, t->slab(left, right, mask, stream_stride, pitch), exist_inst, of.data(), n_boxes, time0, sf, flags);
+}
+
+int leaf_validate_boxes(dvfe_tracker* t, const dvfe_inst_in* const* boxes_of, const int* n_boxes, bool labels, const uint8_t* sflags) {
+    if (!t->inst) { dvfe_set_error("track_dynamic: max_instances must be > 0 at create"); return DVFE_ERR_INVALID; }
+    return insts_validate(t, 0, t->B, boxes_of, n_boxes, labels, sflags);
+}
+
+int leaf_track_dynamic(dvfe_tracker* t, const StepSources& src, const int* exist_inst, const dvfe_inst_in* const* boxes_of,
+                       const int* n_boxes, const double* time0, const uint8_t* sf, unsigned flags) {
+    const bool labels = (flags & DVFE_DYN_LABELS) != 0;
+    DVFE_CUDA(cudaSetDevice(t->cfg.device));
     // SetMaskAndRoi: exist_inst = !boxes2d.empty(); a skipped stream's exist_inst is not read
     std::vector<int> exist(t->B);
     for (int s = 0; s < t->B; s++)
         exist[s] = (sf && (sf[s] & DVFE_FRAME_SKIP)) ? 0 : labels ? (n_boxes[s] > 0 ? 1 : 0) : exist_inst[s];
-    DVFE_CHECK(t->semantic_submit(left, right, mask, stream_stride, pitch, exist.data(), time0, flags, sf));
-    return insts_track_streams(t, 0, t->B, of.data(), n_boxes, time0, true, labels);
+    DVFE_CHECK(t->semantic_submit(src, exist.data(), time0, flags, sf));
+    return insts_track_streams(t, 0, t->B, boxes_of, n_boxes, time0, true, labels);
 }
 
 extern "C" int dvfe_insts_output(dvfe_tracker* t, int stream, dvfe_inst_obs* out, int cap, int* n_out) {

@@ -41,6 +41,14 @@ int launch_build_pyramids(const PyrImgSet& set, int n_img, const PyrDesc& desc, 
                           int level0_mode = DVFE_L0_BUILD);
 int launch_pyr_level0(const PyrImgSet& set, int n_img, const PyrDesc& desc, int spitch, cudaStream_t st);
 bool pyr_level0_writes_border(const PyrDesc& desc);
+// One image of a step's input, per stream (dvfe_track_frames): ptr == null = no image, nothing is read or written for it
+struct ImgSrc {
+    const uint8_t* ptr;
+    int pitch;
+};
+// The gather form of launch_pyr_level0: image i is read at d_src[i] and written, border included when
+// pyr_level0_writes_border, into level 0 of the pyramid at dst + i * dst_stride; absent images are not written
+int launch_pyr_level0_table(const ImgSrc* d_src, uint8_t* dst, size_t dst_stride, int n_img, const PyrDesc& desc, cudaStream_t st);
 // Frame ingest (prep.cu): optional fixed-point cv::remap (undistortion maps) + optional BGR -> gray, B images per launch,
 // written at dst_pitch (straight into level 0 of a padded pyramid, or dense).
 struct IngestArgs {
@@ -63,6 +71,12 @@ struct IngestMaps {
 };
 // d_maps (nullable): [n_img] per-image maps in place of a.map1 / a.map2 (gray output only)
 int launch_ingest(const IngestArgs& a, cudaStream_t st, const IngestMaps* d_maps = nullptr);
+// The table form (gray output only): image i is read at d_src[i] (a.src / a.src_stride / a.src_pitch unused) and written at
+// a.dst + i * a.dst_stride, remapped with d_maps[i] (nullable: a.map1 / a.map2 for every image); absent images are not written
+int launch_ingest_table(const IngestArgs& a, const ImgSrc* d_src, cudaStream_t st, const IngestMaps* d_maps = nullptr);
+// Dense copy of n_img images of `row` bytes x h rows: image i from d_src[i] to dst + i * dst_stride at dst_pitch; absent ones skipped
+int launch_gather_images(const ImgSrc* d_src, uint8_t* dst, size_t dst_stride, int dst_pitch, int row, int h, int n_img,
+                         cudaStream_t st);
 
 int launch_build_pyramids_jobs(const PyrJob* d_jobs, int n_jobs, int max_w, int max_h, int max_levels, cudaStream_t st);
 int launch_crop_jobs(const CropJob* d_jobs, int n_jobs, int max_w, int max_h, cudaStream_t st);

@@ -314,6 +314,59 @@ __global__ void __launch_bounds__(256) k_ingest_remap_each(IngestArgs a, const I
     remap_images<CH, false>(a, m.map1, m.map2, xb, y, s, s + 1);
 }
 
+// Table form of the ingest (every stream's image in its own buffer, dvfe_track_frames): image blockIdx.z is read through its table
+// entry, at its own pitch, and gets the bytes k_ingest_remap_each writes (k_ingest_remap / k_ingest_rows with shared maps)
+template <int CH>
+__global__ void __launch_bounds__(256) k_ingest_table(IngestArgs a, const ImgSrc* __restrict__ srcs, const IngestMaps* __restrict__ maps) {
+    const int s = blockIdx.z;
+    const ImgSrc src = srcs[s];
+    if (src.ptr == nullptr) return;
+    a.src = src.ptr; a.src_pitch = src.pitch;
+    a.dst += (size_t)s * a.dst_stride;
+    const IngestMaps m = maps ? maps[s] : IngestMaps{a.map1, a.map2};
+    const int y = blockIdx.y * 8 + threadIdx.y;
+    if (m.map1 == nullptr) {
+        const int x0 = (blockIdx.x * 32 + threadIdx.x) * 4;
+        if (x0 >= a.w || y >= a.h) return;
+        ingest_rows_px<CH, false>(a, 0, x0, y, min(4, a.w - x0));
+        return;
+    }
+    const int xb = blockIdx.x * 128 + threadIdx.x;
+    if (xb >= a.w || y >= a.h) return;
+    remap_images<CH, false>(a, m.map1, m.map2, xb, y, 0, 1);
+}
+
+int launch_ingest_table(const IngestArgs& a, const ImgSrc* d_src, cudaStream_t st, const IngestMaps* d_maps) {
+    if (a.n_img <= 0) return DVFE_OK;
+    if (a.keep_channels) { dvfe_set_error("ingest: the table form writes gray images only"); return DVFE_ERR_INVALID; }
+    const dim3 blk(32, 8), grid((a.w + 127) / 128, (a.h + 7) / 8, a.n_img);
+    if (a.ch == 3) DVFE_LAUNCH((k_ingest_table<3>), grid, blk, 0, st, a, d_src, d_maps);
+    else DVFE_LAUNCH((k_ingest_table<1>), grid, blk, 0, st, a, d_src, d_maps);
+    return DVFE_OK;
+}
+
+// image blockIdx.z of the table, 4 bytes per thread (word copies where both sides are aligned)
+__global__ void __launch_bounds__(256) k_gather_images(const ImgSrc* __restrict__ srcs, uint8_t* __restrict__ dst, size_t dst_stride,
+                                                       int dst_pitch, int row, int h) {
+    const ImgSrc src = srcs[blockIdx.z];
+    if (src.ptr == nullptr) return;
+    const int x0 = (blockIdx.x * 32 + threadIdx.x) * 4, y = blockIdx.y * 8 + threadIdx.y;
+    if (x0 >= row || y >= h) return;
+    const uint8_t* s = src.ptr + (size_t)y * src.pitch + x0;
+    uint8_t* d = dst + (size_t)blockIdx.z * dst_stride + (size_t)y * dst_pitch + x0;
+    const int n = min(4, row - x0);
+    if (n == 4 && (((uintptr_t)s | (uintptr_t)d) & 3) == 0) *reinterpret_cast<unsigned*>(d) = __ldg(reinterpret_cast<const unsigned*>(s));
+    else for (int i = 0; i < n; i++) d[i] = __ldg(s + i);
+}
+
+int launch_gather_images(const ImgSrc* d_src, uint8_t* dst, size_t dst_stride, int dst_pitch, int row, int h, int n_img,
+                         cudaStream_t st) {
+    if (n_img <= 0) return DVFE_OK;
+    const dim3 blk(32, 8), grid(((row + 3) / 4 + 31) / 32, (h + 7) / 8, n_img);
+    DVFE_LAUNCH(k_gather_images, grid, blk, 0, st, d_src, dst, dst_stride, dst_pitch, row, h);
+    return DVFE_OK;
+}
+
 int launch_ingest(const IngestArgs& a, cudaStream_t st, const IngestMaps* d_maps) {
     if (a.n_img <= 0) return DVFE_OK;
     const int nz = (a.n_img + INGEST_SPT - 1) / INGEST_SPT;

@@ -78,6 +78,64 @@ __global__ void __launch_bounds__(256) k_pyr_level0(PyrImgSet set, PyrLevel L, i
     }
 }
 
+// The body of k_pyr_level0 for one image (dst = pixel (0,0) of the level), for the table form below.  k_pyr_level0 keeps its own
+// copy of these lines: written as a call of this function it compiles to another register count.
+__device__ __forceinline__ void pyr_level0_body(const uint8_t* src, uint8_t* dst, const PyrLevel& L, int spitch, int fuse_border) {
+    const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16;
+    const int y = blockIdx.y * blockDim.y + threadIdx.y;
+    if (x0 >= L.w || y >= L.h) return;
+    const uint8_t* row = src + (size_t)y * spitch + x0;
+    uint8_t* out = dst + (size_t)y * L.pitch + x0;
+    uint4 q;
+    if (x0 + 15 < L.w && (((uintptr_t)row) & 15) == 0) {
+        q = __ldg(reinterpret_cast<const uint4*>(row));
+    } else if (x0 + 15 < L.w && (((uintptr_t)row) & 3) == 0) {
+        const unsigned* p = reinterpret_cast<const unsigned*>(row);
+        q = make_uint4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
+    } else if (x0 + 15 < L.w) {
+        unsigned w4[4];
+#pragma unroll
+        for (int i = 0; i < 4; i++)
+            w4[i] = (unsigned)__ldg(row + 4 * i) | ((unsigned)__ldg(row + 4 * i + 1) << 8) | ((unsigned)__ldg(row + 4 * i + 2) << 16) |
+                    ((unsigned)__ldg(row + 4 * i + 3) << 24);
+        q = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+    } else {
+        for (int i = 0; i < 16 && x0 + i < L.w; i++) out[i] = __ldg(row + i);      // ragged last column (never with fuse_border)
+        return;
+    }
+    *reinterpret_cast<uint4*>(out) = q;
+    if (!fuse_border) return;
+    const unsigned am = __activemask();
+    const unsigned nxt = __shfl_down_sync(am, q.x, 1), prv = __shfl_up_sync(am, q.w, 1);
+    const int padR = L.pitch - DVFE_PADX - L.w, q16 = L.w - 16 - x0;
+    const bool left = x0 < DVFE_PADX, right = q16 < padR;
+    int ys[3], ny = 1;
+    ys[0] = y;
+    if (y >= 1 && y <= DVFE_PADY) ys[ny++] = -y;
+    if (y <= L.h - 2 && y >= L.h - 1 - DVFE_PADY) ys[ny++] = 2 * (L.h - 1) - y;
+    if (!left && !right && ny == 1) return;
+    // pixels x0+1 .. x0+16 reversed -> x' = -x0-16 .. -x0-1 ; pixels x0-1 .. x0+14 reversed -> x' = w+q16 .. w+q16+15
+    const uint4 lb = make_uint4(__byte_perm(q.w, nxt, 0x1234), __byte_perm(q.z, q.w, 0x1234), __byte_perm(q.y, q.z, 0x1234),
+                                __byte_perm(q.x, q.y, 0x1234));
+    const uint4 rb = make_uint4(__byte_perm(q.w, q.z, 0x7012), __byte_perm(q.z, q.y, 0x7012), __byte_perm(q.y, q.x, 0x7012),
+                                __byte_perm(q.x, prv, 0x7012));
+    for (int j = 0; j < ny; j++) {
+        uint8_t* __restrict__ orow = dst + (ptrdiff_t)ys[j] * L.pitch;
+        if (j > 0) *reinterpret_cast<uint4*>(orow + x0) = q;
+        if (left) *reinterpret_cast<uint4*>(orow - x0 - 16) = lb;
+        if (right) *reinterpret_cast<uint4*>(orow + L.w + q16) = rb;
+    }
+}
+
+// one image per grid z, read through the stream's table entry; the whole block leaves when the image is absent
+__global__ void __launch_bounds__(256) k_pyr_level0_table(const ImgSrc* __restrict__ srcs, uint8_t* dst, size_t dst_stride,
+                                                          PyrLevel L, int fuse_border) {
+    const ImgSrc src = srcs[blockIdx.z];
+    if (src.ptr == nullptr) return;
+    pyr_level0_body(src.ptr, dst + (size_t)blockIdx.z * dst_stride + L.offset + (size_t)DVFE_PADY * L.pitch + DVFE_PADX, L,
+                    src.pitch, fuse_border);
+}
+
 // ---- REFLECT_101 border of a level, copied from its own interior; one warp per padded row ------------------
 // Word path (w a multiple of 4, single reflections): an interior word of a band row is an aligned copy; a left border word is
 // the byte permutation (W[j+1].b0, W[j].b3, W[j].b2, W[j].b1) of two adjacent interior words of the source row, a right border
@@ -396,6 +454,14 @@ int launch_pyr_level0(const PyrImgSet& set, int n_img, const PyrDesc& desc, int 
     const PyrLevel& L = desc.lv[0];
     dim3 grid(((L.w + 15) / 16 + 31) / 32, (L.h + 7) / 8, n_img);
     DVFE_LAUNCH(k_pyr_level0, grid, blk, 0, st, set, L, spitch, pyr_level0_writes_border(desc) ? 1 : 0);
+    DVFE_CUDA(cudaGetLastError());
+    return DVFE_OK;
+}
+
+int launch_pyr_level0_table(const ImgSrc* d_src, uint8_t* dst, size_t dst_stride, int n_img, const PyrDesc& desc, cudaStream_t st) {
+    const PyrLevel& L = desc.lv[0];
+    dim3 grid(((L.w + 15) / 16 + 31) / 32, (L.h + 7) / 8, n_img);
+    DVFE_LAUNCH(k_pyr_level0_table, grid, dim3(32, 8), 0, st, d_src, dst, dst_stride, L, pyr_level0_writes_border(desc) ? 1 : 0);
     DVFE_CUDA(cudaGetLastError());
     return DVFE_OK;
 }

@@ -220,6 +220,8 @@ int dvfe_tracker::init() {
         DVFE_CUDA(cudaMallocHost((void**)&h_sflags[p], (size_t)B));
         memset(h_sflags[p], 0, (size_t)B);
     }
+    DVFE_CHECK(dmalloc(&d_src, (size_t)3 * B));
+    for (int p = 0; p < 2; p++) DVFE_CUDA(cudaMallocHost((void**)&h_src[p], (size_t)3 * B * sizeof(ImgSrc)));
     for (int p = 0; p < 2; p++) {
         DVFE_CHECK(dmalloc(&d_obs[p], (size_t)B * 2 * cap));
         DVFE_CHECK(dmalloc(&d_nobs[p], (size_t)B));
@@ -338,6 +340,7 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     cudaFree(t->d_old_idx);
     cudaFree(t->d_sflags); cudaFree(t->d_lane); cudaFree(t->d_pgroups[0]); cudaFree(t->d_pgroups[1]); cudaFree(t->d_pjobs);
     cudaFree(t->d_zero);
+    cudaFree(t->d_src);
     cudaFree(t->d_cam);
     cudaFree(t->d_snap);
     for (int cam = 0; cam < 2; cam++) {
@@ -347,6 +350,7 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     }
     for (int p = 0; p < 2; p++) {
         cudaFreeHost(t->h_sflags[p]);
+        cudaFreeHost(t->h_src[p]);
         cudaFreeHost(t->h_cam[p]);
         cudaFree(t->d_obs[p]); cudaFree(t->d_nobs[p]);
         if (t->ev_packed[p]) cudaEventDestroy(t->ev_packed[p]);
@@ -545,8 +549,9 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
                 DVFE_CUDA(cudaStreamWaitEvent(st, ev_r0[par], 0));
             }
         }
-        // level 0 copied by the kernel above arrives with its border; DMA / ingest kernels leave the border to the graph
-        const bool l0_complete = !in.in_place && pyr_level0_writes_border(desc);
+        // level 0 copied by the kernel above (or by the gather form of it in place_table) arrives with its border; DMA / ingest
+        // kernels leave the border to the graph
+        const bool l0_complete = (!in.in_place && pyr_level0_writes_border(desc)) || in.l0_border;
         const unsigned flags = (semantic ? 1u : 0u) | (stereo_now ? 4u : 0u) | (kc > 0 ? 8u : 0u) | (tcache_valid && !partial ? 16u : 0u) |
                                (l0_complete ? 32u : 0u) | (partial ? 64u : 0u);
         const StepKey key(ph, flags);
@@ -565,7 +570,8 @@ int dvfe_tracker::submit(const StepInput& in, const double* time0, bool semantic
         DVFE_CUDA(cudaGraphLaunch(it->second.exec, st));
         g_dvfe_launches += it->second.n_kernels;
     } else {
-        DVFE_CHECK(enqueue_compute(in.left, in.right, in.stride, in.pitch, semantic, in.in_place ? DVFE_L0_INTERIOR : DVFE_L0_BUILD,
+        DVFE_CHECK(enqueue_compute(in.left, in.right, in.stride, in.pitch, semantic,
+                                   in.in_place ? (in.l0_border ? DVFE_L0_COMPLETE : DVFE_L0_INTERIOR) : DVFE_L0_BUILD,
                                    stereo_now, kc, prof, partial));
     }
     // Template-cache validity per stream: a present frame with a stereo step leaves the templates of its points, a frame without
@@ -690,6 +696,37 @@ int dvfe_tracker::h2d(uint8_t* dst, size_t dst_pitch, size_t dst_stride, const u
     return DVFE_OK;
 }
 
+StepSources slab_sources(int B, const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stride, int pitch,
+                         size_t mask_stride, int mask_pitch) {
+    StepSources src;
+    const uint8_t* base[3] = {left, right, mask};
+    const size_t st[3] = {stride, stride, mask_stride};
+    const int pt[3] = {pitch, pitch, mask_pitch};
+    for (int c = 0; c < 3; c++) {
+        src.img[c].assign(B, ImgSrc{nullptr, pt[c]});
+        if (!base[c]) continue;
+        for (int s = 0; s < B; s++) src.img[c][s].ptr = base[c] + s * st[c];
+        src.uniform[c] = true;
+        src.stride[c] = st[c];
+    }
+    return src;
+}
+
+StepSources dvfe_tracker::slab(const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stride, int pitch) const {
+    const int div = prep_active() ? in_ch : 1;
+    return slab_sources(B, left, right, mask, stride, pitch, stride / (size_t)div, pitch / div);
+}
+
+int dvfe_tracker::upload_sources(const StepSources& src) {
+    if (src_step == frames) return DVFE_OK;
+    // h_src[par] was last the source of step k-2's copy, which has completed (wait_slot)
+    ImgSrc* h = h_src[frames % 2];
+    for (int c = 0; c < 3; c++) memcpy(h + (size_t)c * B, src.img[c].data(), B * sizeof(ImgSrc));
+    DVFE_CUDA(cudaMemcpyAsync(d_src, h, (size_t)3 * B * sizeof(ImgSrc), cudaMemcpyHostToDevice, st));
+    src_step = frames;
+    return DVFE_OK;
+}
+
 // The route depends on where the images are, whether they need the ingest kernel (BGR or undistortion maps) and the width:
 //   device, gray            the step copies the caller's images into level 0 itself;
 //   device, ingest          the ingest kernel writes level 0 on the compute stream;
@@ -697,11 +734,19 @@ int dvfe_tracker::h2d(uint8_t* dst, size_t dst_pitch, size_t dst_stride, const u
 //   host, gray, staged      dense staging, which the step copies into level 0 (pitched DMA of rows that are not a multiple
 //                           of 64 bytes is slow);
 //   host, gray, in place    pitched DMA straight into level 0.
+// A table that is not uniform (place_table) takes the same routes image by image.
 // Host routes end with ev_up[par] on the upload stream, which the compute stream waits for.  The slots written here were
 // last read by step k-2, which wait_slot() has completed.
-int dvfe_tracker::place_input(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch, bool device,
-                              StepInput* in) {
+int dvfe_tracker::place_input(const StepSources& src, bool device, StepInput* in) {
     DVFE_CHECK(wait_slot());
+    const bool has_right = src.any(1);
+    if (!src.uniform[0] || (has_right && (!src.uniform[1] || src.stride[1] != src.stride[0] ||
+                                          src.img[1][0].pitch != src.img[0][0].pitch)))
+        return place_table(src, device, in);
+    const uint8_t* left = src.img[0][0].ptr;
+    const uint8_t* right = has_right ? src.img[1][0].ptr : nullptr;
+    const size_t stream_stride = src.stride[0];
+    const int pitch = src.img[0][0].pitch;
     const bool prep = prep_active();
     *in = StepInput();
     in->has_right = right != nullptr;
@@ -709,29 +754,83 @@ int dvfe_tracker::place_input(const uint8_t* left, const uint8_t* right, size_t 
         in->left = left; in->right = right; in->stride = stream_stride; in->pitch = pitch;
         return DVFE_OK;
     }
-    const uint8_t* src[2] = {left, right};
+    const uint8_t* srcs[2] = {left, right};
     in->in_place = true;
     if (device) {
         for (int cam = 0; cam < 2; cam++)
-            if (src[cam]) DVFE_CHECK(ingest(src[cam], stream_stride, pitch, cam, st));
+            if (srcs[cam]) DVFE_CHECK(ingest(srcs[cam], stream_stride, pitch, cam, st));
         return DVFE_OK;
     }
     const int par = (int)(frames % 2);
     const size_t row = (size_t)W * in_ch, img = row * H;
     for (int cam = 0; cam < 2; cam++) {
-        if (!src[cam]) continue;
+        if (!srcs[cam]) continue;
         if (prep || staged_upload) {
             uint8_t* dst = d_stage[par] + (size_t)cam * B * img;
-            DVFE_CHECK(h2d(dst, row, img, src[cam], (size_t)pitch, stream_stride, row));
+            DVFE_CHECK(h2d(dst, row, img, srcs[cam], (size_t)pitch, stream_stride, row));
             if (prep) DVFE_CHECK(ingest(dst, img, (int)row, cam, cs));
         } else {
-            DVFE_CHECK(h2d(level0(cam), desc.lv[0].pitch, desc.bytes, src[cam], (size_t)pitch, stream_stride, row));
+            DVFE_CHECK(h2d(level0(cam), desc.lv[0].pitch, desc.bytes, srcs[cam], (size_t)pitch, stream_stride, row));
         }
     }
     DVFE_CUDA(cudaEventRecord(ev_up[par], cs));
     DVFE_CUDA(cudaStreamWaitEvent(st, ev_up[par], 0));
     if (!prep && staged_upload) {
         in->left = d_stage[par]; in->right = right ? d_stage[par] + B * img : nullptr;
+        in->stride = img; in->pitch = W; in->in_place = false;
+    }
+    return DVFE_OK;
+}
+
+// Every image from where it lives, absent ones not at all.  Host: one 2-D copy per present image, into level 0 or the staging
+// buffer, which the routes above then treat as a slab.  Device: the table goes to the device and the gather form of the level-0
+// copy (with the border) or of the ingest kernel reads each image through it, on the compute stream.
+int dvfe_tracker::place_table(const StepSources& src, bool device, StepInput* in) {
+    const bool prep = prep_active();
+    *in = StepInput();
+    in->has_right = src.any(1);
+    in->in_place = true;
+    if (device) {
+        DVFE_CHECK(upload_sources(src));
+        for (int cam = 0; cam < 2; cam++) {
+            if (!src.any(cam)) continue;
+            if (prep) {
+                IngestArgs a;
+                a.src = nullptr; a.src_stride = 0; a.src_pitch = 0; a.ch = in_ch;
+                a.map1 = maps_uniform[cam] ? stream_map1(cam, 0) : nullptr;
+                a.map2 = maps_uniform[cam] ? stream_map2(cam, 0) : nullptr;
+                a.dst = level0(cam);
+                a.dst_stride = desc.bytes; a.dst_pitch = desc.lv[0].pitch;
+                a.w = W; a.h = H; a.n_img = B; a.keep_channels = 0;
+                DVFE_CHECK(launch_ingest_table(a, d_src + (size_t)cam * B, st, maps_uniform[cam] ? nullptr : d_imaps[cam]));
+            } else {
+                DVFE_CHECK(launch_pyr_level0_table(d_src + (size_t)cam * B, cam ? right_slot(frames) : left_slot(frames), desc.bytes,
+                                                   B, desc, st));
+            }
+        }
+        in->l0_border = !prep && pyr_level0_writes_border(desc);
+        return DVFE_OK;
+    }
+    const int par = (int)(frames % 2);
+    const size_t row = (size_t)W * in_ch, img = row * H;
+    for (int cam = 0; cam < 2; cam++) {
+        if (!src.any(cam)) continue;
+        uint8_t* stage = d_stage[par] + (size_t)cam * B * img;
+        for (int s = 0; s < B; s++) {
+            const ImgSrc& e = src.img[cam][s];
+            if (!e.ptr) continue;
+            if (prep || staged_upload)
+                DVFE_CUDA(cudaMemcpy2DAsync(stage + s * img, row, e.ptr, (size_t)e.pitch, row, (size_t)H, cudaMemcpyHostToDevice, cs));
+            else
+                DVFE_CUDA(cudaMemcpy2DAsync(level0(cam) + s * (size_t)desc.bytes, (size_t)desc.lv[0].pitch, e.ptr, (size_t)e.pitch, row,
+                                            (size_t)H, cudaMemcpyHostToDevice, cs));
+        }
+        if (prep) DVFE_CHECK(ingest(stage, img, (int)row, cam, cs));
+    }
+    DVFE_CUDA(cudaEventRecord(ev_up[par], cs));
+    DVFE_CUDA(cudaStreamWaitEvent(st, ev_up[par], 0));
+    if (!prep && staged_upload) {
+        in->left = d_stage[par]; in->right = in->has_right ? d_stage[par] + B * img : nullptr;
         in->stride = img; in->pitch = W; in->in_place = false;
     }
     return DVFE_OK;
@@ -855,11 +954,11 @@ static int check_step_args(dvfe_tracker* t, const uint8_t* left, int pitch, cons
 }
 
 // one raw step of a leaf tracker, enqueued; sflags: per-stream DVFE_FRAME_* (validated) or null
-static int leaf_track(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch,
-                      const double* time0, const uint8_t* sflags, bool device) {
+int leaf_track(dvfe_tracker* t, const StepSources& src, const double* time0, const uint8_t* sflags, bool device) {
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
+    t->src_step = -1;                       // this step's table is not on the device yet
     StepInput in;
-    DVFE_CHECK(t->place_input(left, right, stream_stride, pitch, device, &in));
+    DVFE_CHECK(t->place_input(src, device, &in));
     return t->submit(in, time0, false, sflags);
 }
 
@@ -925,7 +1024,7 @@ extern "C" int dvfe_track_image_ex(dvfe_tracker* t, const uint8_t* left, const u
     const uint8_t* sf = nullptr;
     DVFE_CHECK(check_stream_flags(stream_flags, t->B, "track_image_ex", &sf));
     if (IS_GROUP(t)) return grp_track_image_ex(t, left, right, stream_stride, pitch, time0, sf, device);
-    return leaf_track(t, left, right, stream_stride, pitch, time0, sf, device);
+    return leaf_track(t, t->slab(left, right, nullptr, stream_stride, pitch), time0, sf, device);
 }
 
 extern "C" int dvfe_set_lk_mode_site(dvfe_tracker* t, int site, int back_max_level, double fb_threshold) {
@@ -953,43 +1052,45 @@ extern "C" int dvfe_set_detect_mode(dvfe_tracker* t, int mode) {
     return DVFE_OK;
 }
 
-int dvfe_tracker::semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask,
-                                  size_t stream_stride, int pitch, const int* exist_inst, const double* time0, unsigned flags,
+int dvfe_tracker::semantic_submit(const StepSources& src, const int* exist_inst, const double* time0, unsigned flags,
                                   const uint8_t* sflags) {
     DVFE_CHECK(wait_slot());                // before the mask copy: d_inv_in[par] / d_labels[par] are step k-2's until then
+    src_step = -1;                          // this step's table is not on the device yet
     const size_t P = (size_t)W * H;
     const int par = (int)(frames % 2);
-    const bool prep = prep_active();
     const bool device = (flags & DVFE_DYN_DEVICE_INPUT) != 0, labels = (flags & DVFE_DYN_LABELS) != 0;
-    // the region mask / label image is one byte per pixel whatever the image format
-    const size_t mask_stride = prep ? stream_stride / (size_t)in_ch : stream_stride;
-    const int mask_pitch = prep ? pitch / in_ch : pitch;
+    const std::vector<ImgSrc>& mask = src.img[2];
     // a skipped stream counts as one without instances: its mask is neither copied nor eroded
     bool all = true;
     for (int s = 0; s < B; s++) {
         const bool ex = !(sflags && (sflags[s] & DVFE_FRAME_SKIP)) && exist_inst[s];
         h_exist[par][s] = ex ? 1 : 0;
         all = all && ex;
-        if (ex && !mask) { dvfe_set_error("track_semantic_image: exist_inst set but no mask"); return DVFE_ERR_INVALID; }
+        if (ex && !mask[s].ptr) { dvfe_set_error("track_semantic_image: exist_inst set but no mask"); return DVFE_ERR_INVALID; }
     }
-    const uint8_t* d_mask = mask;            // where the erosion reads the mask / label image from
-    size_t d_mask_stride = mask_stride;
-    int d_mask_pitch = mask_pitch;
-    if (!device) {
-        // mask -> device on the upload stream, ahead of the images (one copy when every stream has one)
+    // where the erosion reads the mask / label image from
+    const uint8_t* d_mask = src.uniform[2] ? mask[0].ptr : nullptr;
+    size_t d_mask_stride = src.stride[2];
+    int d_mask_pitch = mask[0].pitch;
+    if (!device || (!src.uniform[2] && src.any(2))) {
+        // host: mask -> device on the upload stream, ahead of the images (one copy when every stream has one);
+        // device masks that are not one slab: gathered on the compute stream
         if (labels && !d_labels[par]) DVFE_CUDA(cudaMalloc((void**)&d_labels[par], (size_t)B * P));
         uint8_t* dst = labels ? d_labels[par] : d_inv_in[par];
-        if (all && mask_pitch == W && mask_stride == P) {
-            DVFE_CUDA(cudaMemcpyAsync(dst, mask, (size_t)B * P, cudaMemcpyHostToDevice, cs));
+        if (device) {
+            DVFE_CHECK(upload_sources(src));
+            DVFE_CHECK(launch_gather_images(d_src + (size_t)2 * B, dst, P, W, W, H, B, st));
+        } else if (all && src.uniform[2] && mask[0].pitch == W && src.stride[2] == P) {
+            DVFE_CUDA(cudaMemcpyAsync(dst, mask[0].ptr, (size_t)B * P, cudaMemcpyHostToDevice, cs));
         } else {
             for (int s = 0; s < B; s++)
                 if (h_exist[par][s])
-                    DVFE_CUDA(cudaMemcpy2DAsync(dst + s * P, W, mask + s * mask_stride, mask_pitch, W, (size_t)H, cudaMemcpyHostToDevice, cs));
+                    DVFE_CUDA(cudaMemcpy2DAsync(dst + s * P, W, mask[s].ptr, mask[s].pitch, W, (size_t)H, cudaMemcpyHostToDevice, cs));
         }
         d_mask = dst; d_mask_stride = P; d_mask_pitch = W;
     }
     StepInput in;                           // a host route's ev_up, recorded after the images, covers the mask copy too
-    DVFE_CHECK(place_input(left, right, stream_stride, pitch, device, &in));
+    DVFE_CHECK(place_input(src, device, &in));
     lab_ptr[par] = labels ? d_mask : nullptr; lab_stride[par] = d_mask_stride; lab_pitch[par] = d_mask_pitch;
     DVFE_CUDA(cudaMemcpyAsync(d_exist, h_exist[par], B * sizeof(int), cudaMemcpyHostToDevice, st));
     // region mask = exist_inst ? erode(inv_merge_mask, mask_morphology_size) : all 255   (:764-772); with a label image
@@ -1016,7 +1117,7 @@ extern "C" int dvfe_track_semantic_ex(dvfe_tracker* t, const uint8_t* left, cons
     DVFE_CHECK(check_stream_flags(stream_flags, t->B, "track_semantic_ex", &sf));
     if (IS_GROUP(t)) return grp_track_semantic(t, left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0, sf, flags);
     DVFE_CUDA(cudaSetDevice(t->cfg.device));
-    return t->semantic_submit(left, right, inv_merge_mask, stream_stride, pitch, exist_inst, time0, flags, sf);
+    return t->semantic_submit(t->slab(left, right, inv_merge_mask, stream_stride, pitch), exist_inst, time0, flags, sf);
 }
 
 extern "C" int dvfe_track_semantic_image(dvfe_tracker* t, const uint8_t* left, const uint8_t* right,

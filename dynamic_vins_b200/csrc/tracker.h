@@ -42,6 +42,32 @@ struct SnapInstDev {
     uint8_t* crop;
 };
 
+// Where each stream's images of a step are: img[0] left, img[1] right, img[2] mask / label image, B entries each.  A null pointer
+// is an absent image: nothing is read or copied for it.  A slab call (base + s * stride) gives a uniform table; dvfe_track_frames
+// gives one entry per camera, uniform only when its cameras happen to lie in one slab.
+struct StepSources {
+    std::vector<ImgSrc> img[3];
+    bool uniform[3] = {false, false, false};         // every stream has image c, all at one pitch, stream s at img[c][0] + s * stride[c]
+    size_t stride[3] = {0, 0, 0};
+    bool any(int c) const {
+        for (const ImgSrc& e : img[c])
+            if (e.ptr) return true;
+        return false;
+    }
+};
+// The table of a slab: every stream has each image whose base is not null
+StepSources slab_sources(int B, const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stride, int pitch,
+                         size_t mask_stride, int mask_pitch);
+
+struct dvfe_tracker;
+// One step of a leaf tracker from a source table, enqueued; sflags: per-stream DVFE_FRAME_* (validated) or null.
+// tracker.cu: the raw step.  instances.cu: the dynamic-mode step, whose boxes (boxes_of[s], n_boxes[s]) leaf_validate_boxes
+// checked before any stream group enqueued.
+int leaf_track(dvfe_tracker* t, const StepSources& src, const double* time0, const uint8_t* sflags, bool device);
+int leaf_validate_boxes(dvfe_tracker* t, const dvfe_inst_in* const* boxes_of, const int* n_boxes, bool labels, const uint8_t* sflags);
+int leaf_track_dynamic(dvfe_tracker* t, const StepSources& src, const int* exist_inst, const dvfe_inst_in* const* boxes_of,
+                       const int* n_boxes, const double* time0, const uint8_t* sflags, unsigned flags);
+
 // Where a frame step finds its images once dvfe_tracker::place_input has put them in place
 struct StepInput {
     const uint8_t* left = nullptr;                   // device images the step copies into level 0 (null when in_place)
@@ -49,6 +75,7 @@ struct StepInput {
     size_t stride = 0;                               // bytes between the streams' images
     int pitch = 0;
     bool in_place = false;                           // level 0 of this step's pyramid slots already holds the images
+    bool l0_border = false;                          // ... with its border (the gather kernel of a device table)
     bool has_right = false;
 };
 
@@ -190,7 +217,17 @@ struct dvfe_tracker {
     int h2d(uint8_t* dst, size_t dst_pitch, size_t dst_stride, const uint8_t* src, size_t src_pitch, size_t src_stride, size_t row);
     int wait_slot();                                 // fewer than two steps in flight: step k-2's buffers are free again
     // wait_slot, then put this step's images (host or device memory) where the step reads them
-    int place_input(const uint8_t* left, const uint8_t* right, size_t stream_stride, int pitch, bool device, StepInput* in);
+    int place_input(const StepSources& src, bool device, StepInput* in);
+    int place_table(const StepSources& src, bool device, StepInput* in);     // the routes of a table that is not uniform
+    // the slab table of this tracker: the mask / label image is one byte per pixel at the stride and pitch of the images divided
+    // by the channel count when the ingest kernel runs
+    StepSources slab(const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stride, int pitch) const;
+    // Per-step device copy of a table's pointers ([3][B], for the gather kernels), uploaded on the compute stream from a pinned
+    // copy per in-flight step; read only by kernels on the compute stream, so one device table serves every step
+    ImgSrc* d_src = nullptr;
+    ImgSrc* h_src[2] = {nullptr, nullptr};
+    long src_step = -1;                              // the step whose table d_src holds
+    int upload_sources(const StepSources& src);
     // enqueue one frame step (no host synchronisation); at most two steps are in flight
     // sflags (nullable): per-stream DVFE_FRAME_* (dvfe_track_image_ex / _semantic_ex / _dynamic_ex2), already validated
     int submit(const StepInput& in, const double* time0, bool semantic, const uint8_t* sflags = nullptr);
@@ -198,8 +235,8 @@ struct dvfe_tracker {
     // flags: DVFE_DYN_DEVICE_INPUT (the three pointers are device memory, nothing is uploaded), DVFE_DYN_LABELS (the mask is a
     // label image: the region is everything no instance bit is set on).  sflags: as submit; a skipped stream's exist_inst and
     // mask are not read, a RESET stream's instance manager starts over too
-    int semantic_submit(const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
-                        int pitch, const int* exist_inst, const double* time0, unsigned flags = 0, const uint8_t* sflags = nullptr);
+    int semantic_submit(const StepSources& src, const int* exist_inst, const double* time0, unsigned flags = 0,
+                        const uint8_t* sflags = nullptr);
     void reset_instances(int stream);                // instances.cu: a newly created InstsFeatManager for one stream
     // instances.cu, for stream snapshots: the instance table of `stream` in ascending track id with where each instance's device state
     // lives, and its last_time; insts_import replaces the table (slots from the free list) and says where the device state goes

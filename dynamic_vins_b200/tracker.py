@@ -10,7 +10,8 @@ set of kernel launches per step).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Optional, Sequence, Tuple
+import dataclasses
+from typing import Any, Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -64,6 +65,21 @@ def obs_to_map(rec: np.ndarray) -> Dict[int, List[Tuple[int, np.ndarray]]]:
     for r in rec:
         out.setdefault(int(r["id"]), []).append((int(r["cam"]), r["v"].copy()))
     return out
+
+
+@dataclasses.dataclass
+class Frame:
+    """One camera's images of a step (dvfe_frame) for BatchTracker.track_frames / track_semantic_frames / track_dynamic_frames.
+    Host input: numpy uint8 arrays, (H, W) gray or (H, W, 3) BGR, at any row stride (each array's strides[0] is its pitch; left
+    and right must share one).  Device input: (address, pitch) pairs of ints.  right None: left image only.  mask: the
+    inv_merge_mask (semantic / dynamic) or the label image (dynamic with labels), one byte per pixel.  A stream without a frame
+    is None in the frame list, not a Frame."""
+    left: Any
+    right: Any = None
+    time0: float = 0.0
+    mask: Any = None
+    exist_inst: int = 0
+    reset: bool = False
 
 
 class BatchTracker:
@@ -208,6 +224,82 @@ class BatchTracker:
         self._keep_t = (t, getattr(self, "_keep_t", (None,))[0])
         L.check(L.lib().dvfe_track_image_ex(self._h, C.c_void_p(d_left), C.c_void_p(d_right) if d_right else None,
                                             stream_stride, pitch, L.ptr(t), L.ptr(f), L.STEP_DEVICE_INPUT))
+
+    # ---- per-camera frame descriptors (dvfe_track_frames) ------------------------------------------
+    def _image(self, a, shape, device: bool, keep: list) -> Tuple[int, int]:
+        """(address, pitch) of one image"""
+        if device:
+            addr, pitch = a
+            return int(addr), int(pitch)
+        a = np.asarray(a)
+        if a.shape != shape or a.dtype != np.uint8:
+            raise ValueError(f"image of shape {shape} uint8 expected, got {a.shape} {a.dtype}")
+        if a.strides[1:] != ((a.shape[2], 1) if a.ndim == 3 else (1,)):
+            a = np.ascontiguousarray(a)          # the pixels of a row must be dense; the row stride may be anything
+        keep.append(a)
+        return a.ctypes.data, a.strides[0]
+
+    def _frames(self, frames, device: bool, masks: bool) -> Tuple[C.Array, list]:
+        """the dvfe_frame array of a step; keep: what has to stay alive until the step is waited for"""
+        frames = list(frames)
+        if len(frames) != self.B:
+            raise ValueError(f"frames: one entry per stream expected ({self.B}), got {len(frames)}")
+        img = (self.H, self.W) if self.ch == 1 else (self.H, self.W, self.ch)
+        arr = (L.FrameDesc * self.B)()
+        keep: list = [arr]
+        for s, f in enumerate(frames):
+            if f is None:
+                continue
+            d = arr[s]
+            if f.left is not None:
+                d.left, d.pitch = self._image(f.left, img, device, keep)
+            if f.right is not None:
+                d.right, pitch = self._image(f.right, img, device, keep)
+                if pitch != d.pitch:
+                    raise ValueError(f"frames[{s}]: left and right must share one row pitch ({d.pitch} != {pitch})")
+            if masks and f.mask is not None:
+                d.mask, d.mask_pitch = self._image(f.mask, (self.H, self.W), device, keep)
+            d.exist_inst = int(f.exist_inst)
+            d.flags = L.FRAME_RESET if f.reset else 0
+            d.time0 = float(f.time0)
+        return arr, keep
+
+    def _keep_step(self, keep) -> None:
+        """hold a step's buffers until the step after the next one is enqueued (at most two steps are in flight)"""
+        self._keep_frames = (keep, getattr(self, "_keep_frames", (None,))[0])
+
+    def track_frames(self, frames: Sequence[Optional[Frame]], device: bool = False) -> None:
+        """TrackImage of one step described camera by camera (include/dvfe.h dvfe_track_frames), enqueued: records after the
+        matching wait().  frames[s]: a Frame, or None when stream s has no frame in this step."""
+        self._leave_naive()
+        arr, keep = self._frames(frames, device, masks=False)
+        self._keep_step(keep)
+        L.check(L.lib().dvfe_track_frames(self._h, arr, L.STEP_DEVICE_INPUT if device else 0))
+
+    def track_semantic_frames(self, frames: Sequence[Optional[Frame]], device: bool = False, naive: bool = False) -> None:
+        """TrackSemanticImage (naive=True: TrackImageNaive, see track_image_naive) of one step described camera by camera
+        (dvfe_track_semantic_frames), enqueued: records after the matching wait().  Frame.mask is the inv_merge_mask."""
+        if naive:
+            self._enter_naive()
+        else:
+            self._leave_naive()
+        arr, keep = self._frames(frames, device, masks=True)
+        self._keep_step(keep)
+        L.check(L.lib().dvfe_track_semantic_frames(self._h, arr, self.DYN_DEVICE_INPUT if device else 0))
+
+    def track_dynamic_frames(self, frames: Sequence[Optional[Frame]], boxes_per_stream, labels: bool = False,
+                             device: bool = False) -> None:
+        """TrackSemanticImage + InstsTrack of one step described camera by camera (dvfe_track_dynamic_frames), enqueued: results
+        after the matching wait().  Frame.mask is the inv_merge_mask, or with labels=True the label image; boxes_per_stream as
+        track_dynamic_async takes them (a stream without a frame has no boxes)."""
+        self._leave_naive()
+        arr, keep = self._frames(frames, device, masks=True)
+        boxes, counts, bkeep = boxes_per_stream if isinstance(boxes_per_stream, tuple) else self.marshal_boxes(boxes_per_stream)
+        if len(counts) != self.B:
+            raise ValueError(f"boxes_per_stream: one box list per stream expected ({self.B}), got {len(counts)}")
+        self._keep_step((keep, boxes, counts, bkeep))
+        flags = (self.DYN_LABELS if labels else 0) | (self.DYN_DEVICE_INPUT if device else 0)
+        L.check(L.lib().dvfe_track_dynamic_frames(self._h, arr, boxes, L.ptr(counts), flags))
 
     LK_RAW_TEMPORAL, LK_RAW_STEREO, LK_SEMANTIC_TEMPORAL, LK_SEMANTIC_STEREO = 0, 1, 2, 3
 

@@ -181,7 +181,8 @@ int dvfe_track_image_device_async(dvfe_tracker* t, const uint8_t* d_left, const 
  *                        next_id = 1, prev_time = 0) and the frame runs as a first frame; may be combined with NO_RIGHT
  * Unknown bits, SKIP|RESET and unknown `flags` bits return DVFE_ERR_INVALID and change nothing.  With right != NULL all B
  * slots of both images must be readable; the pixels of a skipped stream, and of a NO_RIGHT stream's right image, affect no
- * result.  right == NULL makes every stream mono.  flags: DVFE_STEP_DEVICE_INPUT = left / right are device pointers. */
+ * result.  right == NULL makes every stream mono.  flags: DVFE_STEP_DEVICE_INPUT = left / right are device pointers.
+ * dvfe_track_frames takes each camera's images from its own buffer instead, and reads nothing of a camera without a frame. */
 #define DVFE_FRAME_SKIP 1u
 #define DVFE_FRAME_NO_RIGHT 2u
 #define DVFE_FRAME_RESET 4u
@@ -278,6 +279,41 @@ int dvfe_track_dynamic_ex(dvfe_tracker* t, const uint8_t* left, const uint8_t* r
 int dvfe_track_dynamic_ex2(dvfe_tracker* t, const uint8_t* left, const uint8_t* right, const uint8_t* mask, size_t stream_stride,
                            int pitch, const int* exist_inst, const dvfe_inst_in* boxes, const int* n_boxes, const double* time0,
                            const uint8_t* stream_flags, unsigned flags);
+
+/* Per-camera frame descriptors: a step described camera by camera, each image taken from its own buffer at its own pitch
+ * (a decoder's output, a V4L2 / GStreamer buffer, SemanticImage::gray0), with no slab to assemble and nothing uploaded for a
+ * camera without a frame.  frames[s] describes stream s, s < n_streams.  */
+typedef struct dvfe_frame {
+    const uint8_t* left;     /* NULL: no frame from this camera in this step (as DVFE_FRAME_SKIP) */
+    const uint8_t* right;    /* NULL: left image only (as DVFE_FRAME_NO_RIGHT); ignored by a mono tracker */
+    const uint8_t* mask;     /* semantic: inv_merge_mask; dynamic with DVFE_DYN_LABELS: the label image; otherwise NULL */
+    int32_t pitch;           /* bytes per row of left and right, >= width * channels (dvfe_set_input) */
+    int32_t mask_pitch;      /* bytes per row of mask, >= width */
+    int32_t exist_inst;      /* SemanticImage::exist_inst (semantic / dynamic) */
+    uint32_t flags;          /* DVFE_FRAME_RESET; other bits are invalid (SKIP / NO_RIGHT follow from the NULL pointers) */
+    double time0;            /* not read when left == NULL */
+} dvfe_frame;
+
+/* The per-camera forms of dvfe_track_image_ex (TrackImage; flags: DVFE_STEP_DEVICE_INPUT), dvfe_track_semantic_ex
+ * (TrackSemanticImage, and TrackImageNaive through dvfe_set_detect_mode; flags: DVFE_DYN_DEVICE_INPUT) and dvfe_track_dynamic_ex2
+ * (flags: DVFE_DYN_DEVICE_INPUT | DVFE_DYN_LABELS; boxes / n_boxes as there).  Each is enqueued and paired with dvfe_wait.
+ *   Equivalence: a call equals the matching slab call, bit for bit, in records, state and instance tables: the same pixels in
+ *     the present slots and stream_flags[s] = (left == NULL ? DVFE_FRAME_SKIP : 0) | (right == NULL ? DVFE_FRAME_NO_RIGHT : 0) |
+ *     frames[s].flags.  Exception: when no present frame has a right image, the step is the slab call's mono step (right = NULL)
+ *     with the present streams' RESET and the SKIP flags only.
+ *   What is read: nothing behind a NULL pointer, and nothing of an absent image is uploaded.  The pixels, mask, exist_inst and
+ *     time0 of a skipped stream are not read.  Host images are copied row by row (width * channels bytes of each row); a device
+ *     image is read within its height * pitch bytes.
+ *   Invalid input (DVFE_ERR_INVALID, nothing changes, as for the slab calls): frames == NULL, DVFE_FRAME_RESET with left == NULL,
+ *     unknown frame or step flag bits, pitch < width * channels for a present image, mask_pitch < width for a present mask,
+ *     exist_inst set without a mask, boxes for a skipped stream.
+ *   Lifetime: images and masks must stay valid until the step is waited for, as with the asynchronous slab calls.
+ *   Stream groups: each group takes its own range of the array.
+ * A table whose images all lie in one slab at one pitch runs exactly the copies and kernels of the slab call. */
+int dvfe_track_frames(dvfe_tracker* t, const dvfe_frame* frames, unsigned flags);
+int dvfe_track_semantic_frames(dvfe_tracker* t, const dvfe_frame* frames, unsigned flags);
+int dvfe_track_dynamic_frames(dvfe_tracker* t, const dvfe_frame* frames, const dvfe_inst_in* boxes, const int* n_boxes,
+                              unsigned flags);
 
 /* FeatureBackground of stream s of the last step: n_out records, sorted by (id, cam). */
 int dvfe_get_features(dvfe_tracker* t, int stream, dvfe_obs* out, int cap, int* n_out);

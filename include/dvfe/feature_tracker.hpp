@@ -476,6 +476,31 @@ public:
         if ((int)stream_flags.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one stream flag per stream expected");
         dynamic(left, right, inv_merge_mask, stream_stride, step, exist_inst, boxes2d, time0, stream_flags.data());
     }
+    // One step described camera by camera (dvfe_track_frames): frames[s].left == nullptr = no frame from camera s, right == nullptr
+    // = left image only, each camera at its own pitch; only the present images are read.  Enqueued; the images stay valid until
+    // the matching Wait().  `device`: the pointers are device memory.
+    void TrackFramesAsync(const std::vector<dvfe_frame>& frames, bool device = false) {
+        check_frames(frames);
+        if (dvfe_track_frames(h_, frames.data(), device ? DVFE_STEP_DEVICE_INPUT : 0u) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
+    // TrackSemanticImage of every camera, described camera by camera (dvfe_track_semantic_frames; frames[s].mask = inv_merge_mask)
+    void TrackSemanticFramesAsync(const std::vector<dvfe_frame>& frames, bool device = false) {
+        check_frames(frames);
+        if (dvfe_track_semantic_frames(h_, frames.data(), device ? DVFE_DYN_DEVICE_INPUT : 0u) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
+    // TrackSemanticImage + InstsTrack of every camera, described camera by camera (dvfe_track_dynamic_frames); a camera without a
+    // frame has an empty box list.  flags: DVFE_DYN_DEVICE_INPUT | DVFE_DYN_LABELS.
+    void TrackDynamicFramesAsync(const std::vector<dvfe_frame>& frames, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,
+                                 unsigned flags = 0u) {
+        check_frames(frames);
+        std::vector<dvfe_inst_in> in;
+        std::vector<int> n;
+        marshal(boxes2d, &in, &n);
+        if (dvfe_track_dynamic_frames(h_, frames.data(), in.empty() ? nullptr : in.data(), n.data(), flags) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
     // the oldest enqueued frame is finished: Features() / InstsOutput() return its results
     void Wait() {
         if (dvfe_wait(h_) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
@@ -516,23 +541,32 @@ private:
                  const std::vector<int>& exist_inst, const std::vector<std::vector<Box2D::Ptr>>& boxes2d,
                  const std::vector<double>& time0, const uint8_t* stream_flags) {
         check(time0);
-        if ((int)exist_inst.size() != cfg_.n_streams || (int)boxes2d.size() != cfg_.n_streams)
+        if ((int)exist_inst.size() != cfg_.n_streams)
             throw std::runtime_error("BatchFeatureTracker: one exist_inst / box list per stream expected");
         std::vector<dvfe_inst_in> in;
-        std::vector<int> n(boxes2d.size());
+        std::vector<int> n;
+        marshal(boxes2d, &in, &n);
+        if (dvfe_track_dynamic_ex2(h_, left, right, inv_merge_mask, stream_stride, step, exist_inst.data(),
+                                   in.empty() ? nullptr : in.data(), n.data(), time0.data(), stream_flags, 0u) != DVFE_OK)
+            throw std::runtime_error(dvfe_last_error(h_));
+    }
+    // the dvfe_inst_in array (stream by stream) and per-stream counts of a frame's box lists
+    void marshal(const std::vector<std::vector<Box2D::Ptr>>& boxes2d, std::vector<dvfe_inst_in>* in, std::vector<int>* n) const {
+        if ((int)boxes2d.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one exist_inst / box list per stream expected");
+        n->resize(boxes2d.size());
         for (size_t s = 0; s < boxes2d.size(); s++) {
-            n[s] = (int)boxes2d[s].size();
+            (*n)[s] = (int)boxes2d[s].size();
             for (const Box2D::Ptr& b : boxes2d[s]) {
                 dvfe_inst_in d{};
                 d.track_id = (uint32_t)b->track_id;
                 d.x = (int)b->rect.x; d.y = (int)b->rect.y; d.w = (int)b->rect.width; d.h = (int)b->rect.height;
                 d.mask = b->roi ? b->roi->mask_cv.data : nullptr; d.mask_pitch = b->roi ? b->roi->mask_cv.step : 0;
-                in.push_back(d);
+                in->push_back(d);
             }
         }
-        if (dvfe_track_dynamic_ex2(h_, left, right, inv_merge_mask, stream_stride, step, exist_inst.data(),
-                                   in.empty() ? nullptr : in.data(), n.data(), time0.data(), stream_flags, 0u) != DVFE_OK)
-            throw std::runtime_error(dvfe_last_error(h_));
+    }
+    void check_frames(const std::vector<dvfe_frame>& frames) const {
+        if ((int)frames.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one frame descriptor per stream expected");
     }
     void check(const std::vector<double>& time0) const {
         if ((int)time0.size() != cfg_.n_streams) throw std::runtime_error("BatchFeatureTracker: one time0 per stream expected");

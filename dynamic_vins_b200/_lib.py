@@ -90,6 +90,8 @@ SYMBOLS = [
     "dvfe_export_stream", "dvfe_import_stream",
     "dvfe_track_frames", "dvfe_track_semantic_frames", "dvfe_track_dynamic_frames",
 ]
+# every symbol include/dvfe/reject_with_f.h declares (the companion header of the in-step RejectWithF)
+REJECT_SYMBOLS = ["dvfe_set_reject_with_f", "dvfe_f_threshold_from_yaml"]
 
 # dvfe_track_image_ex / _semantic_ex / _dynamic_ex2: per-stream frame flags; dvfe_track_image_ex's step flags (include/dvfe.h)
 FRAME_SKIP, FRAME_NO_RIGHT, FRAME_RESET = 1, 2, 4
@@ -168,6 +170,8 @@ def lib() -> C.CDLL:
         L.dvfe_track_dynamic_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint]
         L.dvfe_op_merge_masks.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
         L.dvfe_set_detect_mode.argtypes = [C.c_void_p, C.c_int]
+        L.dvfe_set_reject_with_f.argtypes = [C.c_void_p, C.c_double]
+        L.dvfe_f_threshold_from_yaml.argtypes = [C.c_char_p, C.POINTER(C.c_double)]
         L.dvfe_op_build_pyramid_bordered.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
         L.dvfe_op_reject_with_f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p,
                                             C.POINTER(C.c_int)]

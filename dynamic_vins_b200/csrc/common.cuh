@@ -5,6 +5,7 @@
 #include <stdio.h>
 
 #include "../../include/dvfe.h"
+#include "../../include/dvfe/reject_with_f.h"
 
 // Padded pyramid storage.  LK reads a 22x22 window whose origin lies in [-21, w-1] x [-21, h-1]
 // (cv::calcOpticalFlowPyrLK keeps a winSize border around every level), plus one more pixel for

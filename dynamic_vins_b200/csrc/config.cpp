@@ -13,6 +13,7 @@
 #include <string>
 
 #include "../../include/dvfe.h"
+#include "../../include/dvfe/reject_with_f.h"
 
 void dvfe_set_error(const char* fmt, ...);
 
@@ -85,6 +86,19 @@ extern "C" int dvfe_camera_from_yaml(const char* path, dvfe_camera* cam) {
     const int rc = read_camera(path, &c);
     if (rc == DVFE_OK) *cam = c;
     return rc;
+}
+
+extern "C" int dvfe_f_threshold_from_yaml(const char* path, double* f) {
+    if (!path || !f) { dvfe_set_error("f_threshold_from_yaml: null argument"); return DVFE_ERR_INVALID; }
+    std::map<std::string, std::string> kv;
+    if (!read_flat_yaml(path, kv)) {
+        dvfe_set_error("ERROR: Wrong path to settings:%s", path);
+        return DVFE_ERR_CONFIG;
+    }
+    double v = 0.0;                           // fs["F_threshold"] >> F_threshold: 0 when the key is absent
+    get_double(kv, "F_threshold", &v);
+    *f = v;
+    return DVFE_OK;
 }
 
 extern "C" int dvfe_config_from_yaml(const char* config_path, dvfe_config* cfg) {

@@ -156,6 +156,11 @@ int grp_set_detect_mode(dvfe_tracker* t, int mode) {
     return DVFE_OK;
 }
 
+int grp_set_reject_with_f(dvfe_tracker* t, double f_threshold) {
+    for (dvfe_tracker* g : t->groups) DVFE_CHECK(dvfe_set_reject_with_f(g, f_threshold));
+    return DVFE_OK;
+}
+
 int grp_profile(dvfe_tracker* t, int enable) {
     for (dvfe_tracker* g : t->groups) DVFE_CHECK(dvfe_profile(g, enable));
     return DVFE_OK;

@@ -27,6 +27,10 @@ int launch_left_post(const PointSetArrays& S, int n_sets, int cap, const CamPara
 int launch_inst_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, int sets_per_cam,
                           const double* d_dt, const uint8_t* d_active, int stereo_now, const uint8_t* d_lane,
                           const uint32_t* d_inst_id, dvfe_inst_obs* out, int* d_n_out, cudaStream_t st);
+// reject.cu: RejectWithF of every present stream's temporal-LK survivors (clears their status); d_models: reject_with_f_models doubles
+size_t reject_with_f_models(int n_sets);
+int launch_reject_with_f_step(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams, const uint8_t* d_lane, int W, int H,
+                              double threshold, double* d_models, cudaStream_t st);
 int launch_clear_sets(int* d_n, const uint8_t* d_flags, int n_sets, cudaStream_t st);
 int launch_right_post_pack(const PointSetArrays& S, int n_sets, int cap, const CamParams* d_cams1, const double* d_dt,
                            int stereo_now, dvfe_obs* obs, int* n_obs, cudaStream_t st, const uint8_t* d_lane = nullptr);

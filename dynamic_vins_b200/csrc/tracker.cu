@@ -43,6 +43,7 @@ int grp_track_semantic(dvfe_tracker* t, const uint8_t* left, const uint8_t* righ
 int grp_route(dvfe_tracker* t, int stream, dvfe_tracker** leaf, int* local);
 int grp_set_lk_mode(dvfe_tracker* t, int site, int back_max_level, double fb);
 int grp_set_detect_mode(dvfe_tracker* t, int mode);
+int grp_set_reject_with_f(dvfe_tracker* t, double f_threshold);
 int grp_profile(dvfe_tracker* t, int enable);
 int grp_profile_read(dvfe_tracker* t, const char** names, double* total_ms, long* steps);
 #define IS_GROUP(t) ((t) != nullptr && !(t)->groups.empty())
@@ -337,7 +338,7 @@ extern "C" void dvfe_destroy(dvfe_tracker* t) {
     for (int s = 0; s < 2; s++) cudaFree(t->pyrR[s]);
     free_point_sets(&t->bg);
     cudaFree(t->d_next_id); cudaFree(t->d_dt); cudaFree(t->d_err); cudaFree(t->d_tcache); cudaFree(t->d_tcache_bwd);
-    cudaFree(t->d_old_idx);
+    cudaFree(t->d_old_idx); cudaFree(t->d_fm_models);
     cudaFree(t->d_sflags); cudaFree(t->d_lane); cudaFree(t->d_pgroups[0]); cudaFree(t->d_pgroups[1]); cudaFree(t->d_pjobs);
     cudaFree(t->d_zero);
     cudaFree(t->d_src);
@@ -441,6 +442,10 @@ int dvfe_tracker::enqueue_compute(const uint8_t* d_left, const uint8_t* d_right,
         DVFE_CHECK(launch_lk(partial ? d_pgroups[0] : d_groups[ph][semantic ? 1 : 0], B, cap, cfg.lk_max_level, cfg.flow_back, st,
                              lk_back_level[site_t], lk_fb_thresh[site_t], (tc_read ? LK_TCACHE_READ : 0) | (reuse ? LK_TCACHE_WRITE_BWD : 0)));
     mark(ST_LK_TEMPORAL + 1);
+    // RejectWithF (dvfe_set_reject_with_f): the survivors that fit no common epipolar geometry lose their status before the
+    // compaction; timed with it (the "compact" stage)
+    if (k > 0 && reject_f > 0.0)
+        DVFE_CHECK(launch_reject_with_f_step(bg, B, cap, d_cam, lane, W, H, reject_f, d_fm_models, st));
     if (k > 0)   // ReduceVector x4 + track_cnt++
         DVFE_CHECK(launch_compact(bg, B, cap, st, lane, reuse ? d_old_idx : nullptr));
     mark(ST_COMPACT + 1);
@@ -1049,6 +1054,22 @@ extern "C" int dvfe_set_detect_mode(dvfe_tracker* t, int mode) {
     if (IS_GROUP(t)) return grp_set_detect_mode(t, mode);
     t->detect_cuda = mode == DVFE_DETECT_CUDA;
     t->drop_graphs();                 // the captured steps carry the old job table
+    return DVFE_OK;
+}
+
+extern "C" int dvfe_set_reject_with_f(dvfe_tracker* t, double f_threshold) {
+    if (!t || !isfinite(f_threshold) || f_threshold < 0.0) {
+        dvfe_set_error("set_reject_with_f: the threshold must be finite and >= 0 (0 = off)");
+        return DVFE_ERR_INVALID;
+    }
+    if (IS_GROUP(t)) return grp_set_reject_with_f(t, f_threshold);
+    if (f_threshold == t->reject_f) return DVFE_OK;
+    if (f_threshold > 0.0 && !t->d_fm_models) {       // steps in flight never read it: they were enqueued with the mode off
+        DVFE_CUDA(cudaSetDevice(t->cfg.device));
+        DVFE_CUDA(cudaMalloc((void**)&t->d_fm_models, reject_with_f_models(t->B) * sizeof(double)));
+    }
+    t->reject_f = f_threshold;
+    t->drop_graphs();                 // the captured steps carry the old threshold (or no rejection)
     return DVFE_OK;
 }
 

@@ -153,6 +153,10 @@ struct dvfe_tracker {
     // the cv::cuda call pattern (TrackRightGPU, background_tracker.cpp:801: 3 levels, 1.0 px)
     int lk_back_level[4] = {1, 1, 1, 3};
     double lk_fb_thresh[4] = {0.5, 0.5, 0.5, 1.0};
+    // dvfe_set_reject_with_f: F_threshold of the in-step RejectWithF (0 = off) and the model scratch of its kernel (allocated when
+    // first enabled)
+    double reject_f = 0.0;
+    double* d_fm_models = nullptr;
 
     // The compute part of a frame step is a fixed launch sequence for a given buffer phase, input location and mode: it is
     // captured once into a CUDA graph and replayed (one launch per step and stream group instead of ~20).

@@ -53,6 +53,13 @@ def make_config(width: int, height: int, max_cnt: int, min_dist: int, cam0: dict
     return c
 
 
+def f_threshold_from_yaml(path: str) -> float:
+    """fe_para::F_threshold of a settings file (0.0 when the key is absent), the value BatchTracker.set_reject_with_f takes"""
+    f = C.c_double(0.0)
+    L.check(L.lib().dvfe_f_threshold_from_yaml(path.encode(), C.byref(f)))
+    return f.value
+
+
 def config_from_yaml(path: str) -> L.Config:
     c = L.Config()
     L.check(L.lib().dvfe_config_from_yaml(path.encode(), C.byref(c)))
@@ -319,6 +326,12 @@ class BatchTracker:
         self._leave_naive()
         L.check(L.lib().dvfe_set_detect_mode(self._h, 1 if cuda_semantics else 0))
         self._detect_cuda = bool(cuda_semantics)
+
+    def set_reject_with_f(self, f_threshold: float) -> None:
+        """RejectWithF inside every background step from the next one on (include/dvfe.h dvfe_set_reject_with_f): the temporal
+        LK's survivors off the fundamental matrix of cv::findFundamentalMat(FM_RANSAC, f_threshold, 0.99) are dropped before the
+        detection.  0 turns it off (the default); negative or non-finite values raise DvfeError."""
+        L.check(L.lib().dvfe_set_reject_with_f(self._h, float(f_threshold)))
 
     # TrackImageNaive switches the two semantic LK sites and the detector; the switch is made when a naive call follows another
     # entry point and undone when another entry point follows a naive call (each switch drops the tracker's captured graphs)

@@ -222,6 +222,12 @@ int dvfe_set_lk_mode_site(dvfe_tracker* t, int site, int back_max_level, double 
 #define DVFE_DETECT_CUDA 1
 int dvfe_set_detect_mode(dvfe_tracker* t, int mode);
 
+/* Epipolar outlier rejection inside the frame step (VINS-Mono's rejectWithF, FeatureTracker::RejectWithF) and the F_threshold
+ * reader: dvfe_set_reject_with_f / dvfe_f_threshold_from_yaml, declared (with their full contract) in the companion header
+ * dvfe/reject_with_f.h, which includes this one.  Off by default: every step is then exactly the step described here.  On, the
+ * survivors of the temporal LK that cv::findFundamentalMat(FM_RANSAC, F_threshold, 0.99) marks as outliers are removed before the
+ * detection; when it finds no model every point is kept (dvfe_op_reject_with_f reports all zeros for the same lists). */
+
 /* FeatureTracker::TrackSemanticImage(SemanticImage&) (front_end/background_tracker.cpp:757-837).
  * inv_merge_mask: HOST, same layout as left (0 = object, 255 = background), may be NULL when no stream has
  * instances; exist_inst[s] = SemanticImage::exist_inst. */
@@ -364,8 +370,8 @@ int dvfe_set_state(dvfe_tracker* t, int stream, const dvfe_state* st);
  * slot index, frame count (also none: the usual target of a migration) and buffer phase.  Its calibration is applied as
  * dvfe_set_stream_camera does; the template caches of the slot are dropped.
  * Not carried: undistortion maps (6 bytes per pixel and camera: the caller sets them on the destination slot with
- * dvfe_set_stream_undistort_maps) and the tracker-wide modes of dvfe_set_lk_mode* / dvfe_set_detect_mode (the continuation is exact
- * under the same modes).  Dynamic mode: take a snapshot between frames, after the frame's InstsTrack if the frame has one (the
+ * dvfe_set_stream_undistort_maps) and the tracker-wide modes of dvfe_set_lk_mode* / dvfe_set_detect_mode / dvfe_set_reject_with_f
+ * (the continuation is exact under the same modes).  Dynamic mode: take a snapshot between frames, after the frame's InstsTrack if the frame has one (the
  * library cannot tell whether a caller still means to call dvfe_insts_track for the last background step).
  * The blob is host-endian and read only by a library of the same snapshot format version (layout: DESIGN.md §2).  Both calls return
  * DVFE_ERR_INVALID and change nothing with a step of the stream's group in flight (not yet waited for), a bad stream index or a NULL

@@ -31,6 +31,7 @@
 #include <vector>
 
 #include "../dvfe.h"
+#include "reject_with_f.h"
 
 namespace dynamic_vins {
 
@@ -199,6 +200,11 @@ public:
         if (dvfe_set_detect_mode(h_, cuda_semantics ? DVFE_DETECT_CUDA : DVFE_DETECT_CPU) != DVFE_OK)
             throw std::runtime_error(dvfe_last_error(h_));
         detect_cuda_ = cuda_semantics;
+    }
+    // FeatureTracker::RejectWithF inside every background step (dvfe_set_reject_with_f): f_threshold = fe_para::F_threshold
+    // (dvfe_f_threshold_from_yaml), 0 = off.  The constructor leaves it off, as the reference's TrackImage never calls it.
+    void SetRejectWithF(double f_threshold) {
+        if (dvfe_set_reject_with_f(h_, f_threshold) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
     }
     // visualisation (DrawTrack) is outside the path: the image stays empty, the accessor exists for source compatibility
     GrayImage& img_track() { return img_vis_; }
@@ -431,6 +437,11 @@ public:
     // flight (dvfe_set_stream_undistort_maps)
     void SetStreamUndistortMaps(int stream, int cam, const int16_t* map1, const uint16_t* map2) {
         if (dvfe_set_stream_undistort_maps(h_, stream, cam, map1, map2) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
+    }
+
+    // RejectWithF inside every step of every stream (dvfe_set_reject_with_f; 0 = off, the default), from the next step on
+    void SetRejectWithF(double f_threshold) {
+        if (dvfe_set_reject_with_f(h_, f_threshold) != DVFE_OK) throw std::runtime_error(dvfe_last_error(h_));
     }
 
     // Everything the next step of one stream reads from earlier frames, as one blob (dvfe_export_stream); no step may be in flight
